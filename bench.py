@@ -2,7 +2,7 @@
 """Benchmark of the per-ray hot path (BASELINE.json: ray-steps/s and full-map wall time incl. GRFF at
 1/2/4/8 B200 next to the host CPU).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]          # this repo's CUDA path
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]   # this repo's CUDA path
     python bench.py --impl reference [...]                       # the reference's CPU algorithm (oracle port)
 
 A "step" is one full ray-traced GR+FF map through the fused kernel (trace + sample + transfer, theta from the
@@ -188,7 +188,7 @@ def reference_numpy_timing(cube, w, budget_rays=4096, n_steps=150):
     (script/resample_with_ray_tracing.py:42-61, :333-352) — plus sample_model_with_rays('cpu').  Bounded: n_steps steps."""
     ref = ROOT / "baseline" / "_ref"
     if not (ref / "raytracingGRFF").is_dir():
-        return {"unavailable": "baseline/_ref is not installed (run baseline/install_ref.sh where /root/reference exists)"}
+        return {"unavailable": "baseline/_ref is not installed (sh baseline/install_ref.sh <raytracingGRFF checkout>)"}
     code = r"""
 import json, os, sys, time
 import numpy as np
@@ -296,6 +296,33 @@ def config_dict(w, args):
         "cross_sections": "pencil rays traced on recorded steps only (the reference computes S at every step but "
                           "outputs only recorded steps, build_rays.py:241-244); RTGRFF_CS_EVERY_STEP=1 restores it",
     }
+
+
+DUMP_BYTES = 64_000_000
+NPY_HEADER_ROOM = 4096       # for the (at most three) .npy headers, so that the files on disk stay within the budget
+
+
+def dump_outputs(image, n_freq, out_dir, max_bytes=DUMP_BYTES):
+    """Write a rendered map as the caller of render_map receives it: tb.npy (T_b [K]) and vi.npy (V/I), float64,
+    one plane per frequency, from `image` = [tb planes | vi planes][row][col] (a torch tensor, any device).  A map
+    whose files would exceed max_bytes is replaced by the same fixed, seeded sample of pixels from every plane;
+    pixel_index.npy then holds their row-major indices into the image.  Returns the names written."""
+    import torch
+    planes, ny, nx = image.shape
+    out = {}
+    data_bytes = max_bytes - NPY_HEADER_ROOM
+    if image.numel() * 8 > data_bytes:
+        m = data_bytes // (planes * 8 + 8)
+        idx = np.sort(np.random.default_rng(0).choice(ny * nx, m, replace=False))
+        image = image.reshape(planes, ny * nx)[:, torch.from_numpy(idx).to(image.device)]
+        out["pixel_index"] = idx.astype(np.float64)
+    host = image.cpu().numpy()
+    out["tb"], out["vi"] = host[:n_freq], host[n_freq:]
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, a in out.items():
+        np.save(out_dir / f"{name}.npy", a)
+    return sorted(out)
 
 
 def lib_fingerprint():
@@ -432,7 +459,13 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the secondary workloads (configs 1-3, the other scaling mode, the numpy reference)")
     ap.add_argument("--e2e-steps", type=int, default=2)
     ap.add_argument("--spherical", action="store_true", help="build the cubes on the GPU from a spherical model")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's T_b and V/I maps to DIR/*.npy "
+                    "(float64, at most 64 MB: a larger map is a fixed pixel sample) to compare builds output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the CUDA arm's maps; the reference arm keeps none")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     w = workload(args.config, args.gpus)
     if args.impl == "reference":
@@ -481,6 +514,8 @@ def main():
     ms_per_step, _, kernel_ms = run.timed(args.steps)
     clk = clocks.stop()
     launches = ses.ctx.launch_count - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(run.image, run.nf, args.dump_outputs)
     active_total, pencil_total, samples_total = run.totals()
     value = run.nominal_total / (ms_per_step * 1e-3)
 

@@ -4,6 +4,7 @@
 """
 from __future__ import annotations
 
+import os
 import shutil
 import subprocess
 import sys
@@ -17,12 +18,17 @@ NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", 
               "-Xcompiler", "-fPIC", "-shared"]
 
 
+def cuda_tool(name):
+    """A CUDA toolkit program (nvcc, cuobjdump): from PATH, else from $CUDA_HOME/bin (default /usr/local/cuda),
+    so that a shell whose PATH lacks the toolkit still builds."""
+    return shutil.which(name) or str(Path(os.environ.get("CUDA_HOME") or "/usr/local/cuda") / "bin" / name)
+
+
 def build_library(force=False, verbose=False):
     srcs = sorted(CSRC.glob("*.cu")) + sorted(CSRC.glob("*.cuh")) + [PKG.parent / "include" / "rtgrff.h"]
     if not force and OUT.exists() and all(s.stat().st_mtime <= OUT.stat().st_mtime for s in srcs):
         return OUT
-    nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"
-    cmd = [nvcc, *NVCC_FLAGS, "-o", str(OUT), str(CSRC / "rtgrff_api.cu")]
+    cmd = [cuda_tool("nvcc"), *NVCC_FLAGS, "-o", str(OUT), str(CSRC / "rtgrff_api.cu")]
     if verbose:
         cmd.insert(1, "-Xptxas=-v")
     res = subprocess.run(cmd, capture_output=True, text=True)

@@ -45,6 +45,39 @@ def test_cuda_arm_fails_loudly_without_a_gpu():
     assert "CUDA" in (p.stderr + p.stdout)
 
 
+def test_steps_and_dump_outputs_are_checked(tmp_path):
+    p = _run(["--impl", "reference", "--config", "c3", "--steps", "0"])
+    assert p.returncode == 2 and "--steps must be at least 1" in p.stderr
+    p = _run(["--impl", "reference", "--config", "c3", "--dump-outputs", str(tmp_path / "out")])
+    assert p.returncode == 2 and "--dump-outputs" in p.stderr and not (tmp_path / "out").exists()
+
+
+def test_dump_outputs_whole_map_and_seeded_sample(tmp_path):
+    """--dump-outputs: a map within the budget is written whole; a larger one as the same seeded pixel sample of
+    every plane, within the budget, identical from run to run."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, str(ROOT))
+    import bench
+    nf, ny, nx = 3, 40, 50
+    image = torch.arange(2 * nf * ny * nx, dtype=torch.float64).reshape(2 * nf, ny, nx)
+    assert bench.dump_outputs(image, nf, tmp_path / "whole") == ["tb", "vi"]
+    np.testing.assert_array_equal(np.load(tmp_path / "whole" / "tb.npy"), image[:nf].numpy())
+    np.testing.assert_array_equal(np.load(tmp_path / "whole" / "vi.npy"), image[nf:].numpy())
+    budget = 20000
+    for d in ("a", "b"):
+        assert bench.dump_outputs(image, nf, tmp_path / d, max_bytes=budget) == ["pixel_index", "tb", "vi"]
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= budget
+    files = {f.stem: np.load(f) for f in (tmp_path / "a").iterdir()}
+    idx = files["pixel_index"].astype(np.int64)
+    assert files["pixel_index"].dtype == np.float64 and len(np.unique(idx)) == len(idx) > 0
+    flat = image.reshape(2 * nf, -1).numpy()
+    np.testing.assert_array_equal(files["tb"], flat[:nf, idx])
+    np.testing.assert_array_equal(files["vi"], flat[nf:, idx])
+    for name, a in files.items():
+        np.testing.assert_array_equal(np.load(tmp_path / "b" / f"{name}.npy"), a)
+
+
 def test_reference_numpy_leg_runs_the_unmodified_reference():
     """bench.py's `extras.reference_numpy`: the UNMODIFIED reference package (baseline/_ref, installed by
     baseline/install_ref.sh) timed in a child process: ray_trace single-process and over a process pool, the CPU sampler."""
@@ -52,7 +85,8 @@ def test_reference_numpy_leg_runs_the_unmodified_reference():
     sys.path.insert(0, str(ROOT))
     import bench
     if not (ROOT / "baseline" / "_ref" / "raytracingGRFF").is_dir():
-        pytest.skip("baseline/_ref is not installed here")
+        pytest.skip("the unmodified raytracingGRFF package is not part of the repository: install it into baseline/_ref "
+                    "with `sh baseline/install_ref.sh <raytracingGRFF checkout>`")
     w = bench.workload("c3", 1)
     w["grid_n"] = 32
     d = bench.reference_numpy_timing(None, w, budget_rays=64, n_steps=12)

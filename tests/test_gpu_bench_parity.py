@@ -69,6 +69,26 @@ def test_config4_bench_variant_matches_oracle_chain(oracle, session):
     _assert_parity(par, max_chaotic_frac=0.01)
 
 
+def test_bench_dump_outputs_are_the_timed_maps(session, tmp_path):
+    """bench.py --dump-outputs writes its last timed step's maps: the T_b and V/I that render_map returns for the
+    same workload (config 3, whole map), bit for bit."""
+    import subprocess
+    p = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--config", "c3", "--steps", "2", "--warmup", "0",
+                        "--no-cpu-baseline", "--no-extras", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=600)
+    assert p.returncode == 0, p.stderr[-2000:]
+    w = bench.workload("c3", 1)
+    c = bench.host_cube(w)
+    g3 = (c["x_grid"], c["y_grid"], c["z_grid"])
+    session.set_omega_cube(c["omega_pe"], *g3)
+    session.set_field_cubes(*g3, c["ne"], c["te"], c["b"], c["bx"], c["by"], c["bz"])
+    _, _, _, tb, vi, _ = _render_full(session, w, w["freq_params"], bench.pixel_area(w))
+    assert sorted(f.name for f in tmp_path.iterdir()) == ["tb.npy", "vi.npy"]
+    shape = (w["n_freq"], w["n_pix_y"], w["n_pix_x"])
+    np.testing.assert_array_equal(np.load(tmp_path / "tb.npy"), tb.reshape(shape))
+    np.testing.assert_array_equal(np.load(tmp_path / "vi.npy"), vi.reshape(shape))
+
+
 def test_config5_bench_variant_matches_oracle_chain(oracle, session):
     from oracle import parity
     w = bench.workload("c5", 8)

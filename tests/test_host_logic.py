@@ -25,12 +25,13 @@ def test_library_loads_and_exports_every_declared_symbol():
 
 
 def test_sass_is_sm100a_only():
-    import shutil
     import subprocess
     from raytracinggrff_b200 import _lib
-    if shutil.which("cuobjdump") is None:
-        pytest.skip("cuobjdump not on PATH")
-    out = subprocess.run(["cuobjdump", "-lelf", str(_lib.LIB_PATH)], capture_output=True, text=True).stdout
+    from raytracinggrff_b200.build import cuda_tool
+    cuobjdump = cuda_tool("cuobjdump")
+    if not Path(cuobjdump).exists():
+        pytest.skip("cuobjdump not found")
+    out = subprocess.run([cuobjdump, "-lelf", str(_lib.LIB_PATH)], capture_output=True, text=True).stdout
     archs = set(re.findall(r"sm_\d+a?", out))
     assert archs == {"sm_100a"}, archs
 
