@@ -257,6 +257,46 @@ int rtgrff_render_map(rtgrff_ctx *ctx, int64_t n_rays, const double *x_start, co
                       int out_on_device, int64_t *stats);
 
 /*
+ * Map diagnostics: where the emission a pixel sees comes from once refraction has bent the ray.  Planes of
+ * rtgrff_render_map_diag's `diag`, float64 (RTGRFF_N_DIAG, n_freq, n_rays), each plane laid out as tb / vi.
+ * They describe the transfer behind T_b: the exact-coupling I_L, I_R in the voxel_order asked for.
+ *  EM_X, EM_Y, EM_Z  emission centroid [R_sun]: every contribution's position weighted by its share of I_L + I_R at
+ *                    the observer.  Computed exactly with weighted transfers W^c that take every source term b as
+ *                    b c and every operator as I does, EM_c = (W^c_L + W^c_R) / (I_L + I_R): the centroid lies in the
+ *                    convex hull of the path.  A voxel's position is its record position (the float32 x, y, z the
+ *                    sampler uses); a gyroresonance or quasi-transverse layer between two voxels takes the midpoint of
+ *                    the two (the previous non-empty voxel), so the centroid is resolved to the record spacing.
+ *  EM_R              contribution-weighted mean of |p| [R_sun] (not |centroid|): the emission height.
+ *                    EM_* are NaN where I_L + I_R is 0 or not finite.
+ *  TAU_L, TAU_R      total optical depth applied to the L and R slot: kappa ds of every slab, routed to L/R by the
+ *                    sign of cos(theta) like the operator, plus the gyroresonance layers; a quasi-transverse layer adds
+ *                    nothing.  +inf where the mode was evanescent somewhere on the path (its intensity was reset).
+ *  RAY_RMIN          smallest |p| [R_sun] over the ray's records with a finite position: the ray's turning point; NaN
+ *                    if there is none.
+ */
+#define RTGRFF_N_DIAG 7
+#define RTGRFF_DIAG_EM_X 0
+#define RTGRFF_DIAG_EM_Y 1
+#define RTGRFF_DIAG_EM_Z 2
+#define RTGRFF_DIAG_EM_R 3
+#define RTGRFF_DIAG_TAU_L 4
+#define RTGRFF_DIAG_TAU_R 5
+#define RTGRFF_DIAG_RAY_RMIN 6
+
+/*
+ * rtgrff_render_map with the diagnostic planes above: the same arguments and the same tb, vi, stats, plus
+ * diag float64 (RTGRFF_N_DIAG, n_freq, n_rays) (plane stride n_rays as tb / vi), host, or a device pointer when
+ * out_on_device != 0.  diag == NULL is RTGRFF_EINVAL.  With tb, vi and diag consecutive in one device slab, the
+ * 9 n_freq planes go through rtgrff_gather_image in one call.
+ */
+int rtgrff_render_map_diag(rtgrff_ctx *ctx, int64_t n_rays, const double *x_start, const double *y_start,
+                           const double *z_start, const double *kvec, const int32_t *ray_order, int n_freq,
+                           const rtgrff_freq_params *freqs, int trace_cs, double perturb_ratio,
+                           double pixel_area_cm2, double r_sun_cm, int em_flag, int s_max, int use_bvec,
+                           int voxel_order, int s_mode, int s_input_on, double *tb, double *vi,
+                           int out_on_device, int64_t *stats, double *diag);
+
+/*
  * Multi-GPU (one process per GPU, the cube replicated on each).  Rays are independent, so the only exchange
  * is the gather of the image at the end; this replaces the reference's ProcessPoolExecutor ray chunks and
  * their concatenate (script/resample_with_ray_tracing.py:42-61, :333-352, the `--workers` switch).

@@ -39,8 +39,11 @@ EXPORTS = (
     "rtgrff_ctx_create_on_stream", "rtgrff_current_device", "rtgrff_get_mw_slice_device", "rtgrff_memcpy",
     "rtgrff_export_cubes", "rtgrff_shard_rows", "rtgrff_comm_unique_id", "rtgrff_comm_init_rank",
     "rtgrff_comm_destroy", "rtgrff_gather_image", "rtgrff_device_alloc", "rtgrff_device_free",
-    "rtgrff_ctx_set_pipeline", "rtgrff_ctx_set_grff64", "rtgrff_place_rows",
+    "rtgrff_ctx_set_pipeline", "rtgrff_ctx_set_grff64", "rtgrff_place_rows", "rtgrff_render_map_diag",
 )
+
+# planes of rtgrff_render_map_diag's output (RTGRFF_DIAG_* in include/rtgrff.h), in plane order
+DIAG_PLANES = ("em_x", "em_y", "em_z", "em_r", "tau_L", "tau_R", "ray_r_min")
 
 
 class FreqParams(ctypes.Structure):
@@ -107,6 +110,7 @@ def load():
     lib.rtgrff_render_map.argtypes = [c_void_p, c_int64, dp, dp, dp, dp, ip, c_int, POINTER(FreqParams), c_int, c_double,
                                       c_double, c_double, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
                                       c_int, POINTER(c_int64)]
+    lib.rtgrff_render_map_diag.argtypes = lib.rtgrff_render_map.argtypes + [c_void_p]
     lib.rtgrff_gaussian_beam.argtypes = [c_void_p, dp, c_int, c_int, c_int, c_double, c_double, dp]
     lib.rtgrff_patch_nan.argtypes = [c_void_p, dp, c_int, c_int, c_int, c_int, POINTER(c_int64)]
     for name in EXPORTS:

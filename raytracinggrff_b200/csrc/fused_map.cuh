@@ -9,6 +9,8 @@
 // called once per frequency as the publication drivers do (script/pub/TbSpectra_gen.py:155-182).
 // A 2048^2 x 500-record map would need 25 GB of paths per frequency if materialised
 // (SURVEY.md §5); here a record lives in registers for the few hundred cycles it is needed.
+// The DIAG instantiations (rtgrff_render_map_diag) also accumulate where each pixel's emission comes from: emission
+// centroid and height, optical depths, the ray's turning point (DiagAcc below, definitions in include/rtgrff.h).
 #pragma once
 
 #include "grff.cuh"
@@ -59,6 +61,73 @@ struct MapArgs {
     int grff64;                          // 1: every voxel through the FP64 evaluation (RTGRFF_GRFF64=1, A/B and validation)
     double *tb, *vi;                     // [freq][ray]
     unsigned long long *active_steps;    // [0] active central steps, [1] steps with the pencil traced, [2] valid samples
+    double *diag;                        // [RTGRFF_N_DIAG][freq][ray], the DIAG variants only
+    int64_t diag_plane;                  // elements from one diagnostic plane to the next: n_freq * n_rays
+};
+
+// ---- map diagnostics (the DIAG variants; planes and definitions in include/rtgrff.h) ----
+// Next to the transfer I four weighted transfers W^c run, c = x, y, z, |p|: every source term b enters them as
+// b c, c the coordinate of the event it belongs to, and every operator acts on W as on I (slab a W + b c, the same
+// L/R mixing at a quasi-transverse layer, acc += M b c in the outward fold).  W^c / I is then the exact
+// contribution-weighted mean of c.  A voxel's coordinate is its record position (the float32 x, y, z the sampler
+// used); an event between two voxels takes the midpoint of the two, so the centroid is resolved to the record
+// spacing.  The optical depths kappa ds of the slabs and gyroresonance layers are summed per slot.
+__device__ __forceinline__ float4 diag_coord(float x, float y, float z)
+{
+    return make_float4(x, y, z, sqrtf(fmaf(x, x, fmaf(y, y, z * z))));
+}
+
+__device__ __forceinline__ float4 diag_mid(const float4 &p, const float4 &q)
+{
+    return make_float4(0.5f * (p.x + q.x), 0.5f * (p.y + q.y), 0.5f * (p.z + q.z), 0.5f * (p.w + q.w));
+}
+
+struct DiagAcc {
+    double wL[4], wR[4];
+    double tauL, tauR;
+    float4 prev;          // coordinate of the previous non-empty voxel the transfer keeps
+    __device__ __forceinline__ void init()
+    {
+#pragma unroll
+        for (int q = 0; q < 4; ++q) { wL[q] = 0.0; wR[q] = 0.0; }
+        tauL = tauR = 0.0;
+    }
+    __device__ __forceinline__ void add_tau(double tl, double tr) { tauL += tl; tauR += tr; }
+    // record order: W <- a W + b c
+    __device__ __forceinline__ void apply(const DiagOp &d, const float4 &c)
+    {
+        const double cc[4] = {(double)c.x, (double)c.y, (double)c.z, (double)c.w};
+#pragma unroll
+        for (int q = 0; q < 4; ++q) { wL[q] = fma(wL[q], d.aL, d.bL * cc[q]); wR[q] = fma(wR[q], d.aR, d.bR * cc[q]); }
+    }
+    __device__ __forceinline__ void qt(double Q)
+    {
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+            const double l = wL[q], r = wR[q];
+            wL[q] = Q * l + (1.0 - Q) * r;
+            wR[q] = Q * r + (1.0 - Q) * l;
+        }
+    }
+    // outward order: W_acc += (M b) c, before M takes the operator
+    __device__ __forceinline__ void fold(double m00, double m01, double m10, double m11, const DiagOp &d, const float4 &c)
+    {
+        const double pL = m00 * d.bL + m01 * d.bR, pR = m10 * d.bL + m11 * d.bR;
+        const double cc[4] = {(double)c.x, (double)c.y, (double)c.z, (double)c.w};
+#pragma unroll
+        for (int q = 0; q < 4; ++q) { wL[q] = fma(pL, cc[q], wL[q]); wR[q] = fma(pR, cc[q], wR[q]); }
+    }
+    // the seven planes of one (pixel, frequency) from the exact-coupling I_L, I_R and the ray's smallest |p|
+    __device__ __forceinline__ void write(double IL, double IR, float rmin, double *out, size_t plane) const
+    {
+        const double I = IL + IR;
+        const bool ok = I != 0.0 && isfinite(I);
+#pragma unroll
+        for (int q = 0; q < 4; ++q) out[(size_t)(RTGRFF_DIAG_EM_X + q) * plane] = ok ? (wL[q] + wR[q]) / I : (double)NAN;
+        out[(size_t)RTGRFF_DIAG_TAU_L * plane] = tauL;
+        out[(size_t)RTGRFF_DIAG_TAU_R * plane] = tauR;
+        out[(size_t)RTGRFF_DIAG_RAY_RMIN * plane] = rmin < INFINITY ? (double)rmin : (double)NAN;
+    }
 };
 
 // Transfer accumulated from the observer outwards (RTGRFF_ORDER_REVERSED): the records arrive
@@ -91,54 +160,110 @@ struct OutwardTransfer {
 // the between-voxel events; with the reference's packing (theta = 90, GR off) it is dead weight.
 // A voxel arrives as the float32 values the sampler produced (VoxLite + sin theta); its slab operator is
 // evaluated in float32 where that is well conditioned (voxel_op_mixed), the intensities live in FP64.
-template <bool NEED_BETWEEN>
+// DIAG: the diagnostics' accumulators (DiagAcc) run alongside; (x, y, z) is the record position of the voxel.
+template <bool NEED_BETWEEN, bool DIAG = false>
 struct RecordTransfer {
     PolState<1> st;
     VoxLite prev;
     bool have_prev;
-    __device__ __forceinline__ void init() { st.clear(); have_prev = false; }
-    __device__ __forceinline__ void push(const FreqC &f, const VoxLite &l, float sth, int flag, int smax, bool force64)
+    DiagAcc dg;
+    __device__ __forceinline__ void init()
+    {
+        st.clear(); have_prev = false;
+        if constexpr (DIAG) dg.init();
+    }
+    __device__ __forceinline__ void push(const FreqC &f, const VoxLite &l, float sth, int flag, int smax, bool force64,
+                                         float x, float y, float z)
     {
         if (!voxel_nonempty_f(l.dz, l.T, l.ne, l.B, l.cth)) { have_prev = false; return; }
+        float4 c;
+        if constexpr (DIAG) c = diag_coord(x, y, z);
         if (NEED_BETWEEN) {
             if (have_prev && prev.B > 0.0f && l.B > 0.0f && between_needed_f(f, prev.cth, prev.B, l.cth, l.B, smax, !(flag & 1)))
             {
                 Between b;
                 between_voxels_cold(f.nu, f.sn, prev, l, flag, smax, &b);
+                if constexpr (DIAG) {
+                    const double2 t = between_tau_cold(f.nu, f.sn, prev, l, flag, smax);
+                    dg.add_tau(t.x, t.y);
+                    const float4 m = diag_mid(dg.prev, c);
+                    dg.apply(b.before, m);
+                    if (b.qt) dg.qt(b.Q);
+                    dg.apply(b.after, m);
+                }
                 st.apply(b);
             }
             prev = l;
             have_prev = true;
+            if constexpr (DIAG) dg.prev = c;
         }
-        st.apply(voxel_op_mixed(f, l.dz, l.T, l.ne, l.B, l.cth, sth, l.scale, flag, smax, force64));
+        if constexpr (DIAG) {
+            const TauOp o = voxel_op_mixed_tau(f, l.dz, l.T, l.ne, l.B, l.cth, sth, l.scale, flag, smax, force64);
+            dg.add_tau(o.tauL, o.tauR);
+            dg.apply(o.op, c);
+            st.apply(o.op);
+        } else {
+            st.apply(voxel_op_mixed(f, l.dz, l.T, l.ne, l.B, l.cth, sth, l.scale, flag, smax, force64));
+        }
     }
     __device__ __forceinline__ void result(double &L, double &R) const { L = st.L[0]; R = st.R[0]; }
 };
 
-template <bool NEED_BETWEEN>
+template <bool NEED_BETWEEN, bool DIAG = false>
 struct OutwardTransferT : OutwardTransfer {
-    __device__ __forceinline__ void push(const FreqC &f, const VoxLite &l, float sth, int flag, int smax, bool force64)
+    DiagAcc dg;
+    __device__ __forceinline__ void init()
+    {
+        OutwardTransfer::init();
+        if constexpr (DIAG) dg.init();
+    }
+    __device__ __forceinline__ void fold_diag(const DiagOp &d, const float4 &c)
+    {
+        dg.fold(m00, m01, m10, m11, d, c);
+        fold(d);
+    }
+    __device__ __forceinline__ void push(const FreqC &f, const VoxLite &l, float sth, int flag, int smax, bool force64,
+                                         float x, float y, float z)
     {
         if (!voxel_nonempty_f(l.dz, l.T, l.ne, l.B, l.cth)) { have_prev = false; return; }
+        float4 c;
+        if constexpr (DIAG) c = diag_coord(x, y, z);
         if (NEED_BETWEEN) {
             if (have_prev && prev.B > 0.0f && l.B > 0.0f && between_needed_f(f, l.cth, l.B, prev.cth, prev.B, smax, !(flag & 1))) {
                 // radiation crosses v -> prev: between_voxels(v, prev) lists the events in that order,
                 // folding outwards meets them last-first
                 Between b;
                 between_voxels_cold(f.nu, f.sn, l, prev, flag, smax, &b);
-                fold(b.after);
-                if (b.qt) fold_qt(b.Q);
-                fold(b.before);
+                if constexpr (DIAG) {
+                    const double2 t = between_tau_cold(f.nu, f.sn, l, prev, flag, smax);
+                    dg.add_tau(t.x, t.y);
+                    const float4 m = diag_mid(dg.prev, c);
+                    fold_diag(b.after, m);
+                    if (b.qt) fold_qt(b.Q);
+                    fold_diag(b.before, m);
+                } else {
+                    fold(b.after);
+                    if (b.qt) fold_qt(b.Q);
+                    fold(b.before);
+                }
             }
             prev = l;
             have_prev = true;
+            if constexpr (DIAG) dg.prev = c;
         }
-        fold(voxel_op_mixed(f, l.dz, l.T, l.ne, l.B, l.cth, sth, l.scale, flag, smax, force64));
+        if constexpr (DIAG) {
+            const TauOp o = voxel_op_mixed_tau(f, l.dz, l.T, l.ne, l.B, l.cth, sth, l.scale, flag, smax, force64);
+            dg.add_tau(o.tauL, o.tauR);
+            fold_diag(o.op, c);
+        } else {
+            fold(voxel_op_mixed(f, l.dz, l.T, l.ne, l.B, l.cth, sth, l.scale, flag, smax, force64));
+        }
     }
     __device__ __forceinline__ void result(double &L, double &R) const { L = accL; R = accR; }
 };
 
-template <bool CS, int ORDER, bool BVEC, bool GR, int MODE>
+// DIAG: also write the diagnostic planes to a.diag (tb / vi are the same as without)
+template <bool CS, int ORDER, bool BVEC, bool GR, int MODE, bool DIAG>
 __global__ void __launch_bounds__(RT_BLOCK, RT_MINB) render_map_kernel(const MapArgs a)
 {
     constexpr bool NEED_BETWEEN = BVEC || GR;
@@ -176,9 +301,10 @@ __global__ void __launch_bounds__(RT_BLOCK, RT_MINB) render_map_kernel(const Map
     int next_rec = 0;
     int death = -1;                       // step at which the ray froze (-1: still moving)
 
-    typename std::conditional<ORDER == RTGRFF_ORDER_RECORD, RecordTransfer<NEED_BETWEEN>,
-                              OutwardTransferT<NEED_BETWEEN>>::type tr;
+    typename std::conditional<ORDER == RTGRFF_ORDER_RECORD, RecordTransfer<NEED_BETWEEN, DIAG>,
+                              OutwardTransferT<NEED_BETWEEN, DIAG>>::type tr;
     tr.init();
+    float rmin = INFINITY;                // DIAG: smallest |p| over the records with a finite position
     bool first = true;
     bool tail_done = !has_ray;            // a frozen ray repeats the same record: ds = 0 -> empty voxel
 
@@ -218,6 +344,7 @@ __global__ void __launch_bounds__(RT_BLOCK, RT_MINB) render_map_kernel(const Map
             if (!tail_done) {
                 // --- sampler (float32, gpu_raytrace.py:642-650) ---
                 const float x = (float)s.rx, y = (float)s.ry, z = (float)s.rz, sv = cumulative ? (float)s_cum : s_step;
+                if (DIAG && isfinite(x) && isfinite(y) && isfinite(z)) rmin = fminf(rmin, diag_coord(x, y, z).w);
                 if (sample_valid(x, y, z, sv)) {
                     ++n_samples;
                     float3 bv = make_float3(0.f, 0.f, 0.f);
@@ -246,7 +373,7 @@ __global__ void __launch_bounds__(RT_BLOCK, RT_MINB) render_map_kernel(const Map
                     if (isfinite(f.ne) && isfinite(f.te) && isfinite(f.b)) {
                         // Parms[14] = S * area (script/resample_with_ray_tracing.py:501): source factor S
                         const VoxLite lite = {ds, f.te, f.ne, f.b, cthf, a.s_input ? sv : 1.0f};
-                        tr.push(fq, lite, sthf, a.em_flag, a.s_max, a.grff64 != 0);
+                        tr.push(fq, lite, sthf, a.em_flag, a.s_max, a.grff64 != 0, x, y, z);
                     }
                     px = x; py = y; pz = z;
                     first = false;
@@ -265,6 +392,7 @@ __global__ void __launch_bounds__(RT_BLOCK, RT_MINB) render_map_kernel(const Map
         tb_vi(IL, IR, fp.nu, a.area, tb, vi);
         a.tb[(size_t)fp.out_row * a.n_rays + ray] = tb;
         a.vi[(size_t)fp.out_row * a.n_rays + ray] = vi;
+        if constexpr (DIAG) tr.dg.write(IL, IR, rmin, a.diag + (size_t)fp.out_row * a.n_rays + ray, (size_t)a.diag_plane);
     }
     if (a.active_steps) {
         // a ray moves on steps [0, death): the counters follow from where it froze

@@ -189,8 +189,10 @@ __host__ __device__ __forceinline__ FreqC make_freq(double nu)
 // are evaluated once).
 // FAST_T (the per-ray kernels, tolerance 1e-4 on T_b): ln T and T^-1.5 in FP32.  The kernel behind the
 // PyGET_MW / get_mw_slice ABIs keeps them FP64 (agrees with the oracle to 1e-14).
-template <bool FAST_T>
-__device__ __forceinline__ DiagOp voxel_op(const FreqC &f, const Voxel &v)
+// TAU: also write the optical depth kappa dz of the L and R slot to tau[0], tau[1] (+inf where the mode is
+// evanescent), for the map diagnostics; the TAU = false instantiation is the plain evaluation.
+template <bool FAST_T, bool TAU = false>
+__device__ __forceinline__ DiagOp voxel_op(const FreqC &f, const Voxel &v, double *tau = nullptr)
 {
     const double nuB = kNuB * v.B;
     const double u = nuB * nuB * f.inv_nu2, vv = kNup2 * v.ne * f.inv_nu2;
@@ -213,6 +215,7 @@ __device__ __forceinline__ DiagOp voxel_op(const FreqC &f, const Voxel &v)
     }
     const double srcb = f.nu2 * kKbC2 * v.T * v.scale;
     double aX = 0.0, bX = 0.0, aO = 0.0, bO = 0.0;
+    double tX = INFINITY, tO = INFINITY;
     if (u > 0.0) {
         const double s2 = v.sth * v.sth, c2 = v.cth * v.cth;
         const double us2 = u * s2;
@@ -241,6 +244,7 @@ __device__ __forceinline__ DiagOp voxel_op(const FreqC &f, const Voxel &v)
             if (n2 > 0.0 && isfinite(n2) && isfinite(F)) {
                 double kap = pref * F * rsqrt(n2);
                 if (!(kap > 0.0) || !isfinite(kap)) kap = 0.0;
+                if constexpr (TAU) tX = kap * v.dz;
                 slab_ab(true, kap * v.dz, n2 * srcb, aX, bX);
             }
         }
@@ -250,6 +254,7 @@ __device__ __forceinline__ DiagOp voxel_op(const FreqC &f, const Voxel &v)
             if (n2 > 0.0 && isfinite(n2) && isfinite(F)) {
                 double kap = pref * F * rsqrt(n2);
                 if (!(kap > 0.0) || !isfinite(kap)) kap = 0.0;
+                if constexpr (TAU) tO = kap * v.dz;
                 slab_ab(true, kap * v.dz, n2 * srcb, aO, bO);
             }
         }
@@ -257,8 +262,13 @@ __device__ __forceinline__ DiagOp voxel_op(const FreqC &f, const Voxel &v)
         // B = 0: one refractive index, unpolarised
         double kap = pref * rsqrt(omv);
         if (!(kap > 0.0) || !isfinite(kap)) kap = 0.0;
+        if constexpr (TAU) tX = tO = kap * v.dz;
         slab_ab(true, kap * v.dz, omv * srcb, aX, bX);
         aO = aX; bO = bX;
+    }
+    if constexpr (TAU) {
+        tau[0] = (v.cth >= 0.0) ? tO : tX;
+        tau[1] = (v.cth >= 0.0) ? tX : tO;
     }
     // X is R where cos(theta) >= 0
     return (v.cth >= 0.0) ? DiagOp{aO, aX, bO, bX} : DiagOp{aX, aO, bX, bO};
@@ -297,14 +307,54 @@ __device__ __forceinline__ DiagOp voxel_op_mixed(const FreqC &f, float dz, float
     return voxel_op_slow(f.nu2, f.inv_nu2, f.ln_nu, f.kff, dz, T, ne, B, cth, sth, scale, flag, smax);
 }
 
+// An operator with the optical depth kappa dz it applies to the L and R slot (+inf: evanescent mode): what the
+// map diagnostics need of each voxel and gyroresonance layer.  Returned by value from the out-of-line
+// evaluations, so that the hot loop keeps it in registers.
+struct TauOp {
+    DiagOp op;
+    double tauL, tauR;
+};
+
+// The slots' optical depths of voxel_op_slow's evaluation.  A function of its own, next to voxel_op_slow rather
+// than folded into a copy of it: the diagnostic kernels take the operator from the very code the plain kernels
+// run, so their T_b stays the plain T_b bit for bit.
+__device__ __noinline__ double2 voxel_tau_slow(double nu2, double inv_nu2, double ln_nu, double kff, float dz, float T,
+                                               float ne, float B, float cth, float sth, float scale, int flag, int smax)
+{
+    FreqC f;
+    f.nu2 = nu2; f.inv_nu2 = inv_nu2; f.ln_nu = ln_nu; f.kff = kff;
+    Voxel v = make_voxel_f(dz, T, ne, B, (double)cth, (double)sth, flag, smax);
+    v.scale = (double)scale;
+    double t[2];
+    voxel_op<true, true>(f, v, t);
+    return make_double2(t[0], t[1]);
+}
+
+// voxel_op_mixed with the optical depths, taken from whichever evaluation produced the operator (never as
+// -log a: in float32 a thin voxel's a rounds to 1)
+__device__ __forceinline__ TauOp voxel_op_mixed_tau(const FreqC &f, float dz, float T, float ne, float B, float cth,
+                                                    float sth, float scale, int flag, int smax, bool force64)
+{
+    if (!force64) {
+        const FastOp o = voxel_op_f32(f.ff, dz, T, ne, B, cth, sth, scale, !(flag & 2));
+        if (o.ok) return TauOp{DiagOp{(double)o.aL, (double)o.aR, (double)o.bL, (double)o.bR}, (double)o.tauL, (double)o.tauR};
+    }
+    const DiagOp op = voxel_op_slow(f.nu2, f.inv_nu2, f.ln_nu, f.kff, dz, T, ne, B, cth, sth, scale, flag, smax);
+    const double2 t = voxel_tau_slow(f.nu2, f.inv_nu2, f.ln_nu, f.kff, dz, T, ne, B, cth, sth, scale, flag, smax);
+    return TauOp{op, t.x, t.y};
+}
+
 // One gyroresonance layer nu = s nu_B at interpolated plasma parameters.  Rare and heavy (lgamma,
-// log, exp, sincos): kept out of line so the hot loops stay small.
-__device__ __noinline__ DiagOp gr_layer_op(double nu, int s, double ne, double T, double th, double LB, double scale)
+// log, exp, sincos): kept out of line (gr_layer_op, gr_layer_op_tau) so the hot loops stay small.
+// TAU: tau[0], tau[1] receive the layer's optical depth on the L and R slot (+inf: evanescent mode).
+template <bool TAU>
+__device__ __forceinline__ DiagOp gr_layer_eval(double nu, int s, double ne, double T, double th, double LB, double scale,
+                                                double *tau)
 {
     double sth, cth;
     sincos(th, &sth, &cth);
     const double Bres = kBres * nu / (double)s;
-    double a[2], b[2];
+    double a[2], b[2], t[2];
 #pragma unroll
     for (int q = 0; q < 2; ++q) {
         const int sg = q == 0 ? -1 : 1;
@@ -318,9 +368,28 @@ __device__ __noinline__ DiagOp gr_layer_op(double nu, int s, double ne, double T
             tau = kGrPref * ne * LB / nu * exp(lg) * pol * pol / (1.0 + Ts * Ts);
             if (!(tau > 0.0) || !isfinite(tau)) tau = 0.0;
         }
+        if constexpr (TAU) t[q] = m.prop ? tau : INFINITY;
         slab_ab(m.prop, tau, m.src * scale, a[q], b[q]);
     }
+    if constexpr (TAU) {
+        tau[0] = (cth >= 0.0) ? t[1] : t[0];
+        tau[1] = (cth >= 0.0) ? t[0] : t[1];
+    }
     return (cth >= 0.0) ? DiagOp{a[1], a[0], b[1], b[0]} : DiagOp{a[0], a[1], b[0], b[1]};
+}
+
+__device__ __noinline__ DiagOp gr_layer_op(double nu, int s, double ne, double T, double th, double LB, double scale)
+{
+    return gr_layer_eval<false>(nu, s, ne, T, th, LB, scale, nullptr);
+}
+
+__device__ __noinline__ TauOp gr_layer_op_tau(double nu, int s, double ne, double T, double th, double LB, double scale)
+{
+    TauOp r;
+    double t[2];
+    r.op = gr_layer_eval<true>(nu, s, ne, T, th, LB, scale, t);
+    r.tauL = t[0]; r.tauR = t[1];
+    return r;
 }
 
 // Everything that happens between the centres of two consecutive non-empty voxels p -> k:
@@ -351,7 +420,10 @@ __device__ __forceinline__ bool between_needed_f(const FreqC &f, float p_cth, fl
     return qt || gr;
 }
 
-__device__ __forceinline__ Between between_voxels(const FreqC &f, const Voxel &p, const Voxel &k)
+// TAU: tau[0], tau[1] accumulate the optical depth of the gyroresonance layers on the L and R slot (a
+// quasi-transverse layer adds none); the TAU = false instantiation is the plain event list.
+template <bool TAU = false>
+__device__ __forceinline__ Between between_voxels(const FreqC &f, const Voxel &p, const Voxel &k, double *tau = nullptr)
 {
     Between o;
     o.before = diag_identity(); o.after = diag_identity(); o.Q = 1.0;
@@ -384,9 +456,18 @@ __device__ __forceinline__ Between between_voxels(const FreqC &f, const Voxel &p
             const double Bres = sn / (double)s;
             if (!((p.B - Bres) * (k.B - Bres) < 0.0)) continue;
             const double t = (Bres - p.B) / (k.B - p.B);
-            const DiagOp g = gr_layer_op(nu, s, p.ne + t * (k.ne - p.ne), p.T + t * (k.T - p.T),
-                                         th_p + t * (th_k - th_p), Bres * dzm / fabs(k.B - p.B),
-                                         p.scale + t * (k.scale - p.scale));
+            DiagOp g;
+            if constexpr (TAU) {
+                const TauOp tg = gr_layer_op_tau(nu, s, p.ne + t * (k.ne - p.ne), p.T + t * (k.T - p.T),
+                                                 th_p + t * (th_k - th_p), Bres * dzm / fabs(k.B - p.B),
+                                                 p.scale + t * (k.scale - p.scale));
+                g = tg.op;
+                tau[0] += tg.tauL; tau[1] += tg.tauR;
+            } else {
+                g = gr_layer_op(nu, s, p.ne + t * (k.ne - p.ne), p.T + t * (k.T - p.T),
+                                th_p + t * (th_k - th_p), Bres * dzm / fabs(k.B - p.B),
+                                p.scale + t * (k.scale - p.scale));
+            }
             if (t >= tqt) o.after = diag_then(o.after, g);
             else o.before = diag_then(o.before, g);
         }
@@ -416,6 +497,17 @@ __device__ __noinline__ void between_voxels_cold(double nu, double sn, VoxLite p
     FreqC f;
     f.nu = nu; f.sn = sn;
     *out = between_voxels(f, voxel_of(p, flag, smax), voxel_of(k, flag, smax));
+}
+
+// The optical depth of between_voxels_cold's gyroresonance layers on the L and R slot (the map diagnostics).  The
+// diagnostic kernels take the events themselves from between_voxels_cold, the code the plain kernels run.
+__device__ __noinline__ double2 between_tau_cold(double nu, double sn, VoxLite p, VoxLite k, int flag, int smax)
+{
+    FreqC f;
+    f.nu = nu; f.sn = sn;
+    double t[2] = {0.0, 0.0};
+    between_voxels<true>(f, voxel_of(p, flag, smax), voxel_of(k, flag, smax), t);
+    return make_double2(t[0], t[1]);
 }
 
 // Polarisation state for the three mode-coupling variants GRFF reports:

@@ -67,6 +67,8 @@ constexpr float kFastGuard = 0.02f;
 struct FastOp {
     float aL, aR, bL, bR;
     bool ok;               // false: ill-conditioned or non-finite -> evaluate this voxel in FP64
+    float tauL, tauR;      // optical depth kappa dz of the slot (+inf: evanescent); read by the map diagnostics
+                           // only, dead code for every other caller
 };
 
 // 1 - e^-tau and e^-tau of a slab
@@ -90,7 +92,7 @@ RTF_HD FastOp voxel_op_f32(const FreqCF &f, float dz, float T, float ne, float B
                            bool ff_on)
 {
     FastOp o;
-    o.aL = o.aR = 1.0f; o.bL = o.bR = 0.0f; o.ok = true;
+    o.aL = o.aR = 1.0f; o.bL = o.bR = 0.0f; o.ok = true; o.tauL = o.tauR = 0.0f;
     // v and w = 1 - v: the product error of cv_hi * ne is recovered exactly with an FMA, 1 - v_hi is exact
     // for v_hi in [0.5, 2]
     const float v = f.cv_hi * ne;
@@ -111,6 +113,7 @@ RTF_HD FastOp voxel_op_f32(const FreqCF &f, float dz, float T, float ne, float B
     }
     const float srcb = f.srcc * T * scale;
     float aX = 0.0f, bX = 0.0f, aO = 0.0f, bO = 0.0f;
+    float tX = INFINITY, tO = INFINITY;
     if (B > 0.0f) {
         const float su = f.c_su * B, u = su * su;
         const float s2 = sth * sth, c2 = cth * cth;
@@ -138,7 +141,8 @@ RTF_HD FastOp voxel_op_f32(const FreqCF &f, float dz, float T, float ne, float B
         {
             float kap = pref * FO * RTF_RSQRT(n2O);
             if (!(kap > 0.0f) || !(kap < INFINITY)) kap = 0.0f;
-            slab_f32(kap * dz, n2O * srcb, aO, bO);
+            tO = kap * dz;
+            slab_f32(tO, n2O * srcb, aO, bO);
         }
         if (x_on) {
             // towards the gyro-resonance (nu -> nu_B) d_X = 2w - su (q + A) is a small difference of O(1) terms and
@@ -149,18 +153,20 @@ RTF_HD FastOp voxel_op_f32(const FreqCF &f, float dz, float T, float ne, float B
             if (!(n2X >= kFastGuard) || !(FX < INFINITY)) { o.ok = false; return o; }
             float kap = pref * FX * RTF_RSQRT(n2X);
             if (!(kap > 0.0f) || !(kap < INFINITY)) kap = 0.0f;
-            slab_f32(kap * dz, n2X * srcb, aX, bX);
+            tX = kap * dz;
+            slab_f32(tX, n2X * srcb, aX, bX);
         }
     } else {
         // B = 0: one refractive index n^2 = w, unpolarised
         float kap = pref * RTF_RSQRT(w);
         if (!(kap > 0.0f) || !(kap < INFINITY)) kap = 0.0f;
-        slab_f32(kap * dz, w * srcb, aX, bX);
-        aO = aX; bO = bX;
+        tX = kap * dz;
+        slab_f32(tX, w * srcb, aX, bX);
+        aO = aX; bO = bX; tO = tX;
     }
     // X is R where cos(theta) >= 0
-    if (cth >= 0.0f) { o.aL = aO; o.aR = aX; o.bL = bO; o.bR = bX; }
-    else { o.aL = aX; o.aR = aO; o.bL = bX; o.bR = bO; }
+    if (cth >= 0.0f) { o.aL = aO; o.aR = aX; o.bL = bO; o.bR = bX; o.tauL = tO; o.tauR = tX; }
+    else { o.aL = aX; o.aR = aO; o.bL = bX; o.bR = bO; o.tauL = tX; o.tauR = tO; }
     o.ok = (o.bL == o.bL) && (o.bR == o.bR) && (o.aL == o.aL) && (o.aR == o.aR);
     return o;
 }

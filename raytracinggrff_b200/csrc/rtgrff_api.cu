@@ -1159,12 +1159,13 @@ int rtgrff_emission_traced(rtgrff_ctx *c, double pixel_area_cm2, double freq0_hz
     return RTGRFF_OK;
 }
 
-int rtgrff_render_map(rtgrff_ctx *c, int64_t n_rays, const double *x_start, const double *y_start,
-                      const double *z_start, const double *kvec, const int32_t *ray_order, int n_freq,
-                      const rtgrff_freq_params *freqs,
-                      int trace_cs, double perturb_ratio, double pixel_area_cm2, double r_sun_cm, int em_flag, int s_max,
-                      int use_bvec, int voxel_order, int s_mode, int s_input_on, double *tb, double *vi, int out_on_device,
-                      int64_t *stats)
+// rtgrff_render_map and rtgrff_render_map_diag: diag == nullptr launches the plain kernels, else the DIAG ones
+static int render_map_impl(rtgrff_ctx *c, int64_t n_rays, const double *x_start, const double *y_start,
+                           const double *z_start, const double *kvec, const int32_t *ray_order, int n_freq,
+                           const rtgrff_freq_params *freqs,
+                           int trace_cs, double perturb_ratio, double pixel_area_cm2, double r_sun_cm, int em_flag, int s_max,
+                           int use_bvec, int voxel_order, int s_mode, int s_input_on, double *tb, double *vi, int out_on_device,
+                           int64_t *stats, double *diag)
 {
     RT_USE(c);
     if (!c->has_wcube) return fail(RTGRFF_ENOCUBE, "rtgrff_set_omega_cube has not been called");
@@ -1214,11 +1215,15 @@ int rtgrff_render_map(rtgrff_ctx *c, int64_t n_rays, const double *x_start, cons
     }
     RT_TRY(c->counters.reserve(64));
     RT_CUDA(cudaMemsetAsync(c->counters.p, 0, 64, c->stream));
-    double *dtb = tb, *dvi = vi;
+    double *dtb = tb, *dvi = vi, *ddiag = diag;
     if (!out_on_device) {
         RT_TRY(c->out0.reserve((size_t)n_freq * nb));
         RT_TRY(c->out1.reserve((size_t)n_freq * nb));
         dtb = c->out0.as<double>(); dvi = c->out1.as<double>();
+        if (diag) {
+            RT_TRY(c->out3.reserve((size_t)RTGRFF_N_DIAG * n_freq * nb));
+            ddiag = c->out3.as<double>();
+        }
     }
     MapArgs a;
     a.cube = rc;
@@ -1237,17 +1242,21 @@ int rtgrff_render_map(rtgrff_ctx *c, int64_t n_rays, const double *x_start, cons
     a.grff64 = c->grff64;
     a.tb = dtb; a.vi = dvi;
     a.active_steps = c->counters.as<unsigned long long>();
+    a.diag = ddiag;
+    a.diag_plane = (int64_t)n_freq * n_rays;     // planes follow the caller's frequency order: FreqDev::out_row
     const dim3 block(RT_BLOCK);
     const bool gr = !(em_flag & 1);
     RT_CUDA(cudaEventRecord(c->ev0, c->stream));
     const int variant = (trace_cs ? 8 : 0) | (voxel_order == RTGRFF_ORDER_REVERSED ? 4 : 0) | (use_bvec ? 2 : 0) | (gr ? 1 : 0);
-#define RT_MAP_CASE(v, CS, ORD, BV, GR)                                                                  \
-    case v:                                                                                              \
-        if (mode == MODE_FAST32) {                                                                       \
-            if (carve >= 0) cudaFuncSetAttribute(render_map_kernel<CS, ORD, BV, GR, MODE_FAST32>,        \
-                                                 cudaFuncAttributePreferredSharedMemoryCarveout, carve);  \
-            render_map_kernel<CS, ORD, BV, GR, MODE_FAST32><<<grid, block, 0, c->stream>>>(a);           \
-        } else render_map_kernel<CS, ORD, BV, GR, MODE_F64><<<grid, block, 0, c->stream>>>(a);           \
+#define RT_MAP_LAUNCH(CS, ORD, BV, GR, DG)                                                                   \
+        if (mode == MODE_FAST32) {                                                                           \
+            if (carve >= 0) cudaFuncSetAttribute(render_map_kernel<CS, ORD, BV, GR, MODE_FAST32, DG>,        \
+                                                 cudaFuncAttributePreferredSharedMemoryCarveout, carve);      \
+            render_map_kernel<CS, ORD, BV, GR, MODE_FAST32, DG><<<grid, block, 0, c->stream>>>(a);           \
+        } else render_map_kernel<CS, ORD, BV, GR, MODE_F64, DG><<<grid, block, 0, c->stream>>>(a);
+#define RT_MAP_CASE(v, CS, ORD, BV, GR)                                                                      \
+    case v:                                                                                                  \
+        if (diag) { RT_MAP_LAUNCH(CS, ORD, BV, GR, true) } else { RT_MAP_LAUNCH(CS, ORD, BV, GR, false) }    \
         break;
     int mode = trace_variant() == 0 ? MODE_FAST32 : MODE_F64;
     // RTGRFF_CARVEOUT=<percent>: preferred shared-memory carve-out of the per-ray kernels (A/B switch; they use no
@@ -1306,17 +1315,44 @@ int rtgrff_render_map(rtgrff_ctx *c, int64_t n_rays, const double *x_start, cons
         }
     }
 #undef RT_MAP_CASE
+#undef RT_MAP_LAUNCH
     RT_CUDA(cudaEventRecord(c->ev1, c->stream));
     c->ev_valid = true;
     if (!out_on_device) {
         RT_TRY(d2h(c, tb, dtb, (size_t)n_freq * nb));
         RT_TRY(d2h(c, vi, dvi, (size_t)n_freq * nb));
+        if (diag) RT_TRY(d2h(c, diag, ddiag, (size_t)RTGRFF_N_DIAG * n_freq * nb));
     }
     unsigned long long act[3] = {0, 0, 0};
     RT_TRY(d2h(c, act, c->counters.p, sizeof(act)));
     RT_CUDA(cudaStreamSynchronize(c->stream));
     if (stats) { stats[0] = nominal; stats[1] = (int64_t)act[0]; stats[2] = (int64_t)act[1]; stats[3] = (int64_t)act[2]; }
     return RTGRFF_OK;
+}
+
+int rtgrff_render_map(rtgrff_ctx *c, int64_t n_rays, const double *x_start, const double *y_start,
+                      const double *z_start, const double *kvec, const int32_t *ray_order, int n_freq,
+                      const rtgrff_freq_params *freqs,
+                      int trace_cs, double perturb_ratio, double pixel_area_cm2, double r_sun_cm, int em_flag, int s_max,
+                      int use_bvec, int voxel_order, int s_mode, int s_input_on, double *tb, double *vi, int out_on_device,
+                      int64_t *stats)
+{
+    return render_map_impl(c, n_rays, x_start, y_start, z_start, kvec, ray_order, n_freq, freqs, trace_cs, perturb_ratio,
+                           pixel_area_cm2, r_sun_cm, em_flag, s_max, use_bvec, voxel_order, s_mode, s_input_on, tb, vi,
+                           out_on_device, stats, nullptr);
+}
+
+int rtgrff_render_map_diag(rtgrff_ctx *c, int64_t n_rays, const double *x_start, const double *y_start,
+                           const double *z_start, const double *kvec, const int32_t *ray_order, int n_freq,
+                           const rtgrff_freq_params *freqs,
+                           int trace_cs, double perturb_ratio, double pixel_area_cm2, double r_sun_cm, int em_flag,
+                           int s_max, int use_bvec, int voxel_order, int s_mode, int s_input_on, double *tb, double *vi,
+                           int out_on_device, int64_t *stats, double *diag)
+{
+    if (!diag) return fail(RTGRFF_EINVAL, "rtgrff_render_map_diag needs the diag output");
+    return render_map_impl(c, n_rays, x_start, y_start, z_start, kvec, ray_order, n_freq, freqs, trace_cs, perturb_ratio,
+                           pixel_area_cm2, r_sun_cm, em_flag, s_max, use_bvec, voxel_order, s_mode, s_input_on, tb, vi,
+                           out_on_device, stats, diag);
 }
 
 // ---- multi-GPU: row sharding + image gather ---------------------------------------------------------

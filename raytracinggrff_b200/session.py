@@ -346,6 +346,28 @@ class RaySession:
         patch (-11 % on config 4); results keep the caller's ray numbering.
         s_mode 'per_step' | 'cumulative': the cross-section ratio a record carries (reference CPU / CUDA
         path); s_input_on: that S multiplies the voxel's source term (``--s-input-on``, see include/rtgrff.h)."""
+        return self._render(False, x_start, y_start, z_start, freq_params, kvec_in_norm, trace_crosssections,
+                            perturb_ratio, pixel_area_cm2, r_sun_cm, em_flag, s_max, use_bvec, voxel_order,
+                            out_device_ptrs, image_shape, tile, ray_order, s_mode, s_input_on)
+
+    def render_map_diag(self, x_start, y_start, z_start, freq_params, kvec_in_norm=None, trace_crosssections=True,
+                        perturb_ratio=2.0, pixel_area_cm2=1.0, r_sun_cm=6.957e10, em_flag=5, s_max=30, use_bvec=False,
+                        voxel_order=_lib.ORDER_RECORD, out_device_ptrs=None, image_shape=None, tile=(4, 8),
+                        ray_order=None, s_mode="per_step", s_input_on=False):
+        """render_map with the map diagnostics (rtgrff_render_map_diag): where the emission of every (pixel,
+        frequency) comes from.  Same keywords and the same tb, vi; returns (tb, vi, stats, diag) with diag a dict of
+        (n_freq, n_rays) float64 arrays: em_x, em_y, em_z (emission centroid [R_sun]), em_r (contribution-weighted
+        mean heliocentric distance [R_sun]), tau_L, tau_R (total optical depth of the L and R slot), ray_r_min
+        (the ray's turning point [R_sun]); definitions in include/rtgrff.h.  With out_device_ptrs=(tb_ptr, vi_ptr,
+        diag_ptr) everything goes to device buffers (diag: 7 n_freq planes of n_rays) and (None, None, stats,
+        None) is returned."""
+        return self._render(True, x_start, y_start, z_start, freq_params, kvec_in_norm, trace_crosssections,
+                            perturb_ratio, pixel_area_cm2, r_sun_cm, em_flag, s_max, use_bvec, voxel_order,
+                            out_device_ptrs, image_shape, tile, ray_order, s_mode, s_input_on)
+
+    def _render(self, diag, x_start, y_start, z_start, freq_params, kvec_in_norm, trace_crosssections, perturb_ratio,
+                pixel_area_cm2, r_sun_cm, em_flag, s_max, use_bvec, voxel_order, out_device_ptrs, image_shape, tile,
+                ray_order, s_mode, s_input_on):
         xs, ys, zs = f64(x_start).ravel(), f64(y_start).ravel(), f64(z_start).ravel()
         n_rays = xs.shape[0]
         kv = None
@@ -371,18 +393,31 @@ class RaySession:
                 p = (p["freq_hz"], p["dt"], p["n_steps"], p["record_stride"])
             arr[i] = FreqParams(float(p[0]), float(p[1]), int(p[2]), int(p[3]))
         stats = (c_int64 * 4)()
+        dg = None
         if out_device_ptrs is None:
             tb = np.empty((nf, n_rays), dtype=np.float64)
             vi = np.empty_like(tb)
             ptb, pvi, on_dev = tb.ctypes.data_as(ctypes.c_void_p), vi.ctypes.data_as(ctypes.c_void_p), 0
+            if diag:
+                dg = np.empty((len(_lib.DIAG_PLANES), nf, n_rays), dtype=np.float64)
+                pdg = dg.ctypes.data_as(ctypes.c_void_p)
         else:
+            if diag and len(out_device_ptrs) != 3:
+                raise ValueError("out_device_ptrs must be (tb_ptr, vi_ptr, diag_ptr)")
             tb = vi = None
             ptb, pvi, on_dev = ctypes.c_void_p(out_device_ptrs[0]), ctypes.c_void_p(out_device_ptrs[1]), 1
-        check(self._lib.rtgrff_render_map(self.ctx.handle, n_rays, ptr(xs, c_double), ptr(ys, c_double),
-                                          ptr(zs, c_double), ptr(kv, c_double), ptr(order, ctypes.c_int32), nf, arr,
-                                          int(bool(trace_crosssections)), float(perturb_ratio), float(pixel_area_cm2),
-                                          float(r_sun_cm), int(em_flag), int(s_max), int(bool(use_bvec)),
-                                          int(voxel_order), _s_mode(s_mode), int(bool(s_input_on)), ptb, pvi, on_dev,
-                                          stats))
-        return tb, vi, {"nominal_ray_steps": int(stats[0]), "active_ray_steps": int(stats[1]),
-                        "pencil_steps": int(stats[2]), "valid_samples": int(stats[3])}
+            if diag:
+                pdg = ctypes.c_void_p(out_device_ptrs[2])
+        args = (self.ctx.handle, n_rays, ptr(xs, c_double), ptr(ys, c_double), ptr(zs, c_double), ptr(kv, c_double),
+                ptr(order, ctypes.c_int32), nf, arr, int(bool(trace_crosssections)), float(perturb_ratio),
+                float(pixel_area_cm2), float(r_sun_cm), int(em_flag), int(s_max), int(bool(use_bvec)), int(voxel_order),
+                _s_mode(s_mode), int(bool(s_input_on)), ptb, pvi, on_dev, stats)
+        if diag:
+            check(self._lib.rtgrff_render_map_diag(*args, pdg))
+        else:
+            check(self._lib.rtgrff_render_map(*args))
+        st = {"nominal_ray_steps": int(stats[0]), "active_ray_steps": int(stats[1]),
+              "pencil_steps": int(stats[2]), "valid_samples": int(stats[3])}
+        if not diag:
+            return tb, vi, st
+        return tb, vi, st, (None if dg is None else dict(zip(_lib.DIAG_PLANES, dg)))

@@ -18,7 +18,7 @@ import numpy as np
 
 from . import synthetic
 from .session import RaySession
-from .workflow import R_sun_cm, R_sun_m, pixel_area_cm2
+from .workflow import R_sun_cm, R_sun_m, diagnostic_maps, pixel_area_cm2
 
 
 def _lowband_params(freq_hz):
@@ -76,10 +76,12 @@ def select_params(freq_hz):
 
 def tb_spectra(model, out_dir, N_pix=128, fmin_mhz=30.0, fmax_mhz=800.0, n_freq=30, start_from_idx=0,
                phi0_offset=-140.0, session=None, quiet=True, params_fn=select_params, use_bvec=False,
-               em_flag=5, max_grid_n=None):
+               em_flag=5, max_grid_n=None, diagnostics=False):
     """Run the sweep.  `model` is a spherical model (cubes.SphericalVariable mapping).  Returns the
     manifest rows [(idx, freq_hz, npz_path)].  Existing files of indices < start_from_idx are kept
-    (the reference's resume switch, :118-119, :141-142)."""
+    (the reference's resume switch, :118-119, :141-142).  diagnostics=True: every npz also holds the keys of
+    workflow.diagnostic_maps (emission centroid and height, optical depths, ray turning point), which over the
+    sweep give the emission height against frequency."""
     out_dir = Path(out_dir)
     out_dir.mkdir(parents=True, exist_ok=True)
     freqs_hz = np.logspace(np.log10(fmin_mhz), np.log10(fmax_mhz), n_freq) * 1e6
@@ -100,15 +102,17 @@ def tb_spectra(model, out_dir, N_pix=128, fmin_mhz=30.0, fmax_mhz=800.0, n_freq=
             ses.set_model_from_spherical(model, g, g, g, phi0_offset=phi0_offset, want_bvec=use_bvec)
             xs, ys, zs, kv = synthetic.ray_launch_geometry(N_pix, float(p["x_fov"]), float(p["z_observer"]))
             area = pixel_area_cm2(float(p["x_fov"]), N_pix)
-            tb, vi, _ = ses.render_map(xs, ys, zs, [(float(freq_hz), float(p["dt"]), int(p["n_steps"]),
-                                                     int(p["record_stride"]))], kvec_in_norm=kv,
-                                       trace_crosssections=True, perturb_ratio=2.0, pixel_area_cm2=area,
-                                       r_sun_cm=R_sun_cm, em_flag=em_flag, use_bvec=use_bvec, image_shape=(N_pix, N_pix))
+            render = ses.render_map_diag if diagnostics else ses.render_map
+            out = render(xs, ys, zs, [(float(freq_hz), float(p["dt"]), int(p["n_steps"]), int(p["record_stride"]))],
+                         kvec_in_norm=kv, trace_crosssections=True, perturb_ratio=2.0, pixel_area_cm2=area,
+                         r_sun_cm=R_sun_cm, em_flag=em_flag, use_bvec=use_bvec, image_shape=(N_pix, N_pix))
+            tb, vi = out[0], out[1]
+            extra = diagnostic_maps(out[3], N_pix) if diagnostics else {}
             coords = np.linspace(-p["x_fov"], p["x_fov"], N_pix) * R_sun_m
             np.savez_compressed(npz_path,                                    # script/...:533-540
                                 emission_cube=np.nan_to_num(tb[0].reshape(N_pix, N_pix, 1), nan=0.0, posinf=0.0, neginf=0.0),
                                 emission_polVI_cube=vi[0].reshape(N_pix, N_pix, 1),
-                                frequencies_Hz=np.array([float(freq_hz)]), x_coords=coords, y_coords=coords)
+                                frequencies_Hz=np.array([float(freq_hz)]), x_coords=coords, y_coords=coords, **extra)
         if not npz_path.exists():
             raise FileNotFoundError(f"Missing expected npz file: {npz_path}")
         rows.append((i, float(freq_hz), str(npz_path)))
@@ -131,12 +135,14 @@ def main(argv=None):
     ap.add_argument("--device", default="cuda", choices=["cpu", "cuda"])
     ap.add_argument("--raytrace-device", default="cuda", choices=["cpu", "cuda"])
     ap.add_argument("--quiet", "-q", action="store_true")
+    ap.add_argument("--diagnostics", action="store_true",
+                    help="also save emission centroid and height, optical depths and ray turning point per pixel")
     a = ap.parse_args(argv)
     if a.device != "cuda" or a.raytrace_device != "cuda":
         raise RuntimeError("raytracinggrff_b200 is CUDA-only (no CPU path, no fallback)")
     model = synthetic.spherical_corona(150, 110, 128, r_max=8.0, active_region=True)
     rows = tb_spectra(model, a.out_dir, a.N_pix, a.fmin_mhz, a.fmax_mhz, a.n_freq, a.start_from_idx, a.phi0_offset,
-                      quiet=a.quiet)
+                      quiet=a.quiet, diagnostics=a.diagnostics)
     print(f"Saved {len(rows)} maps to {a.out_dir}")
 
 

@@ -91,9 +91,19 @@ def _upload_model(ses, model, grid_n, grid_extent, phi0_offset):
         ses.set_model_from_spherical(model, xg, yg, zg, phi0_offset=phi0_offset)
 
 
+def diagnostic_maps(diag, N_pix):
+    """RaySession.render_map_diag's planes ((n_freq, n_rays) each, ray p = i*N_pix + j) -> the result / npz keys of
+    ``diagnostics=True``: emission_centroid_xyz (N_pix, N_pix, n_freq, 3) [R_sun], emission_r_mean, tau_L, tau_R and
+    ray_r_min (N_pix, N_pix, n_freq) each, laid out as emission_cube."""
+    m = {k: np.moveaxis(np.asarray(v).reshape(-1, N_pix, N_pix), 0, -1) for k, v in diag.items()}
+    return {"emission_centroid_xyz": np.stack([m["em_x"], m["em_y"], m["em_z"]], axis=-1),
+            "emission_r_mean": m["em_r"], "tau_L": m["tau_L"], "tau_R": m["tau_R"], "ray_r_min": m["ray_r_min"]}
+
+
 def _emission_of_rays(ses, backend, x_flat, y_flat, z_start, kvec, p, image_shape=None):
     """The hot path for one contiguous range of rays on one GPU: trace -> sample -> GRFF -> T_b.  `p` holds the
-    call's scalar settings.  Returns (tb (n_rays, Nf), vi (n_rays, Nf), sampled or None)."""
+    call's scalar settings.  Returns (tb (n_rays, Nf), vi (n_rays, Nf), sampled or None, diag or None); diag is
+    render_map_diag's dict of (Nf, n_rays) planes when p["diagnostics"]."""
     n_rays = len(x_flat)
     Nf, freq0, freq_hz, freq_log_step, area = p["Nf"], p["freq0"], p["freq_hz"], p["freq_log_step"], p["area"]
     frequencies_Hz = p["frequencies_Hz"]
@@ -102,19 +112,20 @@ def _emission_of_rays(ses, backend, x_flat, y_flat, z_start, kvec, p, image_shap
     ray_start = np.column_stack([x_flat, y_flat, z_start])
     sampled = None
     if backend == "fused":
-        tb, vi, _ = ses.render_map(x_flat, y_flat, z_start, [(freq_hz, p["dt"], p["n_steps"], p["record_stride"])],
-                                   kvec_in_norm=kvec, trace_crosssections=True, perturb_ratio=p["perturb_ratio"],
-                                   pixel_area_cm2=area, r_sun_cm=R_sun_cm, image_shape=image_shape,
-                                   s_mode=p["s_mode"], s_input_on=p["s_input_on"])
-        tb_out[:, 0], vi_out[:, 0] = tb[0], vi[0]
-        return tb_out, vi_out, None
+        render = ses.render_map_diag if p["diagnostics"] else ses.render_map
+        out = render(x_flat, y_flat, z_start, [(freq_hz, p["dt"], p["n_steps"], p["record_stride"])],
+                     kvec_in_norm=kvec, trace_crosssections=True, perturb_ratio=p["perturb_ratio"],
+                     pixel_area_cm2=area, r_sun_cm=R_sun_cm, image_shape=image_shape,
+                     s_mode=p["s_mode"], s_input_on=p["s_input_on"])
+        tb_out[:, 0], vi_out[:, 0] = out[0][0], out[1][0]
+        return tb_out, vi_out, None, (out[3] if p["diagnostics"] else None)
     keep_host = backend in ("get_mw", "fastgrff") or p["return_samples"]
     ses.trace(freq_hz, x_flat, y_flat, z_start, kvec, p["dt"], p["n_steps"], p["record_stride"], True, p["perturb_ratio"],
               s_mode=p["s_mode"], fetch=False)
     sampled = ses.sample_traced(ray_start, R_sun_cm, 0.0, 1e4, 0.0, fetch=keep_host)
     if backend == "device":
         tb, vi = ses.emission_traced(area, freq0, Nf, freq_log_step, s_input_on=p["s_input_on"])
-        return tb, vi, sampled
+        return tb, vi, sampled, None
     if backend == "fastgrff":
         n_rec = sampled["ne"].shape[0]
         Parms_M = pack_parms_batch(sampled, area, p["s_input_on"])
@@ -129,7 +140,7 @@ def _emission_of_rays(ses, backend, x_flat, y_flat, z_start, kvec, p, image_shap
             if status[q] != 0:
                 continue
             tb_out[q], vi_out[q] = tb_from_rl(RL_M[:, :, q], frequencies_Hz, area)
-        return tb_out, vi_out, sampled
+        return tb_out, vi_out, sampled, None
     # 'get_mw': the reference's per-pixel loop, script/resample_with_ray_tracing.py:467-524
     GET_MW = initGET_MW(p["grff_lib"])
     Lparms = np.zeros(5, dtype="int32")
@@ -158,7 +169,7 @@ def _emission_of_rays(ses, backend, x_flat, y_flat, z_start, kvec, p, image_shap
         if GET_MW(L, Rparms, Parms, dummy, dummy, dummy, RL) != 0:
             continue
         tb_out[q], vi_out[q] = tb_from_rl(RL, frequencies_Hz, area)
-    return tb_out, vi_out, sampled
+    return tb_out, vi_out, sampled, None
 
 
 def run_ray_tracing_emission(model, N_pix=64, X_fov=1.44, freq_hz=75e6, z_observer=3.0, dt=6e-3, n_steps=5000,
@@ -166,17 +177,22 @@ def run_ray_tracing_emission(model, N_pix=64, X_fov=1.44, freq_hz=75e6, z_observ
                              freq0=None, freq_log_step=0.0, save_plots=False, verbose=True, device="cuda",
                              fallback_to_cpu=False, raytrace_device="cuda", grff_backend="get_mw",
                              perturb_ratio=2, session=None, return_samples=False, s_mode="per_step",
-                             grid_n=128, grid_extent=3.0, phi0_offset=0.0, consider_beam=False, beam_fwhm=0.2):
+                             grid_n=128, grid_extent=3.0, phi0_offset=0.0, consider_beam=False, beam_fwhm=0.2,
+                             diagnostics=False):
     """``n_workers`` (the reference's ``--workers``, script/resample_with_ray_tracing.py:333-352: contiguous ray
     chunks over a process pool, concatenated on the ray axis) maps to GPUs here: the rays are split into
     ``n_workers`` contiguous chunks exactly as there, chunk k runs on GPU k mod (number of visible GPUs) from its
     own host thread (the library calls release the GIL) with its own context and a replica of the cubes, and the
-    chunks' maps are concatenated.  Rays never interact, so the result does not depend on the split."""
+    chunks' maps are concatenated.  Rays never interact, so the result does not depend on the split.
+    ``diagnostics`` (fused backend only): the result and the npz also hold where each pixel's emission comes from,
+    the keys of diagnostic_maps (RaySession.render_map_diag); every other key is the same as without."""
     if freq0 is None:
         freq0 = freq_hz
     backend = grff_backend.lower()
     if backend not in ("get_mw", "fastgrff", "device", "fused"):
         raise ValueError(f"Unsupported grff_backend '{grff_backend}'. Use 'get_mw', 'fastgrff', 'device' or 'fused'.")
+    if diagnostics and backend != "fused":
+        raise ValueError(f"diagnostics need the fused backend (grff_backend='fused'), not '{grff_backend}'")
     _check_device("device", device)
     _check_device("raytrace_device", raytrace_device)
     # s_input_on (script/resample_with_ray_tracing.py:501): Parms[14] = S * area.  The reference leaves the
@@ -195,13 +211,15 @@ def run_ray_tracing_emission(model, N_pix=64, X_fov=1.44, freq_hz=75e6, z_observ
                          "(or RaySession.render_map for a list of frequencies)")
     p = dict(Nf=Nf, freq0=freq0, freq_hz=freq_hz, freq_log_step=freq_log_step, area=area, frequencies_Hz=frequencies_Hz,
              dt=dt, n_steps=n_steps, record_stride=record_stride, perturb_ratio=perturb_ratio, s_mode=s_mode,
-             s_input_on=s_input_on, return_samples=return_samples, verbose=verbose, grff_lib=grff_lib)
+             s_input_on=s_input_on, return_samples=return_samples, verbose=verbose, grff_lib=grff_lib,
+             diagnostics=bool(diagnostics))
 
     n_workers = max(1, int(n_workers))
     if n_workers == 1 or n_rays < 2:
         ses = session or RaySession(context=_lib.default_context())
         _upload_model(ses, model, grid_n, grid_extent, phi0_offset)
-        tb, vi, sampled = _emission_of_rays(ses, backend, x_flat, y_flat, z_start, kvec, p, image_shape=(N_pix, N_pix))
+        tb, vi, sampled, diag = _emission_of_rays(ses, backend, x_flat, y_flat, z_start, kvec, p,
+                                                  image_shape=(N_pix, N_pix))
     else:
         from concurrent.futures import ThreadPoolExecutor
         n_dev = _lib.load().rtgrff_device_count()
@@ -225,6 +243,9 @@ def run_ray_tracing_emission(model, N_pix=64, X_fov=1.44, freq_hz=75e6, z_observ
         sampled = None
         if parts[0][2]:
             sampled = {k: np.concatenate([q[2][k] for q in parts], axis=1) for k in parts[0][2]}
+        diag = None
+        if parts[0][3]:
+            diag = {k: np.concatenate([q[3][k] for q in parts], axis=1) for k in parts[0][3]}
 
     emission_cube = tb.reshape(N_pix, N_pix, Nf)
     emission_polVI_cube = vi.reshape(N_pix, N_pix, Nf)
@@ -243,6 +264,8 @@ def run_ray_tracing_emission(model, N_pix=64, X_fov=1.44, freq_hz=75e6, z_observ
         beam = emission_cube[:, :, 0].copy()
         beam[beam == 0] = np.nan
         result["emission_map_beam"] = convolve_beam(beam, beam_fwhm, [-X_fov, X_fov], N_pix)
+    if diag is not None:
+        result.update(diagnostic_maps(diag, N_pix))
     if out_path is not None:
         np.savez_compressed(out_path, **result)
     if return_samples and sampled:
@@ -280,6 +303,9 @@ def main(argv=None):
     parser.add_argument("--no-fallback", action="store_true", help="accepted for compatibility; there is no CPU path to fall back to")
     parser.add_argument("--no-plots", action="store_true", help="accepted for compatibility; no plots are made")
     parser.add_argument("--quiet", "-q", action="store_true")
+    parser.add_argument("--diagnostics", action="store_true",
+                        help="also save emission centroid, emission height, optical depths and ray turning point "
+                             "per pixel (fused backend only)")
     args = parser.parse_args(argv)
     if args.model_path == "synthetic":
         model = synthetic.spherical_corona()
@@ -292,7 +318,8 @@ def main(argv=None):
         n_workers=args.workers, s_input_on=args.s_input_on, out_path=args.out_path, grff_lib=args.grff_lib, Nfreq=1,
         freq0=args.freq, freq_log_step=0.0, save_plots=False, verbose=not args.quiet, device=args.device,
         fallback_to_cpu=not args.no_fallback, raytrace_device=args.raytrace_device, grff_backend=args.grff_backend,
-        consider_beam=args.consider_beam, beam_fwhm=args.beam_fwhm, phi0_offset=args.phi0_offset, s_mode=args.s_mode)
+        consider_beam=args.consider_beam, beam_fwhm=args.beam_fwhm, phi0_offset=args.phi0_offset, s_mode=args.s_mode,
+        diagnostics=args.diagnostics)
     if not args.quiet:
         tb = res["emission_cube"]
         print(f"T_b map {tb.shape} at {args.freq / 1e6:.1f} MHz: max {tb.max():.3e} K -> {args.out_path}")
