@@ -297,6 +297,42 @@ int rtgrff_render_map_diag(rtgrff_ctx *ctx, int64_t n_rays, const double *x_star
                            int out_on_device, int64_t *stats, double *diag);
 
 /*
+ * Fused straight line-of-sight map: the straight-LOS counterpart of rtgrff_render_map, which replaces the staged
+ * rtgrff_sample_spherical_los x 5 + GET_MW chain (script/resampling_MAS_LOS.py resample_MAS followed by
+ * script/synthetic_FF_map_single_thread.py SyntheticFF) without materialising the LOS arrays or Parms.
+ *
+ * rtgrff_set_spherical_model: keep one variable of a spherical (phi, latitude, r) model resident on the device in
+ * `slot` (0 rho/n_e [cm^-3], 1 te [K], 2 br, 3 bt, 4 bp [G]; value = data * scale) until the slot is set again.
+ * data: host float32 (np, nt, nr) C-order; phi, lat, r: host float64 node coordinates (rad, rad, R_sun), ascending,
+ * >= 2 per axis.  Independent of the slots of rtgrff_resample_spherical.
+ */
+int rtgrff_set_spherical_model(rtgrff_ctx *ctx, int slot, const float *data, const double *phi, const double *lat,
+                               const double *r, int np, int nt, int nr, double scale);
+
+/*
+ * rtgrff_render_los_map: for every pixel (i, j) at (x[j], y[i]) [R_sun] the straight LOS of
+ * rtgrff_sample_spherical_los (start on the disk surface or behind the limb on the plane of the sky, minus z_eps, then
+ * the offsets zc[k] [R_sun] towards the observer, r < r_min -> no sample), sampled in FP64 from the five slots; then
+ * the reference's packing: a sample with NaN in n_e, T or |B| is dropped, the others keep their order and are handed
+ * to the transfer Sun side first with ds = dz_cm[k] [cm].  use_bvec 0: theta = 90 deg (the reference); 1: cos theta =
+ * B_z / |B| with B rotated to cube axes (the radiation travels +z).  Each voxel goes through the per-ray kernels'
+ * transfer (float32 voxel inputs, FP64 near the cut-offs or with rtgrff_ctx_set_grff64; gyroresonance when
+ * !(em_flag & 1)).  T_b and V/I as SyntheticFF: V/I = (L-R)/(L+R) (NaN where L+R = 0); a LOS without a valid sample
+ * gives T_b = 0, V/I = 0.
+ *  freq_hz: host float64 (n_freq), any n_freq >= 1, any order.
+ *  tb, vi: float64 (n_freq, ny, nx); diag: NULL or float64 (RTGRFF_N_DIAG, n_freq, ny, nx), the planes of
+ *  rtgrff_render_map_diag with a voxel's position its float32 sample position and RAY_RMIN the smallest |p| over
+ *  the LOS samples.  Host, or device pointers when out_on_device != 0: a rank that passes its rows' y values writes
+ *  the slab rtgrff_gather_image assembles.
+ *  stats (optional, host int64[3]): {LOS samples, valid samples, voxel-frequency evaluations}.
+ * RTGRFF_ENOCUBE when a slot has not been set.
+ */
+int rtgrff_render_los_map(rtgrff_ctx *ctx, int nx, int ny, const double *x, const double *y, int nz, const double *zc,
+                          const double *dz_cm, double phi0_offset_deg, double r_min, double z_eps, int n_freq,
+                          const double *freq_hz, double pixel_area_cm2, int em_flag, int s_max, int use_bvec, double *tb,
+                          double *vi, double *diag, int out_on_device, int64_t *stats);
+
+/*
  * Multi-GPU (one process per GPU, the cube replicated on each).  Rays are independent, so the only exchange
  * is the gather of the image at the end; this replaces the reference's ProcessPoolExecutor ray chunks and
  * their concatenate (script/resample_with_ray_tracing.py:42-61, :333-352, the `--workers` switch).

@@ -40,6 +40,7 @@ EXPORTS = (
     "rtgrff_export_cubes", "rtgrff_shard_rows", "rtgrff_comm_unique_id", "rtgrff_comm_init_rank",
     "rtgrff_comm_destroy", "rtgrff_gather_image", "rtgrff_device_alloc", "rtgrff_device_free",
     "rtgrff_ctx_set_pipeline", "rtgrff_ctx_set_grff64", "rtgrff_place_rows", "rtgrff_render_map_diag",
+    "rtgrff_set_spherical_model", "rtgrff_render_los_map",
 )
 
 # planes of rtgrff_render_map_diag's output (RTGRFF_DIAG_* in include/rtgrff.h), in plane order
@@ -111,6 +112,10 @@ def load():
                                       c_double, c_double, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p,
                                       c_int, POINTER(c_int64)]
     lib.rtgrff_render_map_diag.argtypes = lib.rtgrff_render_map.argtypes + [c_void_p]
+    lib.rtgrff_set_spherical_model.argtypes = [c_void_p, c_int, fp, dp, dp, dp, c_int, c_int, c_int, c_double]
+    lib.rtgrff_render_los_map.argtypes = [c_void_p, c_int, c_int, dp, dp, c_int, dp, dp, c_double, c_double, c_double,
+                                          c_int, dp, c_double, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int,
+                                          POINTER(c_int64)]
     lib.rtgrff_gaussian_beam.argtypes = [c_void_p, dp, c_int, c_int, c_int, c_double, c_double, dp]
     lib.rtgrff_patch_nan.argtypes = [c_void_p, dp, c_int, c_int, c_int, c_int, POINTER(c_int64)]
     for name in EXPORTS:

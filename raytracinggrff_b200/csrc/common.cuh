@@ -7,6 +7,8 @@
 #include <stdio.h>
 #include <string.h>
 
+#include <vector>
+
 #include "../../include/rtgrff.h"
 
 // Threads per block / minimum resident blocks per SM of the per-ray kernels (tuned on B200, see
@@ -127,6 +129,14 @@ struct rtgrff_ctx {
     double slot_geom[12] = {0};
     double slot_geoms[5][12] = {{0}};   // geometry each slot was resampled on (compose checks they agree)
     bool stage_has_omega = false;    // `stage` still holds the float64 omega_pe of the last compose (rtgrff_export_cubes)
+
+    // spherical model resident for the straight-LOS map (rtgrff_set_spherical_model): slot 0..4 = rho, te, br, bt, bp,
+    // float32 data on the device, the node coordinates phi, lat, r on the host (uploaded with each map)
+    rtgrff::DevBuf sph_data[5];
+    std::vector<double> sph_nodes[5];
+    int sph_n[5][3] = {{0}};
+    double sph_scale[5] = {0};
+    bool sph_set[5] = {false, false, false, false, false};
 
     // multi-GPU image gather (rtgrff_comm_*): an ncclComm_t behind a void*, NCCL loaded at run time
     void *comm = nullptr;

@@ -144,6 +144,46 @@ __global__ void __launch_bounds__(256) los_spherical_kernel(const LosArgs a)
     }
 }
 
+// los_spherical_kernel's geometry, expression for expression, for the fused LOS map (los_map.cuh), so that its samples
+// are the ones rtgrff_sample_spherical_los returns.
+// z of the first sample of the LOS through (x, y): on the disk surface, or behind the limb on the plane of the sky
+__device__ __forceinline__ double los_z0(double x, double y, double z_eps)
+{
+    const double rho2 = x * x + y * y;
+    return (sqrt(rho2) < 1.0) ? sqrt(1.0 - rho2) - z_eps : -sqrt(rho2 - 1.0) - z_eps;
+}
+
+// cart_to_sph(x, -z, y, phi0) of a cube point: longitude, latitude [rad] and r [R_sun]
+__device__ __forceinline__ void los_sph(double x, double y, double z, double phi0_offset_rad, double &lon, double &lat,
+                                        double &r)
+{
+    const double cx = x, cy = -z, cz = y;
+    r = sqrt(cx * cx + cy * cy + cz * cz);
+    const double colat = acos(fmin(1.0, fmax(-1.0, cz / r)));
+    lon = atan2(cy, cx) + phi0_offset_rad;
+    if (lon < 0.0) lon += 6.283185307179586476925286766559;
+    lat = 1.5707963267948966192313216916398 - colat;
+}
+
+// Spherical (r, theta = colatitude from +y, phi in the x / -z plane) components at cube point (x, y, z) -> cube axes
+// (compose_cubes_kernel's rotation)
+__device__ __forceinline__ void sph_to_cube_b(double x, double y, double z, double br, double bt, double bp, double &bx,
+                                              double &by, double &bz)
+{
+    const double cx = x, cy = -z, cz = y;              // model frame (build_rays.py:93)
+    const double rr = sqrt(cx * cx + cy * cy + cz * cz), rho_c = sqrt(cx * cx + cy * cy);
+    double mx = 0.0, my = 0.0, mz = 0.0;
+    if (rr > 0.0 && rho_c > 0.0) {
+        const double st = rho_c / rr, ct = cz / rr, cp = cx / rho_c, sp = cy / rho_c;
+        mx = br * st * cp + bt * ct * cp - bp * sp;
+        my = br * st * sp + bt * ct * sp + bp * cp;
+        mz = br * ct - bt * st;
+    } else if (rr > 0.0) {
+        mz = br * (cz > 0.0 ? 1.0 : -1.0);
+    }
+    bx = mx; by = mz; bz = -my;                        // model (mx,my,mz) -> cube: x = mx, z = -my, y = mz
+}
+
 // script/resample_with_ray_tracing.py:269-293 on device: rho -> omega_pe (f64, for the gradient
 // kernel) and n_e >= 0; T NaN -> 1e4; |B| = sqrt(br^2+bt^2+bp^2); optional Cartesian B vector.
 struct ComposeArgs {
@@ -170,22 +210,10 @@ __global__ void __launch_bounds__(256) compose_cubes_kernel(const ComposeArgs a)
         const double b = sqrt(br * br + bt * bt + bp * bp);                          // :293
         a.fcube[q] = make_float4((float)ne, (float)te, (float)b, 0.0f);
         if (a.bcube) {
-            // spherical (r, theta = colatitude from +y, phi in the x / -z plane) -> cube axes
             const int k = (int)(q % a.nz), j = (int)((q / a.nz) % a.ny), i = (int)(q / ((int64_t)a.ny * a.nz));
-            const double x = a.xg[i], y = a.yg[j], z = a.zg[k];
-            const double cx = x, cy = -z, cz = y;              // model frame (build_rays.py:93)
-            const double rr = sqrt(cx * cx + cy * cy + cz * cz), rho_c = sqrt(cx * cx + cy * cy);
-            double mx = 0.0, my = 0.0, mz = 0.0;
-            if (rr > 0.0 && rho_c > 0.0) {
-                const double st = rho_c / rr, ct = cz / rr, cp = cx / rho_c, sp = cy / rho_c;
-                mx = br * st * cp + bt * ct * cp - bp * sp;
-                my = br * st * sp + bt * ct * sp + bp * cp;
-                mz = br * ct - bt * st;
-            } else if (rr > 0.0) {
-                mz = br * (cz > 0.0 ? 1.0 : -1.0);
-            }
-            // model (mx,my,mz) -> cube: x = mx, z = -my, y = mz
-            a.bcube[q] = make_float4((float)mx, (float)mz, (float)(-my), 0.0f);
+            double bx, by, bz;
+            sph_to_cube_b(a.xg[i], a.yg[j], a.zg[k], br, bt, bp, bx, by, bz);
+            a.bcube[q] = make_float4((float)bx, (float)by, (float)bz, 0.0f);
         }
     }
 }

@@ -15,6 +15,7 @@
 #include "fused_map.cuh"
 #include "grff.cuh"
 #include "image_ops.cuh"
+#include "los_map.cuh"
 #include "los_sampler.cuh"
 #include "ray_integrator.cuh"
 #include "trace_kernel.cuh"
@@ -475,6 +476,7 @@ int rtgrff_ctx_destroy(rtgrff_ctx *c)
                       &c->out2, &c->out3, &c->out4, &c->out5, &c->stage, &c->counters, &c->gather_buf, &c->image_buf};
     for (DevBuf *b : bufs) b->release();
     for (DevBuf &b : c->slot) b.release();
+    for (DevBuf &b : c->sph_data) b.release();
     c->slot_grids.release();
     if (c->ev0) cudaEventDestroy(c->ev0);
     if (c->ev1) cudaEventDestroy(c->ev1);
@@ -1353,6 +1355,145 @@ int rtgrff_render_map_diag(rtgrff_ctx *c, int64_t n_rays, const double *x_start,
     return render_map_impl(c, n_rays, x_start, y_start, z_start, kvec, ray_order, n_freq, freqs, trace_cs, perturb_ratio,
                            pixel_area_cm2, r_sun_cm, em_flag, s_max, use_bvec, voxel_order, s_mode, s_input_on, tb, vi,
                            out_on_device, stats, diag);
+}
+
+// ---- fused straight line-of-sight map ----------------------------------------------------------------
+int rtgrff_set_spherical_model(rtgrff_ctx *c, int slot, const float *data, const double *phi, const double *lat,
+                               const double *r, int np, int nt, int nr, double scale)
+{
+    RT_USE(c);
+    if (slot < 0 || slot >= kLosSlots) return fail(RTGRFF_EINVAL, "slot %d out of range 0..4", slot);
+    if (!data || !phi || !lat || !r) return fail(RTGRFF_EINVAL, "null argument");
+    if (np < 2 || nt < 2 || nr < 2) return fail(RTGRFF_EINVAL, "spherical mesh needs >= 2 nodes per axis");
+    if ((int64_t)np * nt * nr >= (int64_t)1 << 31) return fail(RTGRFF_EINVAL, "spherical mesh larger than 2^31 nodes");
+    for (int i = 1; i < np; ++i) if (!(phi[i] > phi[i - 1])) return fail(RTGRFF_EINVAL, "phi nodes must ascend");
+    for (int i = 1; i < nt; ++i) if (!(lat[i] > lat[i - 1])) return fail(RTGRFF_EINVAL, "latitude nodes must ascend");
+    for (int i = 1; i < nr; ++i) if (!(r[i] > r[i - 1])) return fail(RTGRFF_EINVAL, "radius nodes must ascend");
+    c->sph_set[slot] = false;
+    RT_TRY(h2d(c, c->sph_data[slot], data, (size_t)np * nt * nr * sizeof(float)));
+    std::vector<double> &n = c->sph_nodes[slot];
+    n.assign(phi, phi + np);
+    n.insert(n.end(), lat, lat + nt);
+    n.insert(n.end(), r, r + nr);
+    c->sph_n[slot][0] = np; c->sph_n[slot][1] = nt; c->sph_n[slot][2] = nr;
+    c->sph_scale[slot] = scale;
+    RT_CUDA(cudaStreamSynchronize(c->stream));   // the host buffer may be reused by the caller
+    c->sph_set[slot] = true;
+    return RTGRFF_OK;
+}
+
+// rtgrff_render_los_map / diag == nullptr launches the plain kernels, else the DIAG ones
+int rtgrff_render_los_map(rtgrff_ctx *c, int nx, int ny, const double *x, const double *y, int nz, const double *zc,
+                          const double *dz_cm, double phi0_offset_deg, double r_min, double z_eps, int n_freq,
+                          const double *freq_hz, double pixel_area_cm2, int em_flag, int s_max, int use_bvec, double *tb,
+                          double *vi, double *diag, int out_on_device, int64_t *stats)
+{
+    RT_USE(c);
+    if (!x || !y || !zc || !dz_cm || !freq_hz || !tb || !vi) return fail(RTGRFF_EINVAL, "null argument");
+    if (nx < 1 || ny < 1 || nz < 1 || n_freq < 1) return fail(RTGRFF_EINVAL, "bad sizes (nx %d, ny %d, nz %d, n_freq %d)",
+                                                              nx, ny, nz, n_freq);
+    if ((int64_t)nx * ny >= (int64_t)1 << 31) return fail(RTGRFF_EINVAL, "image larger than 2^31 pixels");
+    for (int f = 0; f < n_freq; ++f)
+        if (!(freq_hz[f] > 0.0) || !isfinite(freq_hz[f])) return fail(RTGRFF_EINVAL, "bad frequency at index %d", f);
+    static const char *names[kLosSlots] = {"rho", "te", "br", "bt", "bp"};
+    for (int v = 0; v < kLosSlots; ++v)
+        if (!c->sph_set[v]) return fail(RTGRFF_ENOCUBE, "rtgrff_set_spherical_model has not set slot %d (%s)", v, names[v]);
+    if (stats) stats[0] = stats[1] = stats[2] = 0;
+    LosMapArgs a;
+    int n_nodes = 0;
+    for (int v = 0; v < kLosSlots; ++v) {
+        a.var[v].data = c->sph_data[v].as<float>();
+        a.var[v].phi = a.var[v].lat = a.var[v].r = nullptr;
+        a.var[v].np = c->sph_n[v][0]; a.var[v].nt = c->sph_n[v][1]; a.var[v].nr = c->sph_n[v][2];
+        a.scale[v] = c->sph_scale[v];
+        a.node_off[v] = n_nodes;
+        n_nodes += (int)c->sph_nodes[v].size();
+    }
+    // the frequencies of a block: as many groups of at most kLosMaxFreqGroup as needed, balanced
+    const int groups = (n_freq + kLosMaxFreqGroup - 1) / kLosMaxFreqGroup;
+    const int fg = (n_freq + groups - 1) / groups;
+    if (groups > 65535) return fail(RTGRFF_EINVAL, "n_freq %d too large", n_freq);
+    const size_t smem = los_map_smem(fg, n_nodes);
+    int dev_smem = 0;
+    RT_CUDA(cudaDeviceGetAttribute(&dev_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, c->device));
+    if (smem > (size_t)dev_smem)
+        return fail(RTGRFF_EINVAL, "spherical meshes too large: %d nodes need %zu B of shared memory (%d available)", n_nodes,
+                    smem, dev_smem);
+    // inputs: x | y | zc | dz_cm | mesh nodes in one buffer, the per-frequency constants in another
+    std::vector<double> host((size_t)nx + ny + 2 * (size_t)nz + n_nodes);
+    double *h = host.data();
+    memcpy(h, x, nx * sizeof(double));
+    memcpy(h + nx, y, ny * sizeof(double));
+    memcpy(h + nx + ny, zc, nz * sizeof(double));
+    memcpy(h + nx + ny + nz, dz_cm, nz * sizeof(double));
+    for (int v = 0; v < kLosSlots; ++v)
+        memcpy(h + nx + ny + 2 * (size_t)nz + a.node_off[v], c->sph_nodes[v].data(), c->sph_nodes[v].size() * sizeof(double));
+    std::vector<FreqC> fq(n_freq);
+    for (int f = 0; f < n_freq; ++f) fq[f] = make_freq(freq_hz[f]);
+    RT_TRY(h2d(c, c->in0, h, host.size() * sizeof(double)));
+    RT_TRY(h2d(c, c->in1, fq.data(), fq.size() * sizeof(FreqC)));
+    const double *d = c->in0.as<double>();
+    a.x = d; a.y = d + nx; a.zc = d + nx + ny; a.dz_cm = d + nx + ny + nz;
+    a.nodes = d + nx + ny + 2 * (size_t)nz;
+    a.n_nodes = n_nodes;
+    a.nx = nx; a.ny = ny; a.nz = nz;
+    a.tiles_x = (nx + kLosTileW - 1) / kLosTileW;
+    a.phi0_offset_rad = phi0_offset_deg * M_PI / 180.0;
+    a.r_min = r_min; a.z_eps = z_eps;
+    a.freqs = c->in1.as<FreqC>();
+    a.n_freq = n_freq; a.fg = fg;
+    a.area = pixel_area_cm2;
+    a.em_flag = em_flag; a.s_max = s_max; a.grff64 = c->grff64;
+    const size_t npix = (size_t)nx * ny, nb = npix * sizeof(double);
+    double *dtb = tb, *dvi = vi, *ddiag = diag;
+    if (!out_on_device) {
+        RT_TRY(c->out0.reserve((size_t)n_freq * nb));
+        RT_TRY(c->out1.reserve((size_t)n_freq * nb));
+        dtb = c->out0.as<double>(); dvi = c->out1.as<double>();
+        if (diag) {
+            RT_TRY(c->out3.reserve((size_t)RTGRFF_N_DIAG * n_freq * nb));
+            ddiag = c->out3.as<double>();
+        }
+    }
+    a.tb = dtb; a.vi = dvi; a.diag = ddiag;
+    RT_TRY(c->counters.reserve(64));
+    RT_CUDA(cudaMemsetAsync(c->counters.p, 0, 64, c->stream));
+    a.valid_samples = c->counters.as<unsigned long long>();
+    const int64_t tiles = (int64_t)a.tiles_x * ((ny + kLosTileH - 1) / kLosTileH);
+    const dim3 grid((unsigned int)tiles, (unsigned int)groups), block(32 * fg);
+    const bool gr = !(em_flag & 1);
+    const int variant = (use_bvec ? 4 : 0) | (use_bvec || gr ? 2 : 0) | (diag ? 1 : 0);
+    RT_CUDA(cudaEventRecord(c->ev0, c->stream));
+#define RT_LOS_CASE(v, BV, NB, DG)                                                                                \
+    case v:                                                                                                       \
+        if (smem > 48 * 1024)                                                                                     \
+            RT_CUDA(cudaFuncSetAttribute(los_map_kernel<BV, NB, DG>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+                                         (int)smem));                                                             \
+        los_map_kernel<BV, NB, DG><<<grid, block, smem, c->stream>>>(a);                                          \
+        break;
+    switch (variant) {
+        RT_LOS_CASE(0, false, false, false) RT_LOS_CASE(1, false, false, true)
+        RT_LOS_CASE(2, false, true, false) RT_LOS_CASE(3, false, true, true)
+        RT_LOS_CASE(6, true, true, false) RT_LOS_CASE(7, true, true, true)
+    }
+#undef RT_LOS_CASE
+    RT_TRY(launched(c, "los_map_kernel"));
+    RT_CUDA(cudaEventRecord(c->ev1, c->stream));
+    c->ev_valid = true;
+    if (!out_on_device) {
+        RT_TRY(d2h(c, tb, dtb, (size_t)n_freq * nb));
+        RT_TRY(d2h(c, vi, dvi, (size_t)n_freq * nb));
+        if (diag) RT_TRY(d2h(c, diag, ddiag, (size_t)RTGRFF_N_DIAG * n_freq * nb));
+    }
+    unsigned long long n_valid = 0;
+    RT_TRY(d2h(c, &n_valid, c->counters.p, sizeof(n_valid)));
+    RT_CUDA(cudaStreamSynchronize(c->stream));
+    if (stats) {
+        stats[0] = (int64_t)npix * nz;
+        stats[1] = (int64_t)n_valid;
+        stats[2] = (int64_t)n_valid * n_freq;
+    }
+    return RTGRFF_OK;
 }
 
 // ---- multi-GPU: row sharding + image gather ---------------------------------------------------------

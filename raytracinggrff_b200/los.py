@@ -4,7 +4,9 @@
   sample rho, te, br, bt, bp of a spherical model along one straight LOS per pixel on the irregular z
   grid ``dz = dz0 (1 + (5 i/N_z)^2.5)`` and write ``LOS_data.npz``;
 * ``SyntheticFF``   — script/synthetic_FF_map_single_thread.py:108-244: per-pixel NaN filter, Parms
-  packing (theta = 90, flag 1+4, s_max 30), GET_MW, SFU -> T_b, ``<out>.npz``.
+  packing (theta = 90, flag 1+4, s_max 30), GET_MW, SFU -> T_b, ``<out>.npz``;
+* ``render_los_map`` — both in one fused kernel (rtgrff_render_los_map) with nothing materialised, optionally with
+  gyroresonance, theta from the B vector and the emission diagnostics.
 
 The MAS/psipy model is replaced by a mapping of cubes.SphericalVariable (SURVEY.md §8, row 11/12);
 everything after the model read keeps the reference's names, array shapes, units and file keys.
@@ -50,10 +52,8 @@ def _sample_los(ctx, var, x, y, zc, phi0_offset, r_min):
     return out
 
 
-def resample_MAS(model, N_pix, X_range, Y_range, N_z, dz0, variable_spacing_z=True, z_range=None,
-                 out_path="LOS_data.npz", save_plots=False, verbose=True, phi0_offset=0.0, r_min=R_MIN, context=None):
-    """Returns {'Ne_LOS','Te_LOS','B_LOS','ds_LOS' (N_pix,N_pix,N_z) [cm^-3, K, G, cm], 'x_coords',
-    'y_coords','z_coords' [m]} and writes them to `out_path` (script/resampling_MAS_LOS.py:288-300)."""
+def _check_model(model, dz0, variable_spacing_z):
+    """resample_MAS's argument checks (script/resampling_MAS_LOS.py); returns the temperature key."""
     if variable_spacing_z and dz0 > 1.0:
         raise ValueError(f"dz0={dz0:g} is extremely large in R_sun units. Did you mean something like 7e-4 instead of 7e4?")
     temp = "te" if "te" in model else "t"
@@ -62,6 +62,14 @@ def resample_MAS(model, N_pix, X_range, Y_range, N_z, dz0, variable_spacing_z=Tr
     for k in ("br", "bt", "bp"):
         if k not in model:
             raise ValueError("Magnetic field components (br, bt, bp) not all found!")
+    return temp
+
+
+def resample_MAS(model, N_pix, X_range, Y_range, N_z, dz0, variable_spacing_z=True, z_range=None,
+                 out_path="LOS_data.npz", save_plots=False, verbose=True, phi0_offset=0.0, r_min=R_MIN, context=None):
+    """Returns {'Ne_LOS','Te_LOS','B_LOS','ds_LOS' (N_pix,N_pix,N_z) [cm^-3, K, G, cm], 'x_coords',
+    'y_coords','z_coords' [m]} and writes them to `out_path` (script/resampling_MAS_LOS.py:288-300)."""
+    temp = _check_model(model, dz0, variable_spacing_z)
     ctx = context or _lib.default_context()
     zc, dz = z_grid(N_z, dz0, variable_spacing_z, z_range)
     xs = np.linspace(X_range[0], X_range[1], N_pix)
@@ -121,6 +129,44 @@ def SyntheticFF(fname_input, freq0, Nfreq, freq_log_step, fname_output=None, do_
     pol[dead] = 0.0
     result = {"emission_cube": emission.reshape(n_y, n_x, Nf), "emission_polVI_cube": pol.reshape(n_y, n_x, Nf),
               "frequencies_Hz": frequencies_Hz, "x_coords": x_coords, "y_coords": y_coords}
+    if fname_output is not None:
+        np.savez_compressed(str(fname_output) + ".npz", **result)
+    return result
+
+
+def render_los_map(model, N_pix, X_range, Y_range, N_z, dz0, freq0, Nfreq, freq_log_step, variable_spacing_z=True,
+                   z_range=None, phi0_offset=0.0, r_min=R_MIN, em_flag=5, s_max=30, use_bvec=False, diagnostics=False,
+                   fname_output=None, session=None):
+    """resample_MAS followed by SyntheticFF in one fused kernel: the same LOS geometry and samples, the same packing
+    rules and T_b / V/I, with nothing materialised (no LOS arrays, no Parms).  Returns (and writes to
+    ``fname_output + '.npz'``) SyntheticFF's dict.  Beyond the reference: em_flag (4 adds gyroresonance), use_bvec
+    (theta from the B vector instead of 90 deg) and diagnostics=True, which adds the keys of
+    workflow.diagnostic_maps (emission centroid, emission height, optical depths, the LOS's smallest r)."""
+    _check_model(model, dz0, variable_spacing_z)
+    if int(N_pix) < 2:
+        raise ValueError("N_pix must be >= 2 (the pixel area comes from the x spacing)")
+    if int(Nfreq) < 1:
+        raise ValueError("Nfreq must be >= 1")
+    zc, dz = z_grid(N_z, dz0, variable_spacing_z, z_range)
+    xs = np.linspace(X_range[0], X_range[1], N_pix)
+    ys = np.linspace(Y_range[0], Y_range[1], N_pix)
+    x_coords, y_coords = xs * R_sun_m, ys * R_sun_m
+    Nf = int(Nfreq)
+    frequencies_Hz = freq0 * (10.0 ** (freq_log_step * np.arange(Nf)))
+    pixel_size_cm = (x_coords[1] - x_coords[0]) / (R_sun_cm * 1e-2) * R_sun_cm
+    area = pixel_size_cm * pixel_size_cm
+    ses = session or RaySession(context=_lib.default_context())
+    ses.set_spherical_model(model)
+    out = ses.render_los_map(xs, ys, zc, dz * R_sun_cm, frequencies_Hz, phi0_offset=phi0_offset, r_min=r_min,
+                             z_eps=1e-6 / R_sun_m, pixel_area_cm2=area, em_flag=em_flag, s_max=s_max,
+                             use_bvec=use_bvec, diagnostics=diagnostics)
+    tb, vi = out[0], out[1]
+    result = {"emission_cube": np.ascontiguousarray(np.moveaxis(tb, 0, -1)),
+              "emission_polVI_cube": np.ascontiguousarray(np.moveaxis(vi, 0, -1)),
+              "frequencies_Hz": frequencies_Hz, "x_coords": x_coords, "y_coords": y_coords}
+    if diagnostics:
+        from .workflow import diagnostic_maps
+        result.update(diagnostic_maps({k: v.reshape(Nf, -1) for k, v in out[3].items()}, N_pix))
     if fname_output is not None:
         np.savez_compressed(str(fname_output) + ".npz", **result)
     return result

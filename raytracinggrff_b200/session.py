@@ -122,6 +122,32 @@ class RaySession:
         cubes.set_model_from_spherical(self, model, x_grid, y_grid, z_grid, phi0_offset, want_bvec)
         self.cube_shape = (len(x_grid), len(y_grid), len(z_grid))
 
+    def set_spherical_model(self, model):
+        """rtgrff_set_spherical_model for the five variables of a spherical model (a dict of cubes.SphericalVariable
+        with 'rho', 'te' (or 't'), 'br', 'bt', 'bp'): resident on the device for render_los_map.  A variable the
+        context already holds from these very arrays is not uploaded again (see _fingerprint)."""
+        temp = "te" if "te" in model else "t"
+        names = ("rho", temp, "br", "bt", "bp")
+        for name in names:
+            if name not in model:
+                raise ValueError(f"the spherical model has no '{name}' variable")
+        keys = self.ctx.__dict__.setdefault("_sph_keys", [None] * len(names))
+        for slot, name in enumerate(names):
+            var = model[name]
+            key = _fingerprint(var.data, var.phi, var.lat, var.r)
+            if key is not None:
+                key += (float(var.scale),)
+                if keys[slot] == key:
+                    continue
+            keys[slot] = None
+            data, phi, lat, r = f32(var.data), f64(var.phi), f64(var.lat), f64(var.r)
+            if data.shape != (len(phi), len(lat), len(r)):
+                raise ValueError(f"'{name}' data shape {data.shape} does not match its (phi, lat, r) mesh")
+            check(self._lib.rtgrff_set_spherical_model(self.ctx.handle, slot, ptr(data, c_float), ptr(phi, c_double),
+                                                       ptr(lat, c_double), ptr(r, c_double), *data.shape,
+                                                       float(var.scale)))
+            keys[slot] = key
+
     # -- integrator ----------------------------------------------------------------------------
     def trace(self, freq_hz, x_start, y_start, z_start, kvec_in_norm, dt, n_steps, record_stride=10,
               trace_crosssections=False, perturb_ratio=2.0, s_mode=_lib.S_PER_STEP, fetch=True):
@@ -419,5 +445,43 @@ class RaySession:
         st = {"nominal_ray_steps": int(stats[0]), "active_ray_steps": int(stats[1]),
               "pencil_steps": int(stats[2]), "valid_samples": int(stats[3])}
         if not diag:
+            return tb, vi, st
+        return tb, vi, st, (None if dg is None else dict(zip(_lib.DIAG_PLANES, dg)))
+
+    # -- fused straight line-of-sight map ---------------------------------------------------------
+    def render_los_map(self, x, y, zc, dz_cm, freq_hz, phi0_offset=0.0, r_min=0.9999999, z_eps=1e-6 / 6.957e8,
+                       pixel_area_cm2=1.0, em_flag=5, s_max=30, use_bvec=False, diagnostics=False,
+                       out_device_ptrs=None):
+        """Straight-LOS map from the model set_spherical_model left on the device (rtgrff_render_los_map): pixel
+        (i, j) at (x[j], y[i]) [R_sun], LOS samples at the cumulative offsets zc [R_sun] with segment lengths dz_cm
+        [cm], any list of frequencies [Hz].  Returns (tb, vi, stats), tb and vi (n_freq, ny, nx) float64, stats
+        {los_samples, valid_samples, voxel_freq_evaluations}; with diagnostics=True (tb, vi, stats, diag), diag a
+        dict of (n_freq, ny, nx) planes with render_map_diag's keys.  With out_device_ptrs=(tb_ptr, vi_ptr[,
+        diag_ptr]) the results go to those device buffers and the arrays returned are None."""
+        xs, ys, z, d = f64(x).ravel(), f64(y).ravel(), f64(zc).ravel(), f64(dz_cm).ravel()
+        fr = f64(np.atleast_1d(freq_hz)).ravel()
+        if len(d) != len(z):
+            raise ValueError("zc and dz_cm must have the same length")
+        nf, ny, nx = len(fr), len(ys), len(xs)
+        stats = (c_int64 * 3)()
+        tb = vi = dg = None
+        if out_device_ptrs is None:
+            tb = np.empty((nf, ny, nx), dtype=np.float64)
+            vi = np.empty_like(tb)
+            ptb, pvi, on_dev = tb.ctypes.data_as(ctypes.c_void_p), vi.ctypes.data_as(ctypes.c_void_p), 0
+            if diagnostics:
+                dg = np.empty((len(_lib.DIAG_PLANES), nf, ny, nx), dtype=np.float64)
+            pdg = None if dg is None else dg.ctypes.data_as(ctypes.c_void_p)
+        else:
+            if len(out_device_ptrs) != (3 if diagnostics else 2):
+                raise ValueError("out_device_ptrs must be (tb_ptr, vi_ptr) or, with diagnostics, (tb_ptr, vi_ptr, diag_ptr)")
+            ptb, pvi, on_dev = ctypes.c_void_p(out_device_ptrs[0]), ctypes.c_void_p(out_device_ptrs[1]), 1
+            pdg = ctypes.c_void_p(out_device_ptrs[2]) if diagnostics else None
+        check(self._lib.rtgrff_render_los_map(self.ctx.handle, nx, ny, ptr(xs, c_double), ptr(ys, c_double), len(z),
+                                              ptr(z, c_double), ptr(d, c_double), float(phi0_offset), float(r_min),
+                                              float(z_eps), nf, ptr(fr, c_double), float(pixel_area_cm2), int(em_flag),
+                                              int(s_max), int(bool(use_bvec)), ptb, pvi, pdg, on_dev, stats))
+        st = {"los_samples": int(stats[0]), "valid_samples": int(stats[1]), "voxel_freq_evaluations": int(stats[2])}
+        if not diagnostics:
             return tb, vi, st
         return tb, vi, st, (None if dg is None else dict(zip(_lib.DIAG_PLANES, dg)))
