@@ -13,17 +13,17 @@
 
 // Threads per block / minimum resident blocks per SM of the per-ray kernels (tuned on B200, see
 // profiles/): one thread per ray, small blocks so that finished warps free their slots early.
-#ifndef RT_BLOCK
 #define RT_BLOCK 64
-#endif
-#ifndef RT_MINB
 #define RT_MINB 8
-#endif
 
 namespace rtgrff {
 
 // build_rays.py:29-32 (C / R_S with the reference's rounded constants)
 constexpr double kC_R = 2.998e10 / 6.96e10;
+
+// Streams the per-frequency launches of the fused map go round-robin over.  The launches must overlap: each ends
+// on a tail of half-empty SMs that the next one fills (DESIGN.md 4.1: one stream 514 ms, two or more 461 ms).
+constexpr int kMapForkStreams = 8;
 
 // Uniform-grid geometry of a cube.  x0/xl are the first/last node (scipy bounds test,
 // build_rays.py:140), inv_d = 1/mean step (gpu_raytrace.py:21-33).
@@ -91,9 +91,9 @@ struct rtgrff_ctx {
     int pipeline = 1;                // chunked pinned host pipelines on (RTGRFF_PIPELINE, rtgrff_ctx_set_pipeline)
     cudaStream_t copy_stream = nullptr;
     cudaEvent_t chunk_ev[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};   // in[2], kernel[2], out[2]
-    // fork / join of the per-frequency launches of the fused map (RT_FREQ_PER_LAUNCH = 1)
-    cudaStream_t fstream[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
-    cudaEvent_t fev[9] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
+    // fork / join of the per-frequency launches of the fused map: one event per fork stream, the last one forks
+    cudaStream_t fstream[rtgrff::kMapForkStreams] = {};
+    cudaEvent_t fev[rtgrff::kMapForkStreams + 1] = {};
     void *pinned[4] = {nullptr, nullptr, nullptr, nullptr};
     size_t pinned_cap[4] = {0, 0, 0, 0};
     int64_t launches = 0;

@@ -22,8 +22,9 @@
 namespace rtgrff {
 
 // Everything that depends on the frequency only, prepared on the host and passed BY VALUE inside
-// the kernel parameters (constant bank, indexed by blockIdx.y): the ~20 registers these constants
-// used to occupy per thread were spilled around the record-time code.
+// the kernel parameters: the ~20 registers these constants used to occupy per thread were spilled
+// around the record-time code.  One launch per frequency, so that they sit at fixed offsets of the
+// constant bank and become instruction operands.
 struct FreqDev {
     double nu, omega0, dt;
     int64_t n_steps, stride;
@@ -32,18 +33,6 @@ struct FreqDev {
     FreqC fq;
 };
 
-// RT_FREQ_PER_LAUNCH = 1: one launch per frequency (on a few streams, so that the launches still overlap): the
-// per-frequency constants then sit at fixed offsets of the constant bank and become instruction operands, where
-// the multi-frequency launch indexes them with blockIdx.y (an LDC with a register index in the inner loops).
-#ifndef RT_FREQ_PER_LAUNCH
-#define RT_FREQ_PER_LAUNCH 1
-#endif
-constexpr int kMaxFreqPerLaunch = RT_FREQ_PER_LAUNCH;
-
-#ifndef RT_PREFETCH
-#define RT_PREFETCH 0     // 1: L1 prefetch of the sampler's lines one step ahead (A/B)
-#endif
-
 struct MapArgs {
     RayCube cube;
     const float4 *fcube, *bcube;
@@ -51,8 +40,7 @@ struct MapArgs {
     int64_t n_rays;
     const double *x_start, *y_start, *z_start, *kvec;
     const int *ray_order;                // thread t handles ray ray_order[t] (nullptr: t); see rtgrff.h
-    int n_freq;                          // <= kMaxFreqPerLaunch
-    FreqDev freqs[kMaxFreqPerLaunch];
+    FreqDev freq;                        // the frequency of this launch
     double perturb_ratio, area;
     float r_sun_cm, fill_ne, fill_te, fill_b;
     int em_flag, s_max, use_bvec, order, cs_every_step;
@@ -268,11 +256,10 @@ __global__ void __launch_bounds__(RT_BLOCK, RT_MINB) render_map_kernel(const Map
 {
     constexpr bool NEED_BETWEEN = BVEC || GR;
     const int64_t slot = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    const int fi = (kMaxFreqPerLaunch == 1) ? 0 : (int)blockIdx.y;
     const bool has_ray = slot < a.n_rays;
     const int64_t ray = (has_ray && a.ray_order) ? (int64_t)a.ray_order[slot] : slot;
     const RayCube &C = a.cube;
-    const FreqDev &fp = a.freqs[fi];
+    const FreqDev &fp = a.freq;
     const StepConst &K = fp.K;
     const FreqC &fq = fp.fq;
     Cell cache;
@@ -309,30 +296,6 @@ __global__ void __launch_bounds__(RT_BLOCK, RT_MINB) render_map_kernel(const Map
     bool tail_done = !has_ray;            // a frozen ray repeats the same record: ds = 0 -> empty voxel
 
     for (int i = 0; i < n_steps; ++i) {
-#if RT_PREFETCH
-        // the record taken after this step samples the field cubes in (or next to) the cell the ray is in now: ask L1
-        // for those lines a whole step ahead (with a record at every step they are still there from the last one)
-        if (stride > 1 && i == next_rec && alive) {
-            int ci, cj, ck;
-            float ftx, fty, ftz;
-            if (cell_of(a.fg, (float)s.rx, (float)s.ry, (float)s.rz, ci, cj, ck, ftx, fty, ftz)) {
-                const size_t sy = (size_t)a.fg.nz, sx = (size_t)a.fg.ny * a.fg.nz;
-                const size_t off = (size_t)ci * sx + (size_t)cj * sy + (size_t)ck;
-                const float4 *p0 = a.fcube + off;
-                asm volatile("prefetch.global.L1 [%0];" ::"l"(p0));
-                asm volatile("prefetch.global.L1 [%0];" ::"l"(p0 + sy));
-                asm volatile("prefetch.global.L1 [%0];" ::"l"(p0 + sx));
-                asm volatile("prefetch.global.L1 [%0];" ::"l"(p0 + sx + sy));
-                if (BVEC) {
-                    const float4 *p1 = a.bcube + off;
-                    asm volatile("prefetch.global.L1 [%0];" ::"l"(p1));
-                    asm volatile("prefetch.global.L1 [%0];" ::"l"(p1 + sy));
-                    asm volatile("prefetch.global.L1 [%0];" ::"l"(p1 + sx));
-                    asm volatile("prefetch.global.L1 [%0];" ::"l"(p1 + sx + sy));
-                }
-            }
-        }
-#endif
         if (alive) {
             const bool want_s = CS && (i == next_rec || a.cs_every_step || cumulative);
             alive = advance_ray<CS, MODE>(C, K, cache, s, fp.dt, a.perturb_ratio, want_s, s_step);

@@ -14,8 +14,12 @@
 //    ~1e-3 R_sun, so the per-step error is ~1e-10 R_sun and random.
 //  * The cached cell lives in 32 registers as the coefficients of its trilinear polynomial
 //        f = (a0 + az z) + y (ay + ayz z) + x ((ax + axz z) + y (axy + axyz z))
-//    for the channel pairs {omega_pe, d/dx} and {d/dy, d/dz}: one RHS is 14 packed FFMA2 with a
+//    for the channel pairs {omega_pe, d/dz} and {d/dx, d/dy}: one RHS is 14 packed FFMA2 with a
 //    dependency depth of 3 (nested lerps: 14 FMUL2 + 14 FFMA2, depth 6).
+//  * The x,y components of every vector of a stage (position offsets, k, v, g and the RK4 sums)
+//    live in register pairs and are updated with packed FP32x2 instructions (FFMA2 / FMUL2 / FADD2
+//    take a scalar broadcast operand, so nothing has to be duplicated): 15 instead of 22
+//    instructions in the tail of an RHS.
 //  * Fast path of an RHS = one range test (VIMNMX3.U32 + ISETP on the bit patterns: 0 <= t < 1)
 //    + the evaluation, ~55 instructions.  Everything else — leaving the cell, the cube bounds,
 //    the re-fetch — is the slow path (move_cell), which 1-5 of a warp's 32 lanes take at a time:
@@ -29,30 +33,15 @@
 
 #include "ray_integrator.cuh"
 
-// RT_PACK_TAIL = 1: the x,y components of every vector of a stage (position offsets, k, v, g and the RK4 sums)
-// live in register pairs and are updated with packed FP32x2 instructions (FFMA2 / FMUL2 / FADD2 take a scalar
-// broadcast operand, so nothing has to be duplicated): 15 instead of 22 instructions in the tail of an RHS.
-#ifndef RT_PACK_TAIL
-#define RT_PACK_TAIL 1
-#endif
-#ifndef RT_UNROLL_Q
-#define RT_UNROLL_Q 0     // 1: the three rays of a pencil step as three inlined copies of the RK4 (A/B)
-#endif
-
 namespace rtgrff {
 
 // The cached cell: element offset of its (i,j,k) corner (-1 = empty), its integer coordinates and
-// the polynomial coefficients of the channel pairs L = {omega_pe, d/dx}, H = {d/dy, d/dz}.
+// the polynomial coefficients of the channel pairs L = {omega_pe, d/dz}, H = {d/dx, d/dy}.
 struct Cell {
     int off;
     int ci, cj, ck;
     float2 l0, lz, ly, lyz, lx, lxz, lxy, lxyz;
     float2 h0, hz, hy, hyz, hx, hxz, hxy, hxyz;
-};
-
-struct Deriv32 {
-    float vx, vy, vz;   // k / omega            (dr/dt = C_R * v)
-    float gx, gy, gz;   // (omega_pe/omega) * grad omega_pe   (dk/dt = -C_R * g)
 };
 
 __device__ __forceinline__ float2 sub2(float2 a, float2 b) { return __fadd2_rn(a, make_float2(-b.x, -b.y)); }
@@ -73,15 +62,10 @@ __device__ __forceinline__ void cell_poly(const float4 &c000, const float4 &c001
         c.ax = sub2(LO(c100), LO(c000)); c.axz = sub2(d10, d00);                                  \
         c.axy = sub2(y1, y0); c.axyz = sub2(yz1, yz0);                                            \
     }
-#if RT_PACK_TAIL
     // channel pairs L = {omega_pe, d/dz}, H = {d/dx, d/dy}: the x,y components of the gradient come out of the
     // evaluation as one register pair, ready for the packed (FFMA2) stage updates of step32
 #define RT_LO(c) make_float2((c).x, (c).w)
 #define RT_HI(c) make_float2((c).y, (c).z)
-#else
-#define RT_LO(c) make_float2((c).x, (c).y)
-#define RT_HI(c) make_float2((c).z, (c).w)
-#endif
     RT_POLY(RT_LO, l0, lz, ly, lyz, lx, lxz, lxy, lxyz)
     RT_POLY(RT_HI, h0, hz, hy, hyz, hx, hxz, hxy, hxyz)
 #undef RT_POLY
@@ -183,55 +167,17 @@ __device__ __forceinline__ bool move_cell(const RayCube &C, Cell &c, bool edge, 
     return true;
 }
 
-// One RHS evaluation at p + d, all in cell units relative to the CACHED cell: p is the step's base
-// position (rebased when the cache moves), d the offset of this stage of this ray from it.  The
-// common case — the point is inside the cached cell — costs one range test; the cell change, the
-// bounds of the cube and the re-fetch all live on the slow path.
-__device__ __forceinline__ Deriv32 rhs32(const RayCube &C, Cell &cache, bool edge, float &px, float &py, float &pz,
-                                         float dx, float dy, float dz, float kx, float ky, float kz)
-{
-    Deriv32 d;
-    float tx = px + dx, ty = py + dy, tz = pz + dz;
-    if (!(in_unit(tx) & in_unit(ty) & in_unit(tz))) {
-        if (!move_cell(C, cache, edge, px, py, pz, tx, ty, tz)) {
-            d.vx = d.vy = d.vz = d.gx = d.gy = d.gz = 0.0f;
-            return d;
-        }
-    }
-    const float2 tz2 = make_float2(tz, tz), ty2 = make_float2(ty, ty), tx2 = make_float2(tx, tx);
-    // {omega_pe, d/dx}
-    const float2 wg = __ffma2_rn(
-        __ffma2_rn(__ffma2_rn(cache.lxyz, tz2, cache.lxy), ty2, __ffma2_rn(cache.lxz, tz2, cache.lx)), tx2,
-        __ffma2_rn(__ffma2_rn(cache.lyz, tz2, cache.ly), ty2, __ffma2_rn(cache.lz, tz2, cache.l0)));
-    // {d/dy, d/dz}
-    const float2 gg = __ffma2_rn(
-        __ffma2_rn(__ffma2_rn(cache.hxyz, tz2, cache.hxy), ty2, __ffma2_rn(cache.hxz, tz2, cache.hx)), tx2,
-        __ffma2_rn(__ffma2_rn(cache.hyz, tz2, cache.hy), ty2, __ffma2_rn(cache.hz, tz2, cache.h0)));
-    const float w = wg.x;
-    const float om2 = fmaf(w, w, fmaf(kx, kx, fmaf(ky, ky, kz * kz)));
-    float inv_om;
-    asm("rsqrt.approx.ftz.f32 %0, %1;" : "=f"(inv_om) : "f"(om2));   // MUFU.RSQ, 2 ulp; omega^2 ~ 1e17
-    const float a = w * inv_om;
-    d.vx = kx * inv_om; d.vy = ky * inv_om; d.vz = kz * inv_om;
-    d.gx = a * wg.y; d.gy = a * gg.x; d.gz = a * gg.y;
-    // valid = isfinite(omega_pe) & isfinite(omega) & (omega > 0)   (build_rays.py:169); a non-finite
-    // omega_pe or k makes omega^2 non-finite, so one range test on omega^2 covers all three:
-    // 0 < omega^2 < inf  <=>  bit pattern in [1, 0x7f7fffff].  The invalid stage (a zero derivative) is the
-    // rare case: the zeros are written on that branch only, not materialised ahead of every evaluation.
-    if (__builtin_expect(__float_as_uint(om2) - 1u >= 0x7f7fffffu, 0)) d.vx = d.vy = d.vz = d.gx = d.gy = d.gz = 0.0f;
-    return d;
-}
-
-
-#if RT_PACK_TAIL
 struct Deriv32P {
-    float2 vxy; float vz;   // k / omega
-    float2 gxy; float gz;   // (omega_pe/omega) * grad omega_pe
+    float2 vxy; float vz;   // k / omega                          (dr/dt = C_R * v)
+    float2 gxy; float gz;   // (omega_pe/omega) * grad omega_pe   (dk/dt = -C_R * g)
 };
 
 __device__ __forceinline__ float2 bc2(float v) { return make_float2(v, v); }
 
-// rhs32 with the x,y components in register pairs (cell channel pairs L = {omega_pe, d/dz}, H = {d/dx, d/dy}).
+// One RHS evaluation at p + d, all in cell units relative to the CACHED cell: p is the step's base
+// position (rebased when the cache moves), d the offset of this stage of this ray from it; the x,y
+// components in register pairs.  The common case — the point is inside the cached cell — costs one
+// range test; the cell change, the bounds of the cube and the re-fetch all live on the slow path.
 __device__ __forceinline__ Deriv32P rhs32p(const RayCube &C, Cell &cache, bool edge, float2 &pxy, float &pz, float2 dxy, float dz,
                                            float2 kxy, float kz)
 {
@@ -260,13 +206,15 @@ __device__ __forceinline__ Deriv32P rhs32p(const RayCube &C, Cell &cache, bool e
     const float a = w * inv_om;
     d.vxy = __fmul2_rn(kxy, bc2(inv_om)); d.vz = kz * inv_om;
     d.gxy = __fmul2_rn(gg, bc2(a)); d.gz = a * wz.y;
-    // validity as in rhs32: the zeros are written on the rare branch only
+    // valid = isfinite(omega_pe) & isfinite(omega) & (omega > 0)   (build_rays.py:169); a non-finite
+    // omega_pe or k makes omega^2 non-finite, so one range test on omega^2 covers all three:
+    // 0 < omega^2 < inf  <=>  bit pattern in [1, 0x7f7fffff].  The invalid stage (a zero derivative) is the
+    // rare case: the zeros are written on that branch only, not materialised ahead of every evaluation.
     if (__builtin_expect(__float_as_uint(om2) - 1u >= 0x7f7fffffu, 0)) {
         d.vxy = make_float2(0.0f, 0.0f); d.gxy = make_float2(0.0f, 0.0f); d.vz = d.gz = 0.0f;
     }
     return d;
 }
-#endif
 
 // Largest distance, in cells, between the master position of a step and any stage of any of its
 // three rays (|v| <= 1: a full step plus the pencil offset eps = perturb * step).  The FP32 stepper
@@ -342,7 +290,6 @@ __device__ __forceinline__ bool step32(const RayCube &C, const StepConst &K, Cel
     float px = (float)(fx - (double)cache.ci), py = (float)(fy - (double)cache.cj), pz = (float)(fz - (double)cache.ck);
     const float kx = (float)s.kx, ky = (float)s.ky, kz = (float)s.kz;
     const int n_rays = (CS && want_s) ? 3 : 1;
-#if RT_PACK_TAIL
     float2 pxy = make_float2(px, py);
     const float2 kxy = make_float2(kx, ky);
     const float2 ixy = make_float2(K.ix, K.iy), h1xy = make_float2(K.hx, K.hy), h2xy = make_float2(2.0f * K.hx, 2.0f * K.hy);
@@ -353,11 +300,7 @@ __device__ __forceinline__ bool step32(const RayCube &C, const StepConst &K, Cel
     float tx = 0.0f, ty = 0.0f, tz = 0.0f, e2x = 0.0f, e2y = 0.0f, e2z = 0.0f, eps = 0.0f;
     float d1x = 0.0f, d1y = 0.0f, d1z = 0.0f;
     bool moved = false;
-#if RT_UNROLL_Q
-#pragma unroll
-#else
 #pragma unroll 1
-#endif
     for (int q = 0; q < n_rays; ++q) {
         const float2 qxy = __fmul2_rn(oxy, ixy);                      // start of this ray relative to p, cells
         const float qz = oz * K.iz;
@@ -366,7 +309,7 @@ __device__ __forceinline__ bool step32(const RayCube &C, const StepConst &K, Cel
 #pragma unroll          // the four stages unrolled (constant weights), the three rays of a step rolled
         for (int st = 0; st < 4; ++st) {
             const Deriv32P d = rhs32p(C, cache, edge, pxy, pz, dxy, dz, skxy, skz);
-            if (st == 0) {
+            if (st == 0) {        // (0 + x is not x for x = -0: spelled out, the compiler would keep the FADDs)
                 avxy = d.vxy; avz = d.vz; agxy = d.gxy; agz = d.gz;
             } else {
                 const float w = (st == 3) ? 1.0f : 2.0f;
@@ -386,6 +329,8 @@ __device__ __forceinline__ bool step32(const RayCube &C, const StepConst &K, Cel
             s.rx = fma((double)avx, K.c6, s.rx); s.ry = fma((double)avy, K.c6, s.ry); s.rz = fma((double)avz, K.c6, s.rz);
             cvxy = avxy; cvz = avz;
             if (n_rays > 1) {
+                // norms through MUFU.RSQ (2 ulp): S is held to 1e-4, and the reference's +1e-32 / +1e-30
+                // guards only matter for a ray that did not move, whose S is NaN either way
                 const float dx = K.c6r * avx, dy = K.c6r * avy, dz2 = K.c6r * avz;
                 const float d2 = fmaf(dx, dx, fmaf(dy, dy, dz2 * dz2));
                 const float inv = rsqrtf(d2);
@@ -414,69 +359,6 @@ __device__ __forceinline__ bool step32(const RayCube &C, const StepConst &K, Cel
             }
         }
     }
-#else
-    float ox = 0.0f, oy = 0.0f, oz = 0.0f;          // displacement of the current ray from the central one, R_sun
-    float cvx = 0.0f, cvy = 0.0f, cvz = 0.0f;       // central ray: sum of v over the stages
-    float tx = 0.0f, ty = 0.0f, tz = 0.0f, e2x = 0.0f, e2y = 0.0f, e2z = 0.0f, eps = 0.0f;
-    float d1x = 0.0f, d1y = 0.0f, d1z = 0.0f;
-    bool moved = false;
-#pragma unroll 1
-    for (int q = 0; q < n_rays; ++q) {
-        const float qx = ox * K.ix, qy = oy * K.iy, qz = oz * K.iz;    // start of this ray relative to p, cells
-        float dx = qx, dy = qy, dz = qz, skx = kx, sky = ky, skz = kz;
-        float avx = 0.0f, avy = 0.0f, avz = 0.0f, agx = 0.0f, agy = 0.0f, agz = 0.0f;   // k1 + 2 k2 + 2 k3 + k4
-#pragma unroll          // the four stages unrolled (constant weights), the three rays of a step rolled
-        for (int st = 0; st < 4; ++st) {
-            const Deriv32 d = rhs32(C, cache, edge, px, py, pz, dx, dy, dz, skx, sky, skz);
-            if (st == 0) {        // (0 + x is not x for x = -0: spelled out, the compiler would keep six FADDs)
-                avx = d.vx; avy = d.vy; avz = d.vz; agx = d.gx; agy = d.gy; agz = d.gz;
-            } else {
-                const float w = (st == 3) ? 1.0f : 2.0f;
-                avx = fmaf(w, d.vx, avx); avy = fmaf(w, d.vy, avy); avz = fmaf(w, d.vz, avz);
-                agx = fmaf(w, d.gx, agx); agy = fmaf(w, d.gy, agy); agz = fmaf(w, d.gz, agz);
-            }
-            const float a = (st < 2) ? 1.0f : 2.0f;   // stages 2, 3 at dt/2, stage 4 at dt (K.h* are half steps)
-            dx = fmaf(a * K.hx, d.vx, qx); dy = fmaf(a * K.hy, d.vy, qy); dz = fmaf(a * K.hz, d.vz, qz);
-            const float ak = -a * K.hk;
-            skx = fmaf(ak, d.gx, kx); sky = fmaf(ak, d.gy, ky); skz = fmaf(ak, d.gz, kz);
-        }
-        if (q == 0) {
-            moved = (fabsf(avx) + fabsf(avy) + fabsf(avz) + fabsf(agx) + fabsf(agy) + fabsf(agz)) != 0.0f;
-            s.kx = fma((double)agx, -K.c6, s.kx); s.ky = fma((double)agy, -K.c6, s.ky); s.kz = fma((double)agz, -K.c6, s.kz);
-            s.rx = fma((double)avx, K.c6, s.rx); s.ry = fma((double)avy, K.c6, s.ry); s.rz = fma((double)avz, K.c6, s.rz);
-            cvx = avx; cvy = avy; cvz = avz;
-            if (n_rays > 1) {
-                // norms through MUFU.RSQ (2 ulp): S is held to 1e-4, and the reference's +1e-32 / +1e-30
-                // guards only matter for a ray that did not move, whose S is NaN either way
-                const float dx = K.c6r * cvx, dy = K.c6r * cvy, dz = K.c6r * cvz;
-                const float d2 = fmaf(dx, dx, fmaf(dy, dy, dz * dz));
-                const float inv = rsqrtf(d2);
-                const float nrd = d2 * inv;
-                tx = dx * inv; ty = dy * inv; tz = dz * inv;
-                // reference axis: z if |t_z| < 0.9 else y (build_rays.py:188-194); e1 = a x t, e2 = t x e1
-                const bool use_z = fabsf(tz) < 0.9f;
-                float e1x = use_z ? -ty : tz, e1y = use_z ? tx : 0.0f, e1z = use_z ? 0.0f : -tx;
-                const float n1 = rsqrtf(fmaf(e1x, e1x, fmaf(e1y, e1y, e1z * e1z)));
-                e1x *= n1; e1y *= n1; e1z *= n1;
-                e2x = ty * e1z - tz * e1y; e2y = tz * e1x - tx * e1z; e2z = tx * e1y - ty * e1x;
-                const float n2 = rsqrtf(fmaf(e2x, e2x, fmaf(e2y, e2y, e2z * e2z)));
-                e2x *= n2; e2y *= n2; e2z *= n2;
-                eps = K.perturb * nrd;
-                ox = eps * e1x; oy = eps * e1y; oz = eps * e1z;
-            }
-        } else {
-            const float ddx = fmaf(K.c6r, avx - cvx, ox), ddy = fmaf(K.c6r, avy - cvy, oy),
-                        ddz = fmaf(K.c6r, avz - cvz, oz);
-            if (q == 1) {
-                d1x = ddx; d1y = ddy; d1z = ddz;
-                ox = eps * e2x; oy = eps * e2y; oz = eps * e2z;
-            } else {
-                const float cx = d1y * ddz - d1z * ddy, cy = d1z * ddx - d1x * ddz, cz = d1x * ddy - d1y * ddx;
-                s_step = __fdividef(fabsf(fmaf(cx, tx, fmaf(cy, ty, cz * tz))), eps * eps);
-            }
-        }
-    }
-#endif
     return moved;
 }
 

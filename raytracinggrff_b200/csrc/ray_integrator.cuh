@@ -39,9 +39,8 @@ __device__ __forceinline__ bool in_cube(const RayCube &C, double x, double y, do
 __device__ __forceinline__ float lerpf(float a, float b, float t) { return fmaf(t, b - a, a); }
 __device__ __forceinline__ double lerpd(double a, double b, double t) { return fma(t, b - a, a); }
 
-// One RHS evaluation (build_rays.py:158-175).  LERP64: trilinear arithmetic in FP64 (else FP32 on
-// the FP32-stored corners; position, cell fraction, omega and the derivative stay FP64).
-template <bool LERP64>
+// One RHS evaluation (build_rays.py:158-175): trilinear arithmetic in FP32 on the FP32-stored corners;
+// position, cell fraction, omega and the derivative stay FP64.
 __device__ __forceinline__ void rhs_eval(const RayCube &C, const State &s, State &d)
 {
     d.rx = d.ry = d.rz = d.kx = d.ky = d.kz = 0.0;
@@ -54,21 +53,12 @@ __device__ __forceinline__ void rhs_eval(const RayCube &C, const State &s, State
     const float4 c010 = __ldg(p + C.sy), c011 = __ldg(p + C.sy + 1);
     const float4 c100 = __ldg(p + C.sx), c101 = __ldg(p + C.sx + 1);
     const float4 c110 = __ldg(p + C.sx + C.sy), c111 = __ldg(p + C.sx + C.sy + 1);
-    double w, gx, gy, gz;
-    if (LERP64) {
-#define RT_TRI64(m)                                                                               \
-    lerpd(lerpd(lerpd((double)c000.m, (double)c001.m, tz), lerpd((double)c010.m, (double)c011.m, tz), ty), \
-          lerpd(lerpd((double)c100.m, (double)c101.m, tz), lerpd((double)c110.m, (double)c111.m, tz), ty), tx)
-        w = RT_TRI64(x); gx = RT_TRI64(y); gy = RT_TRI64(z); gz = RT_TRI64(w);
-#undef RT_TRI64
-    } else {
-        const float ftx = (float)tx, fty = (float)ty, ftz = (float)tz;
+    const float ftx = (float)tx, fty = (float)ty, ftz = (float)tz;
 #define RT_TRI32(m)                                                                               \
     lerpf(lerpf(lerpf(c000.m, c001.m, ftz), lerpf(c010.m, c011.m, ftz), fty),                     \
           lerpf(lerpf(c100.m, c101.m, ftz), lerpf(c110.m, c111.m, ftz), fty), ftx)
-        w = (double)RT_TRI32(x); gx = (double)RT_TRI32(y); gy = (double)RT_TRI32(z); gz = (double)RT_TRI32(w);
+    const double w = (double)RT_TRI32(x), gx = (double)RT_TRI32(y), gy = (double)RT_TRI32(z), gz = (double)RT_TRI32(w);
 #undef RT_TRI32
-    }
     const double om = sqrt(w * w + ((s.kx * s.kx + s.ky * s.ky) + s.kz * s.kz));
     // valid = isfinite(omega_pe) & isfinite(omega) & (omega > 0); gradients are NOT tested (build_rays.py:169)
     if (!(isfinite(w) && isfinite(om) && om > 0.0)) return;
@@ -87,14 +77,13 @@ __device__ __forceinline__ State axpy(const State &s, double h, const State &d)
 }
 
 // Classic RK4 (build_rays.py:177-182).
-template <bool LERP64>
 __device__ __forceinline__ State rk4_step(const RayCube &C, const State &s, double dt)
 {
     State k1, k2, k3, k4;
-    rhs_eval<LERP64>(C, s, k1);
-    rhs_eval<LERP64>(C, axpy(s, 0.5 * dt, k1), k2);
-    rhs_eval<LERP64>(C, axpy(s, 0.5 * dt, k2), k3);
-    rhs_eval<LERP64>(C, axpy(s, dt, k3), k4);
+    rhs_eval(C, s, k1);
+    rhs_eval(C, axpy(s, 0.5 * dt, k1), k2);
+    rhs_eval(C, axpy(s, 0.5 * dt, k2), k3);
+    rhs_eval(C, axpy(s, dt, k3), k4);
     const double c6 = dt / 6.0;
     State o;
     o.rx = fma(c6, (k1.rx + 2.0 * k2.rx) + 2.0 * k3.rx + k4.rx, s.rx);
@@ -108,7 +97,6 @@ __device__ __forceinline__ State rk4_step(const RayCube &C, const State &s, doub
 
 // Cross-section ratio of one step (build_rays.py:209-239): two rays displaced by eps along the
 // pencil basis (e1,e2) _|_ t_hat, same k0, one RK4 step each; S = |(d1 x d2).t_hat| / eps^2.
-template <bool LERP64>
 __device__ __forceinline__ double cross_section_ratio(const RayCube &C, const State &s0, const State &s1,
                                                       double dt, double perturb_ratio)
 {
@@ -128,8 +116,8 @@ __device__ __forceinline__ double cross_section_ratio(const RayCube &C, const St
     State p1 = s0, p2 = s0;
     p1.rx = fma(eps, e1x, s0.rx); p1.ry = fma(eps, e1y, s0.ry); p1.rz = fma(eps, e1z, s0.rz);
     p2.rx = fma(eps, e2x, s0.rx); p2.ry = fma(eps, e2y, s0.ry); p2.rz = fma(eps, e2z, s0.rz);
-    const State q1 = rk4_step<LERP64>(C, p1, dt);
-    const State q2 = rk4_step<LERP64>(C, p2, dt);
+    const State q1 = rk4_step(C, p1, dt);
+    const State q2 = rk4_step(C, p2, dt);
     const double d1x = q1.rx - s1.rx, d1y = q1.ry - s1.ry, d1z = q1.rz - s1.rz;
     const double d2x = q2.rx - s1.rx, d2y = q2.ry - s1.ry, d2z = q2.rz - s1.rz;
     const double cx = d1y * d2z - d1z * d2y, cy = d1z * d2x - d1x * d2z, cz = d1x * d2y - d1y * d2x;

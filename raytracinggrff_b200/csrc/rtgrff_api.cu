@@ -69,6 +69,26 @@ static int geom_from(const double g[12], int nx, int ny, int nz, GridGeom &o)
     return RTGRFF_OK;
 }
 
+// The float32 view of a geometry geom_from accepted, for the samplers.
+static GridGeomF geomf_from(const double g[12], int nx, int ny, int nz)
+{
+    GridGeomF f;
+    f.nx = nx; f.ny = ny; f.nz = nz;
+    f.x0 = (float)g[0]; f.y0 = (float)g[4]; f.z0 = (float)g[8];
+    f.idx = (float)(1.0 / g[1]); f.idy = (float)(1.0 / g[5]); f.idz = (float)(1.0 / g[9]);
+    f.fxl = (float)(nx - 1); f.fyl = (float)(ny - 1); f.fzl = (float)(nz - 1);
+    return f;
+}
+
+// The node coordinates of a spherical mesh must ascend strictly along every axis.
+static int check_ascending_nodes(const double *phi, int np, const double *lat, int nt, const double *r, int nr)
+{
+    for (int i = 1; i < np; ++i) if (!(phi[i] > phi[i - 1])) return fail(RTGRFF_EINVAL, "phi nodes must ascend");
+    for (int i = 1; i < nt; ++i) if (!(lat[i] > lat[i - 1])) return fail(RTGRFF_EINVAL, "latitude nodes must ascend");
+    for (int i = 1; i < nr; ++i) if (!(r[i] > r[i - 1])) return fail(RTGRFF_EINVAL, "radius nodes must ascend");
+    return RTGRFF_OK;
+}
+
 static RayCube ray_cube_of(const rtgrff_ctx *c)
 {
     RayCube r;
@@ -376,18 +396,6 @@ static int grff64()
     return v;
 }
 
-static int trace_variant()
-{
-    // RTGRFF_MODE selects the ray stepper: 0 (default) FP64 master state + FP32 cell-relative RHS with a
-    // register cell cache; 1 FP64 state and RHS, FP32 trilinear arithmetic; 2 FP64 everything.
-    static int v = -1;
-    if (v < 0) {
-        const char *e = getenv("RTGRFF_MODE");
-        v = (e && e[0] >= '0' && e[0] <= '2') ? (e[0] - '0') : 0;
-    }
-    return v;
-}
-
 }  // namespace rtgrff
 
 using namespace rtgrff;
@@ -582,11 +590,7 @@ int rtgrff_set_field_cubes(rtgrff_ctx *c, const float *ne, const float *te, cons
         RT_TRY(launched(c, "interleave3_kernel"));
     }
     c->fgeom = g;
-    GridGeomF &f = c->fgeomf;
-    f.nx = nx; f.ny = ny; f.nz = nz;
-    f.x0 = (float)geom[0]; f.y0 = (float)geom[4]; f.z0 = (float)geom[8];
-    f.idx = (float)(1.0 / geom[1]); f.idy = (float)(1.0 / geom[5]); f.idz = (float)(1.0 / geom[9]);
-    f.fxl = (float)(nx - 1); f.fyl = (float)(ny - 1); f.fzl = (float)(nz - 1);
+    c->fgeomf = geomf_from(geom, nx, ny, nz);
     c->has_fcube = true;
     c->has_bvec = bvec;
     RT_CUDA(cudaStreamSynchronize(c->stream));
@@ -605,9 +609,7 @@ int rtgrff_resample_spherical(rtgrff_ctx *c, int slot, const float *data, const 
     if (np < 2 || nt < 2 || nr < 2) return fail(RTGRFF_EINVAL, "spherical mesh needs >= 2 nodes per axis");
     GridGeom g;
     RT_TRY(geom_from(geom, nx, ny, nz, g));
-    for (int i = 1; i < np; ++i) if (!(phi[i] > phi[i - 1])) return fail(RTGRFF_EINVAL, "phi nodes must ascend");
-    for (int i = 1; i < nt; ++i) if (!(lat[i] > lat[i - 1])) return fail(RTGRFF_EINVAL, "latitude nodes must ascend");
-    for (int i = 1; i < nr; ++i) if (!(r[i] > r[i - 1])) return fail(RTGRFF_EINVAL, "radius nodes must ascend");
+    RT_TRY(check_ascending_nodes(phi, np, lat, nt, r, nr));
     if (c->slot_nx && (c->slot_nx != nx || c->slot_ny != ny || c->slot_nz != nz))
         for (bool &b : c->slot_set) b = false;           // a new cube shape invalidates the other slots
     const size_t nvox = (size_t)nx * ny * nz, nd = (size_t)np * nt * nr;
@@ -657,9 +659,7 @@ int rtgrff_sample_spherical_los(rtgrff_ctx *c, const float *data, const double *
     RT_USE(c);
     if (!data || !phi || !lat || !r || !x || !y || !zc || !out) return fail(RTGRFF_EINVAL, "null argument");
     if (np < 2 || nt < 2 || nr < 2 || nx < 1 || ny < 1 || nz < 1) return fail(RTGRFF_EINVAL, "bad sizes");
-    for (int i = 1; i < np; ++i) if (!(phi[i] > phi[i - 1])) return fail(RTGRFF_EINVAL, "phi nodes must ascend");
-    for (int i = 1; i < nt; ++i) if (!(lat[i] > lat[i - 1])) return fail(RTGRFF_EINVAL, "latitude nodes must ascend");
-    for (int i = 1; i < nr; ++i) if (!(r[i] > r[i - 1])) return fail(RTGRFF_EINVAL, "radius nodes must ascend");
+    RT_TRY(check_ascending_nodes(phi, np, lat, nt, r, nr));
     const size_t total = (size_t)nx * ny * nz, nd = (size_t)np * nt * nr;
     RT_TRY(h2d(c, c->in0, data, nd * sizeof(float)));
     RT_TRY(c->in1.reserve((size_t)(np + nt + nr + nx + ny + nz) * sizeof(double)));
@@ -730,11 +730,7 @@ int rtgrff_compose_cubes(rtgrff_ctx *c, int want_bvec)
     RT_TRY(build_poly_cube(c, nx, ny, nz));
     RT_CUDA(cudaStreamSynchronize(c->stream));
     c->wgeom = g; c->fgeom = g;
-    GridGeomF &f = c->fgeomf;
-    f.nx = nx; f.ny = ny; f.nz = nz;
-    f.x0 = (float)geom[0]; f.y0 = (float)geom[4]; f.z0 = (float)geom[8];
-    f.idx = (float)(1.0 / geom[1]); f.idy = (float)(1.0 / geom[5]); f.idz = (float)(1.0 / geom[9]);
-    f.fxl = (float)(nx - 1); f.fyl = (float)(ny - 1); f.fzl = (float)(nz - 1);
+    c->fgeomf = geomf_from(geom, nx, ny, nz);
     c->has_wcube = true; c->has_fcube = true; c->has_bvec = want_bvec != 0;
     c->stage_has_omega = true;
     return RTGRFF_OK;
@@ -777,17 +773,16 @@ int rtgrff_trace(rtgrff_ctx *c, int64_t n_rays, const double *x_start, const dou
     a.rec_s = trace_cs ? c->rec_s.as<double>() : nullptr;
     a.active_steps = c->counters.as<unsigned long long>();
     const dim3 grid(blocks_for(n_rays, RT_BLOCK)), block(RT_BLOCK);
-    int l64 = trace_variant();
     // the FP32 cell-relative stepper keeps every stage within a few cells of the cached cell
-    if (l64 == MODE_FAST32 &&
-        !(max_stage_offset_cells(dt, trace_cs ? perturb_ratio : 0.0, c->wgeom.idx, c->wgeom.idy, c->wgeom.idz) < kMaxStageOffsetCells))
-        l64 = MODE_F64;
+    const int mode =
+        max_stage_offset_cells(dt, trace_cs ? perturb_ratio : 0.0, c->wgeom.idx, c->wgeom.idy, c->wgeom.idz) < kMaxStageOffsetCells
+            ? MODE_FAST32 : MODE_F64;
     RT_CUDA(cudaEventRecord(c->ev0, c->stream));
 #define RT_TRACE_CASE(v, CS, M) \
     case v: trace_rays_kernel<CS, M><<<grid, block, 0, c->stream>>>(a); break;
-    switch ((trace_cs ? 3 : 0) + l64) {
-        RT_TRACE_CASE(0, false, 0) RT_TRACE_CASE(1, false, 1) RT_TRACE_CASE(2, false, 2)
-        RT_TRACE_CASE(3, true, 0) RT_TRACE_CASE(4, true, 1) RT_TRACE_CASE(5, true, 2)
+    switch ((trace_cs ? 2 : 0) + mode) {
+        RT_TRACE_CASE(0, false, MODE_FAST32) RT_TRACE_CASE(1, false, MODE_F64)
+        RT_TRACE_CASE(2, true, MODE_FAST32) RT_TRACE_CASE(3, true, MODE_F64)
     }
 #undef RT_TRACE_CASE
     RT_TRY(launched(c, "trace_rays_kernel"));
@@ -1161,6 +1156,38 @@ int rtgrff_emission_traced(rtgrff_ctx *c, double pixel_area_cm2, double freq0_hz
     return RTGRFF_OK;
 }
 
+// The T_b, V/I and diagnostic outputs of a map.  The kernel writes the caller's arrays when they are device
+// memory, else the context's out0 / out1 / out3, which map_outputs_read_back then copies to the caller.
+struct MapOutputs {
+    double *tb, *vi, *diag;      // the caller's arrays; diag may be null
+    size_t bytes;                // of tb and of vi; diag holds RTGRFF_N_DIAG times that
+    bool on_device;
+    double *dtb, *dvi, *ddiag;   // where the kernel writes
+};
+
+static int map_outputs_on_device(rtgrff_ctx *c, MapOutputs &o)
+{
+    o.dtb = o.tb; o.dvi = o.vi; o.ddiag = o.diag;
+    if (o.on_device) return RTGRFF_OK;
+    RT_TRY(c->out0.reserve(o.bytes));
+    RT_TRY(c->out1.reserve(o.bytes));
+    o.dtb = c->out0.as<double>(); o.dvi = c->out1.as<double>();
+    if (o.diag) {
+        RT_TRY(c->out3.reserve((size_t)RTGRFF_N_DIAG * o.bytes));
+        o.ddiag = c->out3.as<double>();
+    }
+    return RTGRFF_OK;
+}
+
+static int map_outputs_read_back(rtgrff_ctx *c, const MapOutputs &o)
+{
+    if (o.on_device) return RTGRFF_OK;
+    RT_TRY(d2h(c, o.tb, o.dtb, o.bytes));
+    RT_TRY(d2h(c, o.vi, o.dvi, o.bytes));
+    if (o.diag) RT_TRY(d2h(c, o.diag, o.ddiag, (size_t)RTGRFF_N_DIAG * o.bytes));
+    return RTGRFF_OK;
+}
+
 // rtgrff_render_map and rtgrff_render_map_diag: diag == nullptr launches the plain kernels, else the DIAG ones
 static int render_map_impl(rtgrff_ctx *c, int64_t n_rays, const double *x_start, const double *y_start,
                            const double *z_start, const double *kvec, const int32_t *ray_order, int n_freq,
@@ -1217,16 +1244,8 @@ static int render_map_impl(rtgrff_ctx *c, int64_t n_rays, const double *x_start,
     }
     RT_TRY(c->counters.reserve(64));
     RT_CUDA(cudaMemsetAsync(c->counters.p, 0, 64, c->stream));
-    double *dtb = tb, *dvi = vi, *ddiag = diag;
-    if (!out_on_device) {
-        RT_TRY(c->out0.reserve((size_t)n_freq * nb));
-        RT_TRY(c->out1.reserve((size_t)n_freq * nb));
-        dtb = c->out0.as<double>(); dvi = c->out1.as<double>();
-        if (diag) {
-            RT_TRY(c->out3.reserve((size_t)RTGRFF_N_DIAG * n_freq * nb));
-            ddiag = c->out3.as<double>();
-        }
-    }
+    MapOutputs out{tb, vi, diag, (size_t)n_freq * nb, out_on_device != 0};
+    RT_TRY(map_outputs_on_device(c, out));
     MapArgs a;
     a.cube = rc;
     a.fcube = c->fcube.as<float4>();
@@ -1242,28 +1261,25 @@ static int render_map_impl(rtgrff_ctx *c, int64_t n_rays, const double *x_start,
     a.cs_every_step = cs_every_step();
     a.s_mode = s_mode; a.s_input = s_input_on ? 1 : 0;
     a.grff64 = c->grff64;
-    a.tb = dtb; a.vi = dvi;
+    a.tb = out.dtb; a.vi = out.dvi;
     a.active_steps = c->counters.as<unsigned long long>();
-    a.diag = ddiag;
+    a.diag = out.ddiag;
     a.diag_plane = (int64_t)n_freq * n_rays;     // planes follow the caller's frequency order: FreqDev::out_row
-    const dim3 block(RT_BLOCK);
+    const dim3 grid(blocks_for(n_rays, RT_BLOCK)), block(RT_BLOCK);
     const bool gr = !(em_flag & 1);
     RT_CUDA(cudaEventRecord(c->ev0, c->stream));
     const int variant = (trace_cs ? 8 : 0) | (voxel_order == RTGRFF_ORDER_REVERSED ? 4 : 0) | (use_bvec ? 2 : 0) | (gr ? 1 : 0);
 #define RT_MAP_LAUNCH(CS, ORD, BV, GR, DG)                                                                   \
-        if (mode == MODE_FAST32) {                                                                           \
-            if (carve >= 0) cudaFuncSetAttribute(render_map_kernel<CS, ORD, BV, GR, MODE_FAST32, DG>,        \
-                                                 cudaFuncAttributePreferredSharedMemoryCarveout, carve);      \
+        if (mode == MODE_FAST32)                                                                             \
             render_map_kernel<CS, ORD, BV, GR, MODE_FAST32, DG><<<grid, block, 0, c->stream>>>(a);           \
-        } else render_map_kernel<CS, ORD, BV, GR, MODE_F64, DG><<<grid, block, 0, c->stream>>>(a);
+        else                                                                                                 \
+            render_map_kernel<CS, ORD, BV, GR, MODE_F64, DG><<<grid, block, 0, c->stream>>>(a);
 #define RT_MAP_CASE(v, CS, ORD, BV, GR)                                                                      \
     case v:                                                                                                  \
         if (diag) { RT_MAP_LAUNCH(CS, ORD, BV, GR, true) } else { RT_MAP_LAUNCH(CS, ORD, BV, GR, false) }    \
         break;
-    int mode = trace_variant() == 0 ? MODE_FAST32 : MODE_F64;
-    // RTGRFF_CARVEOUT=<percent>: preferred shared-memory carve-out of the per-ray kernels (A/B switch; they use no
-    // shared memory and the default already gives them the whole unified array as L1: measured equal)
-    static const int carve = getenv("RTGRFF_CARVEOUT") ? atoi(getenv("RTGRFF_CARVEOUT")) : -1;
+    // the FP32 cell-relative stepper keeps every stage within a few cells of the cached cell
+    int mode = MODE_FAST32;
     for (int f = 0; f < n_freq; ++f)
         if (!(max_stage_offset_cells(freqs[f].dt, trace_cs ? perturb_ratio : 0.0, c->wgeom.idx, c->wgeom.idy,
                                      c->wgeom.idz) < kMaxStageOffsetCells))
@@ -1276,42 +1292,38 @@ static int render_map_impl(rtgrff_ctx *c, int64_t n_rays, const double *x_start,
         };
         return cost(x) > cost(y);
     });
-    // the per-frequency constants travel in the kernel parameters: kMaxFreqPerLaunch frequencies per launch
-    const bool fork = kMaxFreqPerLaunch == 1 && n_freq > 1;
-    // launches in flight at once (RTGRFF_FORK_STREAMS, 1..8): the frequencies go round-robin over that many streams
-    static const int n_fork = [] { const char *e = getenv("RTGRFF_FORK_STREAMS"); int v = e ? atoi(e) : 8; return v < 1 ? 1 : (v > 8 ? 8 : v); }();
+    // one launch per frequency (its constants travel in the kernel parameters), round-robin over the fork streams
+    const bool fork = n_freq > 1;
     cudaStream_t main_stream = c->stream;
     if (fork) {
-        for (int q = 0; q < 8; ++q)
+        for (int q = 0; q < kMapForkStreams; ++q)
             if (!c->fstream[q]) RT_CUDA(cudaStreamCreateWithFlags(&c->fstream[q], cudaStreamNonBlocking));
-        for (int q = 0; q < 9; ++q)
+        for (int q = 0; q <= kMapForkStreams; ++q)
             if (!c->fev[q]) RT_CUDA(cudaEventCreateWithFlags(&c->fev[q], cudaEventDisableTiming));
-        RT_CUDA(cudaEventRecord(c->fev[8], main_stream));
-        for (int q = 0; q < 8; ++q) RT_CUDA(cudaStreamWaitEvent(c->fstream[q], c->fev[8], 0));
+        RT_CUDA(cudaEventRecord(c->fev[kMapForkStreams], main_stream));
+        for (int q = 0; q < kMapForkStreams; ++q) RT_CUDA(cudaStreamWaitEvent(c->fstream[q], c->fev[kMapForkStreams], 0));
     }
-    for (int f0 = 0; f0 < n_freq; f0 += kMaxFreqPerLaunch) {
-    a.n_freq = n_freq - f0 < kMaxFreqPerLaunch ? n_freq - f0 : kMaxFreqPerLaunch;
-    for (int f = 0; f < a.n_freq; ++f) a.freqs[f] = fd[f0 + f];
-    const dim3 grid(blocks_for(n_rays, RT_BLOCK), (unsigned int)a.n_freq);
-    struct StreamSwap {           // the launches below go to c->stream
-        rtgrff_ctx *c; cudaStream_t keep;
-        ~StreamSwap() { c->stream = keep; }
-    } swap{c, main_stream};
-    if (fork) c->stream = c->fstream[f0 % n_fork];
-    switch (variant) {
-        RT_MAP_CASE(0, false, 0, false, false) RT_MAP_CASE(1, false, 0, false, true)
-        RT_MAP_CASE(2, false, 0, true, false) RT_MAP_CASE(3, false, 0, true, true)
-        RT_MAP_CASE(4, false, 1, false, false) RT_MAP_CASE(5, false, 1, false, true)
-        RT_MAP_CASE(6, false, 1, true, false) RT_MAP_CASE(7, false, 1, true, true)
-        RT_MAP_CASE(8, true, 0, false, false) RT_MAP_CASE(9, true, 0, false, true)
-        RT_MAP_CASE(10, true, 0, true, false) RT_MAP_CASE(11, true, 0, true, true)
-        RT_MAP_CASE(12, true, 1, false, false) RT_MAP_CASE(13, true, 1, false, true)
-        RT_MAP_CASE(14, true, 1, true, false) RT_MAP_CASE(15, true, 1, true, true)
-    }
-    RT_TRY(launched(c, "render_map_kernel"));
+    for (int f = 0; f < n_freq; ++f) {
+        a.freq = fd[f];
+        struct StreamSwap {           // the launches below go to c->stream
+            rtgrff_ctx *c; cudaStream_t keep;
+            ~StreamSwap() { c->stream = keep; }
+        } swap{c, main_stream};
+        if (fork) c->stream = c->fstream[f % kMapForkStreams];
+        switch (variant) {
+            RT_MAP_CASE(0, false, 0, false, false) RT_MAP_CASE(1, false, 0, false, true)
+            RT_MAP_CASE(2, false, 0, true, false) RT_MAP_CASE(3, false, 0, true, true)
+            RT_MAP_CASE(4, false, 1, false, false) RT_MAP_CASE(5, false, 1, false, true)
+            RT_MAP_CASE(6, false, 1, true, false) RT_MAP_CASE(7, false, 1, true, true)
+            RT_MAP_CASE(8, true, 0, false, false) RT_MAP_CASE(9, true, 0, false, true)
+            RT_MAP_CASE(10, true, 0, true, false) RT_MAP_CASE(11, true, 0, true, true)
+            RT_MAP_CASE(12, true, 1, false, false) RT_MAP_CASE(13, true, 1, false, true)
+            RT_MAP_CASE(14, true, 1, true, false) RT_MAP_CASE(15, true, 1, true, true)
+        }
+        RT_TRY(launched(c, "render_map_kernel"));
     }
     if (fork) {
-        for (int q = 0; q < 8; ++q) {
+        for (int q = 0; q < kMapForkStreams; ++q) {
             RT_CUDA(cudaEventRecord(c->fev[q], c->fstream[q]));
             RT_CUDA(cudaStreamWaitEvent(main_stream, c->fev[q], 0));
         }
@@ -1320,11 +1332,7 @@ static int render_map_impl(rtgrff_ctx *c, int64_t n_rays, const double *x_start,
 #undef RT_MAP_LAUNCH
     RT_CUDA(cudaEventRecord(c->ev1, c->stream));
     c->ev_valid = true;
-    if (!out_on_device) {
-        RT_TRY(d2h(c, tb, dtb, (size_t)n_freq * nb));
-        RT_TRY(d2h(c, vi, dvi, (size_t)n_freq * nb));
-        if (diag) RT_TRY(d2h(c, diag, ddiag, (size_t)RTGRFF_N_DIAG * n_freq * nb));
-    }
+    RT_TRY(map_outputs_read_back(c, out));
     unsigned long long act[3] = {0, 0, 0};
     RT_TRY(d2h(c, act, c->counters.p, sizeof(act)));
     RT_CUDA(cudaStreamSynchronize(c->stream));
@@ -1366,9 +1374,7 @@ int rtgrff_set_spherical_model(rtgrff_ctx *c, int slot, const float *data, const
     if (!data || !phi || !lat || !r) return fail(RTGRFF_EINVAL, "null argument");
     if (np < 2 || nt < 2 || nr < 2) return fail(RTGRFF_EINVAL, "spherical mesh needs >= 2 nodes per axis");
     if ((int64_t)np * nt * nr >= (int64_t)1 << 31) return fail(RTGRFF_EINVAL, "spherical mesh larger than 2^31 nodes");
-    for (int i = 1; i < np; ++i) if (!(phi[i] > phi[i - 1])) return fail(RTGRFF_EINVAL, "phi nodes must ascend");
-    for (int i = 1; i < nt; ++i) if (!(lat[i] > lat[i - 1])) return fail(RTGRFF_EINVAL, "latitude nodes must ascend");
-    for (int i = 1; i < nr; ++i) if (!(r[i] > r[i - 1])) return fail(RTGRFF_EINVAL, "radius nodes must ascend");
+    RT_TRY(check_ascending_nodes(phi, np, lat, nt, r, nr));
     c->sph_set[slot] = false;
     RT_TRY(h2d(c, c->sph_data[slot], data, (size_t)np * nt * nr * sizeof(float)));
     std::vector<double> &n = c->sph_nodes[slot];
@@ -1445,17 +1451,9 @@ int rtgrff_render_los_map(rtgrff_ctx *c, int nx, int ny, const double *x, const 
     a.area = pixel_area_cm2;
     a.em_flag = em_flag; a.s_max = s_max; a.grff64 = c->grff64;
     const size_t npix = (size_t)nx * ny, nb = npix * sizeof(double);
-    double *dtb = tb, *dvi = vi, *ddiag = diag;
-    if (!out_on_device) {
-        RT_TRY(c->out0.reserve((size_t)n_freq * nb));
-        RT_TRY(c->out1.reserve((size_t)n_freq * nb));
-        dtb = c->out0.as<double>(); dvi = c->out1.as<double>();
-        if (diag) {
-            RT_TRY(c->out3.reserve((size_t)RTGRFF_N_DIAG * n_freq * nb));
-            ddiag = c->out3.as<double>();
-        }
-    }
-    a.tb = dtb; a.vi = dvi; a.diag = ddiag;
+    MapOutputs out{tb, vi, diag, (size_t)n_freq * nb, out_on_device != 0};
+    RT_TRY(map_outputs_on_device(c, out));
+    a.tb = out.dtb; a.vi = out.dvi; a.diag = out.ddiag;
     RT_TRY(c->counters.reserve(64));
     RT_CUDA(cudaMemsetAsync(c->counters.p, 0, 64, c->stream));
     a.valid_samples = c->counters.as<unsigned long long>();
@@ -1480,11 +1478,7 @@ int rtgrff_render_los_map(rtgrff_ctx *c, int nx, int ny, const double *x, const 
     RT_TRY(launched(c, "los_map_kernel"));
     RT_CUDA(cudaEventRecord(c->ev1, c->stream));
     c->ev_valid = true;
-    if (!out_on_device) {
-        RT_TRY(d2h(c, tb, dtb, (size_t)n_freq * nb));
-        RT_TRY(d2h(c, vi, dvi, (size_t)n_freq * nb));
-        if (diag) RT_TRY(d2h(c, diag, ddiag, (size_t)RTGRFF_N_DIAG * n_freq * nb));
-    }
+    RT_TRY(map_outputs_read_back(c, out));
     unsigned long long n_valid = 0;
     RT_TRY(d2h(c, &n_valid, c->counters.p, sizeof(n_valid)));
     RT_CUDA(cudaStreamSynchronize(c->stream));

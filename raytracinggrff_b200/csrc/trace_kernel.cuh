@@ -6,9 +6,10 @@
 
 namespace rtgrff {
 
-// Stepper selection: 0 = FP64 master state + FP32 cell-relative RHS + register cell cache (default),
-// 1 = FP64 state and RHS with FP32 trilinear arithmetic, 2 = FP64 everything.
-enum { MODE_FAST32 = 0, MODE_F64 = 1, MODE_F64_LERP64 = 2 };
+// Stepper: MODE_FAST32 = FP64 master state + FP32 cell-relative RHS + register cell cache; MODE_F64 = FP64
+// state and RHS with FP32 trilinear arithmetic, which the host picks when a step plus the pencil offset
+// reaches kMaxStageOffsetCells.
+enum { MODE_FAST32 = 0, MODE_F64 = 1 };
 
 // Advance one ray by one step with the selected stepper.  Returns whether the ray is still alive.
 // A step that leaves the state untouched (outside the cube, NaN, omega = 0) repeats forever: the
@@ -27,10 +28,9 @@ __device__ __forceinline__ bool advance_ray(const RayCube &C, const StepConst &K
     if (MODE == MODE_FAST32) {
         moved = step32<CS>(C, K, cache, s, want_s, s_step);
     } else {
-        constexpr bool L64 = (MODE == MODE_F64_LERP64);
         const State s0 = s;
-        s = rk4_step<L64>(C, s0, dt);
-        if (CS && want_s) s_step = (float)cross_section_ratio<L64>(C, s0, s, dt, perturb_ratio);
+        s = rk4_step(C, s0, dt);
+        if (CS && want_s) s_step = (float)cross_section_ratio(C, s0, s, dt, perturb_ratio);
         moved = in_cube(C, s0.rx, s0.ry, s0.rz) && state_differs(s, s0);
     }
     if (CS && !moved) s_step = nanf("");

@@ -27,7 +27,6 @@ def timeit(fn, n=3):
 
 def main():
     which = sys.argv[1] if len(sys.argv) > 1 else "all"
-    print("RTGRFF_MODE =", os.environ.get("RTGRFF_MODE", "0"))
     ses = RaySession(0)
     if which in ("all", "c3"):
         c = synthetic.corona_cube(128, 3.0)

@@ -494,7 +494,8 @@ def test_workflow_command_line(tmp_path, oracle):
 def test_trace_steps_longer_than_a_cell(oracle, session):
     """Low-frequency presets on a fine cube make a step (plus the pencil offset) span more than one
     cell (BASELINE config 5 at 20-24 MHz: 1.1 cells).  The FP32 stepper handles whole-cell shifts of
-    any size; the face margin grows with the step (StepConst.margin)."""
+    any size; the face margin grows with the step (StepConst.margin).  From 8 cells on the host runs
+    the FP64 stepper instead (kMaxStageOffsetCells)."""
     n = 160
     g = np.linspace(-1.2, 1.2, n)
     X, Y, Z = np.meshgrid(g, g, g, indexing="ij")
@@ -508,7 +509,7 @@ def test_trace_steps_longer_than_a_cell(oracle, session):
     zs[:4] = [1.2000001, 1.19, 1.0, 0.5]
     kv = np.column_stack([rng.normal(scale=0.15, size=m), rng.normal(scale=0.15, size=m), -np.ones(m)])
     kv /= np.linalg.norm(kv, axis=1, keepdims=True)
-    for dt, steps in ((0.0134, 500), (0.03, 260)):       # 1.15 and 2.6 cells per (step + pencil)
+    for dt, steps in ((0.0134, 500), (0.03, 260), (0.1, 80)):    # 1.15, 2.6 and 8.6 cells per (step + pencil)
         cells = 3 * dt * (2.998e10 / 6.96e10) * (n - 1) / 2.4
         assert cells > 1.1
         rr, ss, act = session.trace(80e6, xs, ys, zs, kv, dt, steps, 7, True, 2.0)
@@ -596,8 +597,8 @@ def test_trace_backwards_in_time(oracle, session):
 
 
 def test_render_map_many_frequencies_order_and_chunks(session):
-    """More frequencies than fit one launch (16 per launch, dispatched longest first): every row of the
-    result must equal the single-frequency render of that frequency, bit for bit."""
+    """More frequencies than fork streams (one launch per frequency, dispatched longest first over 8 streams):
+    every row of the result must equal the single-frequency render of that frequency, bit for bit."""
     c = synthetic.corona_cube(48, 3.0, active_region=True)
     session.set_omega_cube(c["omega_pe"], c["x_grid"], c["y_grid"], c["z_grid"])
     session.set_field_cubes(c["x_grid"], c["y_grid"], c["z_grid"], c["ne"], c["te"], c["b"], c["bx"], c["by"], c["bz"])
