@@ -282,7 +282,10 @@ __global__ void __launch_bounds__(RT_BLOCK, RT_MINB) render_map_kernel(const Map
     bool alive = has_ray;
     float s_step = CS ? 0.0f : 1.0f;
     double s_cum = 1.0;
+    // launch-uniform modes, read once
     const bool cumulative = CS && a.s_mode == RTGRFF_S_CUMULATIVE;
+    const bool pencil_every_step = CS && (cumulative || a.cs_every_step);
+    const bool s_input = a.s_input != 0, force64 = a.grff64 != 0;
     unsigned int n_samples = 0;
     const int n_steps = (int)fp.n_steps, stride = (int)fp.stride;     // < 2^31, checked on the host
     int next_rec = 0;
@@ -295,10 +298,14 @@ __global__ void __launch_bounds__(RT_BLOCK, RT_MINB) render_map_kernel(const Map
     bool first = true;
     bool tail_done = !has_ray;            // a frozen ray repeats the same record: ds = 0 -> empty voxel
 
-    for (int i = 0; i < n_steps; ++i) {
+    // The steps go in intervals: one step with the pencil traced (CS), then up to the next such step the central
+    // ray only, in a tight loop with no record bookkeeping (most steps: the record strides are 1-6).  In the per-step
+    // S schedule the interval is the record stride and its first step is the recorded one.  Cumulative S and
+    // RTGRFF_CS_EVERY_STEP=1 need the pencil at every step: intervals of one step, a record at every stride-th.
+    const int interval = pencil_every_step ? 1 : stride;
+    for (int i = 0; i < n_steps;) {
         if (alive) {
-            const bool want_s = CS && (i == next_rec || a.cs_every_step || cumulative);
-            alive = advance_ray<CS, MODE>(C, K, cache, s, fp.dt, a.perturb_ratio, want_s, s_step);
+            alive = advance_ray<CS, MODE>(C, K, cache, s, fp.dt, a.perturb_ratio, CS, s_step);
             if (cumulative) s_cum *= s_step;     // gpu_raytrace.py:398-408
             if (!alive) death = i;
         }
@@ -335,8 +342,8 @@ __global__ void __launch_bounds__(RT_BLOCK, RT_MINB) render_map_kernel(const Map
                     // --- Parms packing rules (script/resample_with_ray_tracing.py:472-501) ---
                     if (isfinite(f.ne) && isfinite(f.te) && isfinite(f.b)) {
                         // Parms[14] = S * area (script/resample_with_ray_tracing.py:501): source factor S
-                        const VoxLite lite = {ds, f.te, f.ne, f.b, cthf, a.s_input ? sv : 1.0f};
-                        tr.push(fq, lite, sthf, a.em_flag, a.s_max, a.grff64 != 0, x, y, z);
+                        const VoxLite lite = {ds, f.te, f.ne, f.b, cthf, s_input ? sv : 1.0f};
+                        tr.push(fq, lite, sthf, a.em_flag, a.s_max, force64, x, y, z);
                     }
                     px = x; py = y; pz = z;
                     first = false;
@@ -348,6 +355,20 @@ __global__ void __launch_bounds__(RT_BLOCK, RT_MINB) render_map_kernel(const Map
         // a frozen ray still owes its first post-freeze record (with the cross-sections off its S is 1 and the
         // record counts, exactly as in trace -> sample -> emission): leave only when every lane has handed it over
         if (!__any_sync(0xffffffffu, alive || !tail_done)) break;
+        // The rest of the interval.  Its loop carries only the interval's own moving / frozen_at: with the ray's
+        // alive / death / s_step in it (live across the whole kernel, so in spill slots), every step reloaded and
+        // stored them.  A ray frozen here hands its record over at the start of the next interval (it no longer moves).
+        const int end = n_steps - i > interval ? i + interval : n_steps;
+        bool moving = alive;
+        int frozen_at = end;
+        for (int j = i + 1; j < end; ++j)
+            if (moving && !advance_central<MODE>(C, K, cache, s, fp.dt)) { moving = false; frozen_at = j; }
+        if (frozen_at < end) {
+            alive = false;
+            death = frozen_at;
+            if (CS) s_step = nanf("");      // as advance_ray
+        }
+        i = end;
     }
     if (has_ray) {
         double tb, vi, IL, IR;
@@ -361,7 +382,7 @@ __global__ void __launch_bounds__(RT_BLOCK, RT_MINB) render_map_kernel(const Map
         // a ray moves on steps [0, death): the counters follow from where it froze
         unsigned long long moved_steps = has_ray ? (unsigned long long)(death >= 0 ? death : n_steps) : 0ull;
         const unsigned long long pencil_steps =
-            !CS ? 0ull : ((a.cs_every_step || cumulative) ? moved_steps : (moved_steps + stride - 1) / stride);
+            !CS ? 0ull : (pencil_every_step ? moved_steps : (moved_steps + stride - 1) / stride);
         unsigned long long ps = pencil_steps, ns = n_samples;
         for (int off = 16; off > 0; off >>= 1) {
             moved_steps += __shfl_down_sync(0xffffffffu, moved_steps, off);

@@ -29,6 +29,8 @@
 //    of a step (central + two pencil rays) are a rolled loop, the face handling is a run-time
 //    flag: the stepper is ~1500 SASS instructions where the first version (16 inlined copies of
 //    the RHS, 134 KB of SASS) lost 30 % of its issue slots to instruction-cache misses.
+//    render_map_kernel inlines one more copy of the central ray's stages (step32_central, ~660
+//    instructions) for the steps between two records.
 #pragma once
 
 #include "ray_integrator.cuh"
@@ -264,15 +266,10 @@ __device__ __forceinline__ void init_cell(const RayCube &C, const State &s, Cell
     load_cell(C, (cache.ci * C.ny + cache.cj) * C.nz + cache.ck, cache);
 }
 
-// One full step of the master state `s`: classic RK4 (build_rays.py:177-182) of the central ray
-// and, when `want_s` (warp-uniform), the same RK4 on the two pencil rays displaced by eps along
-// (e1, e2) _|_ t_hat with the cross-section ratio of this step (build_rays.py:209-239, with
-// d = r_pert' - r_central' = eps*e + c6*(sum_v_pert - sum_v_central)).  Returns false when the ray
-// is frozen: outside the cube / NaN, or every stage derivative exactly zero (the reference's
-// update is then exactly zero too, for ever).
-template <bool CS>
-__device__ __forceinline__ bool step32(const RayCube &C, const StepConst &K, Cell &cache, State &s, bool want_s,
-                                       float &s_step)
+// Start of a step, shared by step32 and step32_central: the `edge` flag, the master position relative to
+// the cached cell (FP64 -> FP32 once per step) and k in FP32.  Returns false when the ray is frozen.
+__device__ __forceinline__ bool step32_begin(const RayCube &C, const StepConst &K, const Cell &cache, const State &s,
+                                             bool &edge, float2 &pxy, float &pz, float2 &kxy, float &kz)
 {
     const double fx = (s.rx - C.x0) * C.idx, fy = (s.ry - C.y0) * C.idy, fz = (s.rz - C.z0) * C.idz;
     if (cache.off < 0) return false;      // the ray started outside the cube (init_cell): frozen for ever
@@ -283,16 +280,70 @@ __device__ __forceinline__ bool step32(const RayCube &C, const StepConst &K, Cel
     // that reaches a face can the master or a stage be outside the cube: exact scipy tests then (a
     // frozen ray stays in this state), none in the interior.
     const int mg = K.margin;
-    const bool edge = (cache.ci < mg) | (cache.ci > C.nx - 2 - mg) | (cache.cj < mg) | (cache.cj > C.ny - 2 - mg) |
-                      (cache.ck < mg) | (cache.ck > C.nz - 2 - mg);
+    edge = (cache.ci < mg) | (cache.ci > C.nx - 2 - mg) | (cache.cj < mg) | (cache.cj > C.ny - 2 - mg) |
+           (cache.ck < mg) | (cache.ck > C.nz - 2 - mg);
     if (edge && !in_cube(C, s.rx, s.ry, s.rz)) return false;
-    // master position relative to the cached cell (FP64 -> FP32 once per step)
-    float px = (float)(fx - (double)cache.ci), py = (float)(fy - (double)cache.cj), pz = (float)(fz - (double)cache.ck);
-    const float kx = (float)s.kx, ky = (float)s.ky, kz = (float)s.kz;
+    pxy = make_float2((float)(fx - (double)cache.ci), (float)(fy - (double)cache.cj));
+    pz = (float)(fz - (double)cache.ck);
+    kxy = make_float2((float)s.kx, (float)s.ky);
+    kz = (float)s.kz;
+    return true;
+}
+
+// The four RK4 stages of one ray that starts (qxy, qz) cells from the step's base position: the sums
+// k1 + 2 k2 + 2 k3 + k4 of v and of g.
+__device__ __forceinline__ void rk4_stages32(const RayCube &C, const StepConst &K, Cell &cache, bool edge, float2 &pxy,
+                                             float &pz, float2 qxy, float qz, float2 kxy, float kz, float2 &avxy,
+                                             float &avz, float2 &agxy, float &agz)
+{
+    const float2 h1xy = make_float2(K.hx, K.hy), h2xy = make_float2(2.0f * K.hx, 2.0f * K.hy);
+    float2 dxy = qxy, skxy = kxy;
+    float dz = qz, skz = kz;
+#pragma unroll          // the four stages unrolled (constant weights); the rays of a step are a rolled loop (step32)
+    for (int st = 0; st < 4; ++st) {
+        const Deriv32P d = rhs32p(C, cache, edge, pxy, pz, dxy, dz, skxy, skz);
+        if (st == 0) {        // (0 + x is not x for x = -0: spelled out, the compiler would keep the FADDs)
+            avxy = d.vxy; avz = d.vz; agxy = d.gxy; agz = d.gz;
+        } else {
+            const float w = (st == 3) ? 1.0f : 2.0f;
+            avxy = __ffma2_rn(bc2(w), d.vxy, avxy); avz = fmaf(w, d.vz, avz);
+            agxy = __ffma2_rn(bc2(w), d.gxy, agxy); agz = fmaf(w, d.gz, agz);
+        }
+        // stages 2, 3 at dt/2, stage 4 at dt (K.h* are half steps)
+        dxy = __ffma2_rn((st < 2) ? h1xy : h2xy, d.vxy, qxy);
+        dz = fmaf((st < 2) ? K.hz : 2.0f * K.hz, d.vz, qz);
+        const float ak = (st < 2) ? -K.hk : -2.0f * K.hk;
+        skxy = __ffma2_rn(bc2(ak), d.gxy, kxy); skz = fmaf(ak, d.gz, kz);
+    }
+}
+
+// The central ray's sums -> the FP64 master state.  Returns whether the ray moved (some stage derivative
+// is not exactly zero).
+__device__ __forceinline__ bool step32_commit(const StepConst &K, State &s, float2 avxy, float avz, float2 agxy, float agz)
+{
+    const float avx = avxy.x, avy = avxy.y, agx = agxy.x, agy = agxy.y;
+    const bool moved = (fabsf(avx) + fabsf(avy) + fabsf(avz) + fabsf(agx) + fabsf(agy) + fabsf(agz)) != 0.0f;
+    s.kx = fma((double)agx, -K.c6, s.kx); s.ky = fma((double)agy, -K.c6, s.ky); s.kz = fma((double)agz, -K.c6, s.kz);
+    s.rx = fma((double)avx, K.c6, s.rx); s.ry = fma((double)avy, K.c6, s.ry); s.rz = fma((double)avz, K.c6, s.rz);
+    return moved;
+}
+
+// One full step of the master state `s`: classic RK4 (build_rays.py:177-182) of the central ray
+// and, when `want_s` (warp-uniform), the same RK4 on the two pencil rays displaced by eps along
+// (e1, e2) _|_ t_hat with the cross-section ratio of this step (build_rays.py:209-239, with
+// d = r_pert' - r_central' = eps*e + c6*(sum_v_pert - sum_v_central)).  Returns false when the ray
+// is frozen: outside the cube / NaN, or every stage derivative exactly zero (the reference's
+// update is then exactly zero too, for ever).
+template <bool CS>
+__device__ __forceinline__ bool step32(const RayCube &C, const StepConst &K, Cell &cache, State &s, bool want_s,
+                                       float &s_step)
+{
+    bool edge;
+    float2 pxy, kxy;
+    float pz, kz;
+    if (!step32_begin(C, K, cache, s, edge, pxy, pz, kxy, kz)) return false;
     const int n_rays = (CS && want_s) ? 3 : 1;
-    float2 pxy = make_float2(px, py);
-    const float2 kxy = make_float2(kx, ky);
-    const float2 ixy = make_float2(K.ix, K.iy), h1xy = make_float2(K.hx, K.hy), h2xy = make_float2(2.0f * K.hx, 2.0f * K.hy);
+    const float2 ixy = make_float2(K.ix, K.iy);
     float2 oxy = make_float2(0.0f, 0.0f);           // displacement of the current ray from the central one, R_sun
     float oz = 0.0f;
     float2 cvxy = make_float2(0.0f, 0.0f);          // central ray: sum of v over the stages
@@ -304,29 +355,12 @@ __device__ __forceinline__ bool step32(const RayCube &C, const StepConst &K, Cel
     for (int q = 0; q < n_rays; ++q) {
         const float2 qxy = __fmul2_rn(oxy, ixy);                      // start of this ray relative to p, cells
         const float qz = oz * K.iz;
-        float2 dxy = qxy, skxy = kxy, avxy, agxy;                     // k1 + 2 k2 + 2 k3 + k4
-        float dz = qz, skz = kz, avz, agz;
-#pragma unroll          // the four stages unrolled (constant weights), the three rays of a step rolled
-        for (int st = 0; st < 4; ++st) {
-            const Deriv32P d = rhs32p(C, cache, edge, pxy, pz, dxy, dz, skxy, skz);
-            if (st == 0) {        // (0 + x is not x for x = -0: spelled out, the compiler would keep the FADDs)
-                avxy = d.vxy; avz = d.vz; agxy = d.gxy; agz = d.gz;
-            } else {
-                const float w = (st == 3) ? 1.0f : 2.0f;
-                avxy = __ffma2_rn(bc2(w), d.vxy, avxy); avz = fmaf(w, d.vz, avz);
-                agxy = __ffma2_rn(bc2(w), d.gxy, agxy); agz = fmaf(w, d.gz, agz);
-            }
-            // stages 2, 3 at dt/2, stage 4 at dt (K.h* are half steps)
-            dxy = __ffma2_rn((st < 2) ? h1xy : h2xy, d.vxy, qxy);
-            dz = fmaf((st < 2) ? K.hz : 2.0f * K.hz, d.vz, qz);
-            const float ak = (st < 2) ? -K.hk : -2.0f * K.hk;
-            skxy = __ffma2_rn(bc2(ak), d.gxy, kxy); skz = fmaf(ak, d.gz, kz);
-        }
-        const float avx = avxy.x, avy = avxy.y, agx = agxy.x, agy = agxy.y;
+        float2 avxy, agxy;
+        float avz, agz;
+        rk4_stages32(C, K, cache, edge, pxy, pz, qxy, qz, kxy, kz, avxy, avz, agxy, agz);
+        const float avx = avxy.x, avy = avxy.y;
         if (q == 0) {
-            moved = (fabsf(avx) + fabsf(avy) + fabsf(avz) + fabsf(agx) + fabsf(agy) + fabsf(agz)) != 0.0f;
-            s.kx = fma((double)agx, -K.c6, s.kx); s.ky = fma((double)agy, -K.c6, s.ky); s.kz = fma((double)agz, -K.c6, s.kz);
-            s.rx = fma((double)avx, K.c6, s.rx); s.ry = fma((double)avy, K.c6, s.ry); s.rz = fma((double)avz, K.c6, s.rz);
+            moved = step32_commit(K, s, avxy, avz, agxy, agz);
             cvxy = avxy; cvz = avz;
             if (n_rays > 1) {
                 // norms through MUFU.RSQ (2 ulp): S is held to 1e-4, and the reference's +1e-32 / +1e-30
@@ -360,6 +394,21 @@ __device__ __forceinline__ bool step32(const RayCube &C, const StepConst &K, Cel
         }
     }
     return moved;
+}
+
+// step32 without the pencil: the central ray's step, for the steps whose cross-section ratio is never observed.
+// The same operations as step32's central ray, so the master state is bit-identical (that ray starts at offset
+// 0 * 1/dx = +0 cells there, the literal zero here).
+__device__ __forceinline__ bool step32_central(const RayCube &C, const StepConst &K, Cell &cache, State &s)
+{
+    bool edge;
+    float2 pxy, kxy;
+    float pz, kz;
+    if (!step32_begin(C, K, cache, s, edge, pxy, pz, kxy, kz)) return false;
+    float2 avxy, agxy;
+    float avz, agz;
+    rk4_stages32(C, K, cache, edge, pxy, pz, make_float2(0.0f, 0.0f), 0.0f, kxy, kz, avxy, avz, agxy, agz);
+    return step32_commit(K, s, avxy, avz, agxy, agz);
 }
 
 }  // namespace rtgrff

@@ -37,6 +37,18 @@ __device__ __forceinline__ bool advance_ray(const RayCube &C, const StepConst &K
     return moved;
 }
 
+// advance_ray with want_s = false, without the pencil's state: the steps whose cross-section ratio no
+// record carries (render_map_kernel's steps between two records).  Returns whether the ray moved; the
+// caller sets the frozen ray's S to NaN as advance_ray does.
+template <int MODE>
+__device__ __forceinline__ bool advance_central(const RayCube &C, const StepConst &K, Cell &cache, State &s, double dt)
+{
+    if (MODE == MODE_FAST32) return step32_central(C, K, cache, s);
+    const State s0 = s;
+    s = rk4_step(C, s0, dt);
+    return in_cube(C, s0.rx, s0.ry, s0.rz) && state_differs(s, s0);
+}
+
 struct TraceArgs {
     RayCube cube;
     int64_t n_rays;
