@@ -107,6 +107,31 @@ int rtgrff_resample_spherical(rtgrff_ctx *ctx, int slot, const float *data, cons
                               double scale, double fill, int fill_nonfinite, double *out);
 
 /*
+ * Observer view.  The rtgrff_*_view entry points take the solar B0 and P angles [deg] of the observer, right after
+ * phi0_offset_deg; the entry points without _view are the same calls with B0 = P = 0 (the model's equatorial plane
+ * seen edge-on, solar north along image +y), and both give bit-identical results there.
+ *
+ * The observer frame is the cube frame: +z towards the observer, +y image up, +x image right (solar west when
+ * P = 0; longitude grows towards +x, as Carrington longitude grows towards the west).  A cube or LOS point
+ * p = (x, y, z) goes to model-aligned coordinates in two steps, then through the fixed mapping:
+ *   1. undo P, a rotation about the line of sight:  x1 = x cos P + y sin P,  y1 = -x sin P + y cos P,  z1 = z
+ *   2. undo B0, a rotation about x:                 x2 = x1,  y2 = y1 cos B0 + z1 sin B0,  z2 = -y1 sin B0 + z1 cos B0
+ *   3. cart_to_sph(x2, -z2, y2, phi0).
+ * Solar north in the observer frame is n = (-sin P cos B0, cos P cos B0, sin B0): B0 > 0 tilts the north pole towards
+ * the observer, P > 0 turns north from +y towards -x (east), the ephemeris convention.  phi0_offset_deg keeps its
+ * meaning: the central meridian does not depend on B0 or P.  The B vector is evaluated at (x2, y2, z2) and turned
+ * back to the observer frame with the transpose of the same rotation.  The straight-LOS geometry (start on the disk
+ * or on the plane of the sky behind the limb) is spherical and does not change.  B0 and P must be finite and
+ * |B0| <= 90 deg, else RTGRFF_EINVAL.  Multiples of 90 deg are exact (P = 90 is an exact quarter turn).
+ */
+int rtgrff_resample_spherical_view(rtgrff_ctx *ctx, int slot, const float *data, const double *phi,
+                                   const double *lat, const double *r, int np, int nt, int nr,
+                                   const double *x_grid, const double *y_grid, const double *z_grid, int nx,
+                                   int ny, int nz, const double geom[12], double phi0_offset_deg, double b0_deg,
+                                   double p_deg, double r_min, double scale, double fill, int fill_nonfinite,
+                                   double *out);
+
+/*
  * Sample one spherical variable along straight lines of sight (the resampler of the straight-LOS
  * workflow, script/resampling_MAS_LOS.py:141-231): pixel (i,j) at (x[j], y[i]) [R_sun]; each LOS
  * starts on the solar surface / the plane of the sky behind the limb, minus z_eps, and runs towards
@@ -117,13 +142,19 @@ int rtgrff_sample_spherical_los(rtgrff_ctx *ctx, const float *data, const double
                                 const double *r, int np, int nt, int nr, const double *x, const double *y,
                                 const double *zc, int nx, int ny, int nz, double phi0_offset_deg,
                                 double r_min, double scale, double z_eps, double *out);
+int rtgrff_sample_spherical_los_view(rtgrff_ctx *ctx, const float *data, const double *phi, const double *lat,
+                                     const double *r, int np, int nt, int nr, const double *x, const double *y,
+                                     const double *zc, int nx, int ny, int nz, double phi0_offset_deg,
+                                     double b0_deg, double p_deg, double r_min, double scale, double z_eps,
+                                     double *out);
 
 /*
  * Build the device cubes of the ray path from the five resampled slots with the reference's rules
  * (script/resample_with_ray_tracing.py:269-293): omega_pe = 2 pi 8.93e3 sqrt(max(rho,0)) (NaN -> 0)
  * and its numpy.gradient, n_e = max(rho,0), T NaN -> 1e4, |B| = sqrt(br^2+bt^2+bp^2); with
  * want_bvec also the Cartesian B vector (for theta from B.t).  Equivalent to rtgrff_set_omega_cube
- * + rtgrff_set_field_cubes without the cubes ever visiting the host.
+ * + rtgrff_set_field_cubes without the cubes ever visiting the host.  The B vector is turned to the observer frame
+ * with the view the slots were resampled with; RTGRFF_EINVAL if the five slots were resampled with different views.
  */
 int rtgrff_compose_cubes(rtgrff_ctx *ctx, int want_bvec);
 
@@ -331,6 +362,13 @@ int rtgrff_render_los_map(rtgrff_ctx *ctx, int nx, int ny, const double *x, cons
                           const double *dz_cm, double phi0_offset_deg, double r_min, double z_eps, int n_freq,
                           const double *freq_hz, double pixel_area_cm2, int em_flag, int s_max, int use_bvec, double *tb,
                           double *vi, double *diag, int out_on_device, int64_t *stats);
+/* rtgrff_render_los_map from the observer view (b0_deg, p_deg) (see "Observer view" above): the sample positions and,
+ * with use_bvec, the B vector whose z component gives cos theta.  The diagnostic planes stay in the observer frame. */
+int rtgrff_render_los_map_view(rtgrff_ctx *ctx, int nx, int ny, const double *x, const double *y, int nz,
+                               const double *zc, const double *dz_cm, double phi0_offset_deg, double b0_deg,
+                               double p_deg, double r_min, double z_eps, int n_freq, const double *freq_hz,
+                               double pixel_area_cm2, int em_flag, int s_max, int use_bvec, double *tb, double *vi,
+                               double *diag, int out_on_device, int64_t *stats);
 
 /*
  * Multi-GPU (one process per GPU, the cube replicated on each).  Rays are independent, so the only exchange

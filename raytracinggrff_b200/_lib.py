@@ -40,7 +40,8 @@ EXPORTS = (
     "rtgrff_export_cubes", "rtgrff_shard_rows", "rtgrff_comm_unique_id", "rtgrff_comm_init_rank",
     "rtgrff_comm_destroy", "rtgrff_gather_image", "rtgrff_device_alloc", "rtgrff_device_free",
     "rtgrff_ctx_set_pipeline", "rtgrff_ctx_set_grff64", "rtgrff_place_rows", "rtgrff_render_map_diag",
-    "rtgrff_set_spherical_model", "rtgrff_render_los_map",
+    "rtgrff_set_spherical_model", "rtgrff_render_los_map", "rtgrff_resample_spherical_view",
+    "rtgrff_sample_spherical_los_view", "rtgrff_render_los_map_view",
 )
 
 # planes of rtgrff_render_map_diag's output (RTGRFF_DIAG_* in include/rtgrff.h), in plane order
@@ -95,9 +96,14 @@ def load():
     lib.rtgrff_set_field_cubes.argtypes = [c_void_p, fp, fp, fp, fp, fp, fp, c_int, c_int, c_int, dp]
     lib.rtgrff_resample_spherical.argtypes = [c_void_p, c_int, fp, dp, dp, dp, c_int, c_int, c_int, dp, dp, dp, c_int,
                                               c_int, c_int, dp, c_double, c_double, c_double, c_double, c_int, dp]
+    # the _view entry points: the same arguments plus b0_deg, p_deg right after phi0_offset_deg
+    a = lib.rtgrff_resample_spherical.argtypes
+    lib.rtgrff_resample_spherical_view.argtypes = a[:17] + [c_double, c_double] + a[17:]
     lib.rtgrff_compose_cubes.argtypes = [c_void_p, c_int]
     lib.rtgrff_sample_spherical_los.argtypes = [c_void_p, fp, dp, dp, dp, c_int, c_int, c_int, dp, dp, dp, c_int, c_int,
                                                 c_int, c_double, c_double, c_double, c_double, dp]
+    a = lib.rtgrff_sample_spherical_los.argtypes
+    lib.rtgrff_sample_spherical_los_view.argtypes = a[:15] + [c_double, c_double] + a[15:]
     lib.rtgrff_trace.argtypes = [c_void_p, c_int64, dp, dp, dp, dp, c_double, c_double, c_int64, c_int64, c_int,
                                  c_double, c_int, dp, dp, POINTER(c_int64)]
     lib.rtgrff_sample.argtypes = [c_void_p, c_int64, c_int64, fp, fp, fp, c_double, c_double, c_double, c_double,
@@ -116,6 +122,8 @@ def load():
     lib.rtgrff_render_los_map.argtypes = [c_void_p, c_int, c_int, dp, dp, c_int, dp, dp, c_double, c_double, c_double,
                                           c_int, dp, c_double, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p, c_int,
                                           POINTER(c_int64)]
+    a = lib.rtgrff_render_los_map.argtypes
+    lib.rtgrff_render_los_map_view.argtypes = a[:9] + [c_double, c_double] + a[9:]
     lib.rtgrff_gaussian_beam.argtypes = [c_void_p, dp, c_int, c_int, c_int, c_double, c_double, dp]
     lib.rtgrff_patch_nan.argtypes = [c_void_p, dp, c_int, c_int, c_int, c_int, POINTER(c_int64)]
     for name in EXPORTS:

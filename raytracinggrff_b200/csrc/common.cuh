@@ -128,6 +128,7 @@ struct rtgrff_ctx {
     int slot_nx = 0, slot_ny = 0, slot_nz = 0;
     double slot_geom[12] = {0};
     double slot_geoms[5][12] = {{0}};   // geometry each slot was resampled on (compose checks they agree)
+    double slot_views[5][2] = {{0}};    // the view (b0, p) [deg] each slot was resampled with (compose turns B with it)
     bool stage_has_omega = false;    // `stage` still holds the float64 omega_pe of the last compose (rtgrff_export_cubes)
 
     // spherical model resident for the straight-LOS map (rtgrff_set_spherical_model): slot 0..4 = rho, te, br, bt, bp,

@@ -77,6 +77,34 @@ __device__ __forceinline__ double sample_spherical(const SphMesh &m, double lon,
     return v;
 }
 
+// The observer's view of the model (include/rtgrff.h, "Observer view"): sin / cos of the solar B0 and P angles.  `on`
+// is 0 for B0 = P = 0, and the launch then picks the VIEW = false instantiation of a kernel: the fixed equatorial
+// view's code as it was, so that its results are the same bit for bit.  (A run-time branch around the rotation is not
+// enough: it changes which products the compiler contracts into FMAs elsewhere in the kernel.)
+struct ViewRot {
+    int on;
+    double sb, cb, sp, cp;
+};
+
+// observer-frame point -> model-aligned point: undo P (a rotation about the line of sight z), then B0 (about x)
+__device__ __forceinline__ void view_to_model(const ViewRot &v, double &x, double &y, double &z)
+{
+    const double x1 = x * v.cp + y * v.sp, y1 = -x * v.sp + y * v.cp;
+    x = x1;
+    y = y1 * v.cb + z * v.sb;
+    z = -y1 * v.sb + z * v.cb;
+}
+
+// model-aligned vector -> observer frame: the transpose of view_to_model
+__device__ __forceinline__ void model_to_view(const ViewRot &v, double &x, double &y, double &z)
+{
+    const double y1 = y * v.cb - z * v.sb, z1 = y * v.sb + z * v.cb;
+    const double x0 = x;
+    x = x0 * v.cp - y1 * v.sp;
+    y = x0 * v.sp + y1 * v.cp;
+    z = z1;
+}
+
 struct ResampleArgs {
     SphMesh mesh;
     int nx, ny, nz;
@@ -86,17 +114,20 @@ struct ResampleArgs {
     double phi0_offset_rad, r_min, scale, fill;
     int fill_nonfinite;              // 1: NaN/inf -> fill (fill_nan is not None); 0: keep NaN
     double *out;                     // [nx][ny][nz]
+    ViewRot view;
 };
 
-// One thread per cube node.  cart_to_sph(x, -z, y, phi0) as build_rays.py:93: the solar rotation
-// axis is the cube's +y, longitude is measured in the x / -z plane.
+// One thread per cube node.  cart_to_sph(x, -z, y, phi0) as build_rays.py:93 of the model-aligned point: the solar
+// rotation axis is its +y, longitude is measured in the x / -z plane.
+template <bool VIEW>
 __global__ void __launch_bounds__(256) resample_spherical_kernel(const ResampleArgs a)
 {
     const int64_t nvox = (int64_t)a.nx * a.ny * a.nz;
     for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q < nvox;
          q += (int64_t)gridDim.x * blockDim.x) {
         const int k = (int)(q % a.nz), j = (int)((q / a.nz) % a.ny), i = (int)(q / ((int64_t)a.ny * a.nz));
-        const double x = a.xg[i], y = a.yg[j], z = a.zg[k];
+        double x = a.xg[i], y = a.yg[j], z = a.zg[k];
+        if constexpr (VIEW) view_to_model(a.view, x, y, z);
         const double cx = x, cy = -z, cz = y;
         const double r = sqrt(cx * cx + cy * cy + cz * cz);
         const double colat = acos(fmin(1.0, fmax(-1.0, cz / r)));
@@ -120,18 +151,22 @@ struct LosArgs {
     int nx, ny, nz;
     double phi0_offset_rad, r_min, scale, z_eps;   // z_eps = 1e-6 m in R_sun (:199, :201)
     double *out;                  // [ny][nx][nz]
+    ViewRot view;
 };
 
+// The LOS geometry is spherical, so it is laid out in the observer frame; only the sample point is turned to the model.
+template <bool VIEW>
 __global__ void __launch_bounds__(256) los_spherical_kernel(const LosArgs a)
 {
     const int64_t total = (int64_t)a.ny * a.nx * a.nz;
     for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q < total;
          q += (int64_t)gridDim.x * blockDim.x) {
         const int k = (int)(q % a.nz), j = (int)((q / a.nz) % a.nx), i = (int)(q / ((int64_t)a.nx * a.nz));
-        const double x = a.x[j], y = a.y[i];
+        double x = a.x[j], y = a.y[i];
         const double rho2 = x * x + y * y;
         const double z0 = (sqrt(rho2) < 1.0) ? sqrt(1.0 - rho2) - a.z_eps : -sqrt(rho2 - 1.0) - a.z_eps;
-        const double z = z0 + a.zc[k];
+        double z = z0 + a.zc[k];
+        if constexpr (VIEW) view_to_model(a.view, x, y, z);
         const double cx = x, cy = -z, cz = y;
         const double r = sqrt(cx * cx + cy * cy + cz * cz);
         const double colat = acos(fmin(1.0, fmax(-1.0, cz / r)));
@@ -184,6 +219,17 @@ __device__ __forceinline__ void sph_to_cube_b(double x, double y, double z, doub
     bx = mx; by = mz; bz = -my;                        // model (mx,my,mz) -> cube: x = mx, z = -my, y = mz
 }
 
+// sph_to_cube_b in the observer's view: the components are taken at the model-aligned point and the vector is turned
+// back to the observer frame.  (x, y, z) is the observer-frame point.  VIEW = false: sph_to_cube_b itself.
+template <bool VIEW>
+__device__ __forceinline__ void sph_to_view_b(const ViewRot &v, double x, double y, double z, double br, double bt,
+                                              double bp, double &bx, double &by, double &bz)
+{
+    if constexpr (VIEW) view_to_model(v, x, y, z);
+    sph_to_cube_b(x, y, z, br, bt, bp, bx, by, bz);
+    if constexpr (VIEW) model_to_view(v, bx, by, bz);
+}
+
 // script/resample_with_ray_tracing.py:269-293 on device: rho -> omega_pe (f64, for the gradient
 // kernel) and n_e >= 0; T NaN -> 1e4; |B| = sqrt(br^2+bt^2+bp^2); optional Cartesian B vector.
 struct ComposeArgs {
@@ -192,8 +238,10 @@ struct ComposeArgs {
     const double *xg, *yg, *zg;
     double *omega_pe;                        // out f64
     float4 *fcube, *bcube;                   // out {ne, te, |B|, 0}, {bx, by, bz, 0} (bcube may be null)
+    ViewRot view;                            // the view the slots were resampled with: B is turned back with it
 };
 
+template <bool VIEW>
 __global__ void __launch_bounds__(256) compose_cubes_kernel(const ComposeArgs a)
 {
     const int64_t nvox = (int64_t)a.nx * a.ny * a.nz;
@@ -212,7 +260,7 @@ __global__ void __launch_bounds__(256) compose_cubes_kernel(const ComposeArgs a)
         if (a.bcube) {
             const int k = (int)(q % a.nz), j = (int)((q / a.nz) % a.ny), i = (int)(q / ((int64_t)a.ny * a.nz));
             double bx, by, bz;
-            sph_to_cube_b(a.xg[i], a.yg[j], a.zg[k], br, bt, bp, bx, by, bz);
+            sph_to_view_b<VIEW>(a.view, a.xg[i], a.yg[j], a.zg[k], br, bt, bp, bx, by, bz);
             a.bcube[q] = make_float4((float)bx, (float)by, (float)bz, 0.0f);
         }
     }

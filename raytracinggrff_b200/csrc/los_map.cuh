@@ -41,6 +41,7 @@ struct LosMapArgs {
     double *tb, *vi;                     // [freq][ny][nx]
     double *diag;                        // [RTGRFF_N_DIAG][freq][ny][nx], the DIAG variants only
     unsigned long long *valid_samples;
+    ViewRot view;                        // the observer's B0 / P (cube_builder.cuh)
 };
 
 // dynamic shared memory: FreqC[fg] | float ne, te, b, cth, sth [kLosChunk][32] | double nodes[n_nodes]
@@ -62,8 +63,9 @@ __device__ __forceinline__ void tb_vi_los(double IL, double IR, double nu, doubl
     vi = (l - r) / (l + r);
 }
 
-// NEED_BETWEEN: gyroresonance on or theta from the B vector (BVEC); DIAG: the planes of rtgrff_render_map_diag
-template <bool BVEC, bool NEED_BETWEEN, bool DIAG>
+// NEED_BETWEEN: gyroresonance on or theta from the B vector (BVEC); DIAG: the planes of rtgrff_render_map_diag;
+// VIEW: a non-zero observer view (ViewRot, cube_builder.cuh)
+template <bool BVEC, bool NEED_BETWEEN, bool DIAG, bool VIEW>
 __global__ void __launch_bounds__(kLosMaxFreqGroup * 32, 2) los_map_kernel(const LosMapArgs a)
 {
     extern __shared__ double smem_d[];
@@ -112,7 +114,9 @@ __global__ void __launch_bounds__(kLosMaxFreqGroup * 32, 2) los_map_kernel(const
                 const double x = a.x[j], y = a.y[i];
                 const double z = los_z0(x, y, a.z_eps) + a.zc[k];
                 double lon, lat, r;
-                los_sph(x, y, z, a.phi0_offset_rad, lon, lat, r);
+                double mx = x, my = y, mz = z;      // the sample point in model-aligned axes
+                if constexpr (VIEW) view_to_model(a.view, mx, my, mz);
+                los_sph(mx, my, mz, a.phi0_offset_rad, lon, lat, r);
                 if (r >= a.r_min) {
                     // the values resample_MAS stores, |B| in FP64 (los.py), SyntheticFF's NaN filter
                     const double rho = sample_spherical(mesh[0], lon, lat, r) * a.scale[0];
@@ -127,7 +131,7 @@ __global__ void __launch_bounds__(kLosMaxFreqGroup * 32, 2) los_map_kernel(const
                         if (BVEC && bm > 0.0) {
                             // theta between B and the propagation direction +z (towards the observer)
                             double bx, by, bz;
-                            sph_to_cube_b(x, y, z, br, bt, bp, bx, by, bz);
+                            sph_to_view_b<VIEW>(a.view, x, y, z, br, bt, bp, bx, by, bz);
                             cth = (float)fmin(1.0, fmax(-1.0, bz / bm));
                             sth = (float)fmin(1.0, sqrt(bx * bx + by * by) / bm);
                         }

@@ -89,6 +89,32 @@ static int check_ascending_nodes(const double *phi, int np, const double *lat, i
     return RTGRFF_OK;
 }
 
+// sin and cos of an angle in degrees, exact at multiples of 90 deg (so that P = 90 is an exact quarter turn)
+static void sincos_deg(double deg, double &s, double &c)
+{
+    const double q = deg / 90.0;
+    if (q == floor(q) && fabs(q) < 1e15) {
+        const int k = (int)(((long long)q % 4 + 4) % 4);
+        s = (k == 1) ? 1.0 : (k == 3) ? -1.0 : 0.0;
+        c = (k == 0) ? 1.0 : (k == 2) ? -1.0 : 0.0;
+        return;
+    }
+    s = sin(deg * M_PI / 180.0);
+    c = cos(deg * M_PI / 180.0);
+}
+
+// The observer's view (include/rtgrff.h, "Observer view"): finite angles, |B0| <= 90 deg.  B0 = P = 0 leaves the
+// rotation off: the launches pick the VIEW = false kernels, the fixed equatorial view's code.
+static int view_from(double b0_deg, double p_deg, ViewRot &v)
+{
+    if (!isfinite(b0_deg) || !isfinite(p_deg)) return fail(RTGRFF_EINVAL, "view angles must be finite (b0 %g, p %g)", b0_deg, p_deg);
+    if (fabs(b0_deg) > 90.0) return fail(RTGRFF_EINVAL, "|b0| must be <= 90 deg (b0 %g)", b0_deg);
+    v.on = (b0_deg != 0.0 || p_deg != 0.0) ? 1 : 0;
+    sincos_deg(b0_deg, v.sb, v.cb);
+    sincos_deg(p_deg, v.sp, v.cp);
+    return RTGRFF_OK;
+}
+
 static RayCube ray_cube_of(const rtgrff_ctx *c)
 {
     RayCube r;
@@ -603,10 +629,22 @@ int rtgrff_resample_spherical(rtgrff_ctx *c, int slot, const float *data, const 
                               double phi0_offset_deg, double r_min, double scale, double fill, int fill_nonfinite,
                               double *out)
 {
+    return rtgrff_resample_spherical_view(c, slot, data, phi, lat, r, np, nt, nr, x_grid, y_grid, z_grid, nx, ny, nz, geom,
+                                          phi0_offset_deg, 0.0, 0.0, r_min, scale, fill, fill_nonfinite, out);
+}
+
+int rtgrff_resample_spherical_view(rtgrff_ctx *c, int slot, const float *data, const double *phi, const double *lat,
+                                   const double *r, int np, int nt, int nr, const double *x_grid, const double *y_grid,
+                                   const double *z_grid, int nx, int ny, int nz, const double geom[12],
+                                   double phi0_offset_deg, double b0_deg, double p_deg, double r_min, double scale,
+                                   double fill, int fill_nonfinite, double *out)
+{
     RT_USE(c);
     if (slot < 0 || slot > 4) return fail(RTGRFF_EINVAL, "slot %d out of range 0..4", slot);
     if (!data || !phi || !lat || !r || !geom || !x_grid || !y_grid || !z_grid) return fail(RTGRFF_EINVAL, "null argument");
     if (np < 2 || nt < 2 || nr < 2) return fail(RTGRFF_EINVAL, "spherical mesh needs >= 2 nodes per axis");
+    ViewRot view;
+    RT_TRY(view_from(b0_deg, p_deg, view));
     GridGeom g;
     RT_TRY(geom_from(geom, nx, ny, nz, g));
     RT_TRY(check_ascending_nodes(phi, np, lat, nt, r, nr));
@@ -633,12 +671,14 @@ int rtgrff_resample_spherical(rtgrff_ctx *c, int slot, const float *data, const 
     a.xg = gx; a.yg = gx + nx; a.zg = gx + nx + ny;
     a.phi0_offset_rad = phi0_offset_deg * M_PI / 180.0;
     a.r_min = r_min; a.scale = scale; a.fill = fill; a.fill_nonfinite = fill_nonfinite;
+    a.view = view;
     a.out = c->slot[slot].as<double>();
     unsigned int blocks = blocks_for((int64_t)nvox, 256);
     const unsigned int cap = (unsigned int)c->sm_count * 32;
     if (blocks > cap) blocks = cap;
     RT_CUDA(cudaEventRecord(c->ev0, c->stream));
-    resample_spherical_kernel<<<blocks, 256, 0, c->stream>>>(a);
+    if (view.on) resample_spherical_kernel<true><<<blocks, 256, 0, c->stream>>>(a);
+    else resample_spherical_kernel<false><<<blocks, 256, 0, c->stream>>>(a);
     RT_TRY(launched(c, "resample_spherical_kernel"));
     RT_CUDA(cudaEventRecord(c->ev1, c->stream));
     c->ev_valid = true;
@@ -648,6 +688,7 @@ int rtgrff_resample_spherical(rtgrff_ctx *c, int slot, const float *data, const 
     c->slot_nx = nx; c->slot_ny = ny; c->slot_nz = nz;
     memcpy(c->slot_geom, geom, sizeof(c->slot_geom));
     memcpy(c->slot_geoms[slot], geom, sizeof(c->slot_geom));
+    c->slot_views[slot][0] = b0_deg; c->slot_views[slot][1] = p_deg;
     return RTGRFF_OK;
 }
 
@@ -656,9 +697,20 @@ int rtgrff_sample_spherical_los(rtgrff_ctx *c, const float *data, const double *
                                 int ny, int nz, double phi0_offset_deg, double r_min, double scale, double z_eps,
                                 double *out)
 {
+    return rtgrff_sample_spherical_los_view(c, data, phi, lat, r, np, nt, nr, x, y, zc, nx, ny, nz, phi0_offset_deg, 0.0,
+                                            0.0, r_min, scale, z_eps, out);
+}
+
+int rtgrff_sample_spherical_los_view(rtgrff_ctx *c, const float *data, const double *phi, const double *lat,
+                                     const double *r, int np, int nt, int nr, const double *x, const double *y,
+                                     const double *zc, int nx, int ny, int nz, double phi0_offset_deg, double b0_deg,
+                                     double p_deg, double r_min, double scale, double z_eps, double *out)
+{
     RT_USE(c);
     if (!data || !phi || !lat || !r || !x || !y || !zc || !out) return fail(RTGRFF_EINVAL, "null argument");
     if (np < 2 || nt < 2 || nr < 2 || nx < 1 || ny < 1 || nz < 1) return fail(RTGRFF_EINVAL, "bad sizes");
+    ViewRot view;
+    RT_TRY(view_from(b0_deg, p_deg, view));
     RT_TRY(check_ascending_nodes(phi, np, lat, nt, r, nr));
     const size_t total = (size_t)nx * ny * nz, nd = (size_t)np * nt * nr;
     RT_TRY(h2d(c, c->in0, data, nd * sizeof(float)));
@@ -682,12 +734,14 @@ int rtgrff_sample_spherical_los(rtgrff_ctx *c, const float *data, const double *
     a.nx = nx; a.ny = ny; a.nz = nz;
     a.phi0_offset_rad = phi0_offset_deg * M_PI / 180.0;
     a.r_min = r_min; a.scale = scale; a.z_eps = z_eps;
+    a.view = view;
     a.out = c->out0.as<double>();
     unsigned int blocks = blocks_for((int64_t)total, 256);
     const unsigned int cap = (unsigned int)c->sm_count * 32;
     if (blocks > cap) blocks = cap;
     RT_CUDA(cudaEventRecord(c->ev0, c->stream));
-    los_spherical_kernel<<<blocks, 256, 0, c->stream>>>(a);
+    if (view.on) los_spherical_kernel<true><<<blocks, 256, 0, c->stream>>>(a);
+    else los_spherical_kernel<false><<<blocks, 256, 0, c->stream>>>(a);
     RT_TRY(launched(c, "los_spherical_kernel"));
     RT_CUDA(cudaEventRecord(c->ev1, c->stream));
     c->ev_valid = true;
@@ -706,6 +760,12 @@ int rtgrff_compose_cubes(rtgrff_ctx *c, int want_bvec)
     for (int s = 0; s < 5; ++s)
         if (memcmp(c->slot_geoms[s], geom, sizeof(c->slot_geom)) != 0)
             return fail(RTGRFF_EINVAL, "spherical slot %d was resampled on a different cube geometry than the last one", s);
+    for (int s = 1; s < 5; ++s)
+        if (memcmp(c->slot_views[s], c->slot_views[0], sizeof(c->slot_views[0])) != 0)
+            return fail(RTGRFF_EINVAL, "spherical slot %d was resampled with view (b0 %g, p %g), slot 0 with (b0 %g, p %g)",
+                        s, c->slot_views[s][0], c->slot_views[s][1], c->slot_views[0][0], c->slot_views[0][1]);
+    ViewRot view;
+    RT_TRY(view_from(c->slot_views[0][0], c->slot_views[0][1], view));
     GridGeom g;
     RT_TRY(geom_from(geom, nx, ny, nz, g));
     const size_t nvox = (size_t)nx * ny * nz;
@@ -721,8 +781,10 @@ int rtgrff_compose_cubes(rtgrff_ctx *c, int want_bvec)
     a.omega_pe = c->stage.as<double>();
     a.fcube = c->fcube.as<float4>();
     a.bcube = want_bvec ? c->bcube.as<float4>() : nullptr;
+    a.view = view;
     unsigned int blocks = blocks_for((int64_t)nvox, 256);
-    compose_cubes_kernel<<<blocks, 256, 0, c->stream>>>(a);
+    if (view.on) compose_cubes_kernel<true><<<blocks, 256, 0, c->stream>>>(a);
+    else compose_cubes_kernel<false><<<blocks, 256, 0, c->stream>>>(a);
     RT_TRY(launched(c, "compose_cubes_kernel"));
     build_ray_cube_kernel<<<blocks, 256, 0, c->stream>>>(c->stage.as<double>(), c->wcube.as<float4>(), nx, ny, nz,
                                                           geom[3], geom[7], geom[11]);
@@ -1394,8 +1456,21 @@ int rtgrff_render_los_map(rtgrff_ctx *c, int nx, int ny, const double *x, const 
                           const double *freq_hz, double pixel_area_cm2, int em_flag, int s_max, int use_bvec, double *tb,
                           double *vi, double *diag, int out_on_device, int64_t *stats)
 {
+    return rtgrff_render_los_map_view(c, nx, ny, x, y, nz, zc, dz_cm, phi0_offset_deg, 0.0, 0.0, r_min, z_eps, n_freq,
+                                      freq_hz, pixel_area_cm2, em_flag, s_max, use_bvec, tb, vi, diag, out_on_device,
+                                      stats);
+}
+
+int rtgrff_render_los_map_view(rtgrff_ctx *c, int nx, int ny, const double *x, const double *y, int nz,
+                               const double *zc, const double *dz_cm, double phi0_offset_deg, double b0_deg,
+                               double p_deg, double r_min, double z_eps, int n_freq, const double *freq_hz,
+                               double pixel_area_cm2, int em_flag, int s_max, int use_bvec, double *tb, double *vi,
+                               double *diag, int out_on_device, int64_t *stats)
+{
     RT_USE(c);
     if (!x || !y || !zc || !dz_cm || !freq_hz || !tb || !vi) return fail(RTGRFF_EINVAL, "null argument");
+    ViewRot view;
+    RT_TRY(view_from(b0_deg, p_deg, view));
     if (nx < 1 || ny < 1 || nz < 1 || n_freq < 1) return fail(RTGRFF_EINVAL, "bad sizes (nx %d, ny %d, nz %d, n_freq %d)",
                                                               nx, ny, nz, n_freq);
     if ((int64_t)nx * ny >= (int64_t)1 << 31) return fail(RTGRFF_EINVAL, "image larger than 2^31 pixels");
@@ -1446,6 +1521,7 @@ int rtgrff_render_los_map(rtgrff_ctx *c, int nx, int ny, const double *x, const 
     a.tiles_x = (nx + kLosTileW - 1) / kLosTileW;
     a.phi0_offset_rad = phi0_offset_deg * M_PI / 180.0;
     a.r_min = r_min; a.z_eps = z_eps;
+    a.view = view;
     a.freqs = c->in1.as<FreqC>();
     a.n_freq = n_freq; a.fg = fg;
     a.area = pixel_area_cm2;
@@ -1462,17 +1538,20 @@ int rtgrff_render_los_map(rtgrff_ctx *c, int nx, int ny, const double *x, const 
     const bool gr = !(em_flag & 1);
     const int variant = (use_bvec ? 4 : 0) | (use_bvec || gr ? 2 : 0) | (diag ? 1 : 0);
     RT_CUDA(cudaEventRecord(c->ev0, c->stream));
-#define RT_LOS_CASE(v, BV, NB, DG)                                                                                \
-    case v:                                                                                                       \
-        if (smem > 48 * 1024)                                                                                     \
-            RT_CUDA(cudaFuncSetAttribute(los_map_kernel<BV, NB, DG>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                         (int)smem));                                                             \
-        los_map_kernel<BV, NB, DG><<<grid, block, smem, c->stream>>>(a);                                          \
+#define RT_LOS_CASE(v, BV, NB, DG, VW)                                                                                \
+    case v:                                                                                                           \
+        if (smem > 48 * 1024)                                                                                         \
+            RT_CUDA(cudaFuncSetAttribute(los_map_kernel<BV, NB, DG, VW>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
+                                         (int)smem));                                                                 \
+        los_map_kernel<BV, NB, DG, VW><<<grid, block, smem, c->stream>>>(a);                                          \
         break;
-    switch (variant) {
-        RT_LOS_CASE(0, false, false, false) RT_LOS_CASE(1, false, false, true)
-        RT_LOS_CASE(2, false, true, false) RT_LOS_CASE(3, false, true, true)
-        RT_LOS_CASE(6, true, true, false) RT_LOS_CASE(7, true, true, true)
+    switch (variant | (view.on ? 8 : 0)) {
+        RT_LOS_CASE(0, false, false, false, false) RT_LOS_CASE(1, false, false, true, false)
+        RT_LOS_CASE(2, false, true, false, false) RT_LOS_CASE(3, false, true, true, false)
+        RT_LOS_CASE(6, true, true, false, false) RT_LOS_CASE(7, true, true, true, false)
+        RT_LOS_CASE(8, false, false, false, true) RT_LOS_CASE(9, false, false, true, true)
+        RT_LOS_CASE(10, false, true, false, true) RT_LOS_CASE(11, false, true, true, true)
+        RT_LOS_CASE(14, true, true, false, true) RT_LOS_CASE(15, true, true, true, true)
     }
 #undef RT_LOS_CASE
     RT_TRY(launched(c, "los_map_kernel"));

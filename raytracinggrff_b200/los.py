@@ -19,6 +19,7 @@ import numpy as np
 
 from . import _lib
 from ._lib import check, f32, f64, ptr
+from .cubes import check_view
 from .session import RaySession
 
 R_sun_cm = 6.957e10     # script/resampling_MAS_LOS.py constants
@@ -41,14 +42,16 @@ def z_grid(N_z, dz0, variable_spacing_z=True, z_range=None):
     return z, np.abs(np.diff(z, prepend=z[0]))
 
 
-def _sample_los(ctx, var, x, y, zc, phi0_offset, r_min):
+def _sample_los(ctx, var, x, y, zc, phi0_offset, r_min, b0_angle, p_angle):
     data = f32(var.data)
     phi, lat, r = f64(var.phi), f64(var.lat), f64(var.r)
     out = np.empty((len(y), len(x), len(zc)), dtype=np.float64)
-    check(_lib.load().rtgrff_sample_spherical_los(ctx.handle, ptr(data, c_float), ptr(phi, c_double), ptr(lat, c_double),
-                                                  ptr(r, c_double), *data.shape, ptr(x, c_double), ptr(y, c_double),
-                                                  ptr(zc, c_double), len(x), len(y), len(zc), float(phi0_offset),
-                                                  float(r_min), float(var.scale), 1e-6 / R_sun_m, ptr(out, c_double)))
+    check(_lib.load().rtgrff_sample_spherical_los_view(ctx.handle, ptr(data, c_float), ptr(phi, c_double),
+                                                       ptr(lat, c_double), ptr(r, c_double), *data.shape,
+                                                       ptr(x, c_double), ptr(y, c_double), ptr(zc, c_double), len(x),
+                                                       len(y), len(zc), float(phi0_offset), b0_angle, p_angle,
+                                                       float(r_min), float(var.scale), 1e-6 / R_sun_m,
+                                                       ptr(out, c_double)))
     return out
 
 
@@ -66,15 +69,18 @@ def _check_model(model, dz0, variable_spacing_z):
 
 
 def resample_MAS(model, N_pix, X_range, Y_range, N_z, dz0, variable_spacing_z=True, z_range=None,
-                 out_path="LOS_data.npz", save_plots=False, verbose=True, phi0_offset=0.0, r_min=R_MIN, context=None):
+                 out_path="LOS_data.npz", save_plots=False, verbose=True, phi0_offset=0.0, r_min=R_MIN, context=None,
+                 b0_angle=0.0, p_angle=0.0):
     """Returns {'Ne_LOS','Te_LOS','B_LOS','ds_LOS' (N_pix,N_pix,N_z) [cm^-3, K, G, cm], 'x_coords',
-    'y_coords','z_coords' [m]} and writes them to `out_path` (script/resampling_MAS_LOS.py:288-300)."""
+    'y_coords','z_coords' [m]} and writes them to `out_path` (script/resampling_MAS_LOS.py:288-300).
+    b0_angle, p_angle [deg]: the observer's view of the model (include/rtgrff.h, "Observer view")."""
     temp = _check_model(model, dz0, variable_spacing_z)
+    b0, p = check_view(b0_angle, p_angle)
     ctx = context or _lib.default_context()
     zc, dz = z_grid(N_z, dz0, variable_spacing_z, z_range)
     xs = np.linspace(X_range[0], X_range[1], N_pix)
     ys = np.linspace(Y_range[0], Y_range[1], N_pix)
-    s = {k: _sample_los(ctx, model[k], xs, ys, zc, phi0_offset, r_min) for k in ("rho", temp, "br", "bt", "bp")}
+    s = {k: _sample_los(ctx, model[k], xs, ys, zc, phi0_offset, r_min, b0, p) for k in ("rho", temp, "br", "bt", "bp")}
     B = np.sqrt(s["br"] ** 2 + s["bt"] ** 2 + s["bp"] ** 2)
     invalid = np.isnan(s["rho"])
     for a in (s[temp], B):
@@ -136,13 +142,15 @@ def SyntheticFF(fname_input, freq0, Nfreq, freq_log_step, fname_output=None, do_
 
 def render_los_map(model, N_pix, X_range, Y_range, N_z, dz0, freq0, Nfreq, freq_log_step, variable_spacing_z=True,
                    z_range=None, phi0_offset=0.0, r_min=R_MIN, em_flag=5, s_max=30, use_bvec=False, diagnostics=False,
-                   fname_output=None, session=None):
+                   fname_output=None, session=None, b0_angle=0.0, p_angle=0.0):
     """resample_MAS followed by SyntheticFF in one fused kernel: the same LOS geometry and samples, the same packing
     rules and T_b / V/I, with nothing materialised (no LOS arrays, no Parms).  Returns (and writes to
     ``fname_output + '.npz'``) SyntheticFF's dict.  Beyond the reference: em_flag (4 adds gyroresonance), use_bvec
     (theta from the B vector instead of 90 deg) and diagnostics=True, which adds the keys of
-    workflow.diagnostic_maps (emission centroid, emission height, optical depths, the LOS's smallest r)."""
+    workflow.diagnostic_maps (emission centroid, emission height, optical depths, the LOS's smallest r), and the
+    observer's view b0_angle, p_angle [deg] (include/rtgrff.h, "Observer view")."""
     _check_model(model, dz0, variable_spacing_z)
+    check_view(b0_angle, p_angle)
     if int(N_pix) < 2:
         raise ValueError("N_pix must be >= 2 (the pixel area comes from the x spacing)")
     if int(Nfreq) < 1:
@@ -159,7 +167,7 @@ def render_los_map(model, N_pix, X_range, Y_range, N_z, dz0, freq0, Nfreq, freq_
     ses.set_spherical_model(model)
     out = ses.render_los_map(xs, ys, zc, dz * R_sun_cm, frequencies_Hz, phi0_offset=phi0_offset, r_min=r_min,
                              z_eps=1e-6 / R_sun_m, pixel_area_cm2=area, em_flag=em_flag, s_max=s_max,
-                             use_bvec=use_bvec, diagnostics=diagnostics)
+                             use_bvec=use_bvec, diagnostics=diagnostics, b0_angle=b0_angle, p_angle=p_angle)
     tb, vi = out[0], out[1]
     result = {"emission_cube": np.ascontiguousarray(np.moveaxis(tb, 0, -1)),
               "emission_polVI_cube": np.ascontiguousarray(np.moveaxis(vi, 0, -1)),

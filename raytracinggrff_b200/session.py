@@ -114,12 +114,15 @@ class RaySession:
                                                *shape, ptr(geom, c_double)))
         keys["fields"] = key
 
-    def set_model_from_spherical(self, model, x_grid, y_grid, z_grid, phi0_offset=0.0, want_bvec=False):
+    def set_model_from_spherical(self, model, x_grid, y_grid, z_grid, phi0_offset=0.0, want_bvec=False, b0_angle=0.0,
+                                 p_angle=0.0):
         """Cubes straight from a spherical (phi, latitude, r) model, never visiting the host
-        (cubes.set_model_from_spherical; script/resample_with_ray_tracing.py:263-293)."""
+        (cubes.set_model_from_spherical; script/resample_with_ray_tracing.py:263-293), seen from the observer view
+        b0_angle, p_angle [deg] (include/rtgrff.h, "Observer view")."""
         from . import cubes
         self.ctx.__dict__["_cube_keys"] = {}
-        cubes.set_model_from_spherical(self, model, x_grid, y_grid, z_grid, phi0_offset, want_bvec)
+        cubes.set_model_from_spherical(self, model, x_grid, y_grid, z_grid, phi0_offset, want_bvec, b0_angle=b0_angle,
+                                       p_angle=p_angle)
         self.cube_shape = (len(x_grid), len(y_grid), len(z_grid))
 
     def set_spherical_model(self, model):
@@ -451,13 +454,17 @@ class RaySession:
     # -- fused straight line-of-sight map ---------------------------------------------------------
     def render_los_map(self, x, y, zc, dz_cm, freq_hz, phi0_offset=0.0, r_min=0.9999999, z_eps=1e-6 / 6.957e8,
                        pixel_area_cm2=1.0, em_flag=5, s_max=30, use_bvec=False, diagnostics=False,
-                       out_device_ptrs=None):
+                       out_device_ptrs=None, b0_angle=0.0, p_angle=0.0):
         """Straight-LOS map from the model set_spherical_model left on the device (rtgrff_render_los_map): pixel
         (i, j) at (x[j], y[i]) [R_sun], LOS samples at the cumulative offsets zc [R_sun] with segment lengths dz_cm
         [cm], any list of frequencies [Hz].  Returns (tb, vi, stats), tb and vi (n_freq, ny, nx) float64, stats
         {los_samples, valid_samples, voxel_freq_evaluations}; with diagnostics=True (tb, vi, stats, diag), diag a
         dict of (n_freq, ny, nx) planes with render_map_diag's keys.  With out_device_ptrs=(tb_ptr, vi_ptr[,
-        diag_ptr]) the results go to those device buffers and the arrays returned are None."""
+        diag_ptr]) the results go to those device buffers and the arrays returned are None.  b0_angle, p_angle [deg]:
+        the observer's view of the model (include/rtgrff.h, "Observer view"); the diagnostic planes stay in the
+        observer frame."""
+        from .cubes import check_view
+        b0, p = check_view(b0_angle, p_angle)
         xs, ys, z, d = f64(x).ravel(), f64(y).ravel(), f64(zc).ravel(), f64(dz_cm).ravel()
         fr = f64(np.atleast_1d(freq_hz)).ravel()
         if len(d) != len(z):
@@ -477,10 +484,11 @@ class RaySession:
                 raise ValueError("out_device_ptrs must be (tb_ptr, vi_ptr) or, with diagnostics, (tb_ptr, vi_ptr, diag_ptr)")
             ptb, pvi, on_dev = ctypes.c_void_p(out_device_ptrs[0]), ctypes.c_void_p(out_device_ptrs[1]), 1
             pdg = ctypes.c_void_p(out_device_ptrs[2]) if diagnostics else None
-        check(self._lib.rtgrff_render_los_map(self.ctx.handle, nx, ny, ptr(xs, c_double), ptr(ys, c_double), len(z),
-                                              ptr(z, c_double), ptr(d, c_double), float(phi0_offset), float(r_min),
-                                              float(z_eps), nf, ptr(fr, c_double), float(pixel_area_cm2), int(em_flag),
-                                              int(s_max), int(bool(use_bvec)), ptb, pvi, pdg, on_dev, stats))
+        check(self._lib.rtgrff_render_los_map_view(self.ctx.handle, nx, ny, ptr(xs, c_double), ptr(ys, c_double),
+                                                   len(z), ptr(z, c_double), ptr(d, c_double), float(phi0_offset), b0, p,
+                                                   float(r_min), float(z_eps), nf, ptr(fr, c_double),
+                                                   float(pixel_area_cm2), int(em_flag), int(s_max), int(bool(use_bvec)),
+                                                   ptb, pvi, pdg, on_dev, stats))
         st = {"los_samples": int(stats[0]), "valid_samples": int(stats[1]), "voxel_freq_evaluations": int(stats[2])}
         if not diagnostics:
             return tb, vi, st

@@ -76,12 +76,15 @@ def select_params(freq_hz):
 
 def tb_spectra(model, out_dir, N_pix=128, fmin_mhz=30.0, fmax_mhz=800.0, n_freq=30, start_from_idx=0,
                phi0_offset=-140.0, session=None, quiet=True, params_fn=select_params, use_bvec=False,
-               em_flag=5, max_grid_n=None, diagnostics=False):
+               em_flag=5, max_grid_n=None, diagnostics=False, b0_angle=0.0, p_angle=0.0):
     """Run the sweep.  `model` is a spherical model (cubes.SphericalVariable mapping).  Returns the
     manifest rows [(idx, freq_hz, npz_path)].  Existing files of indices < start_from_idx are kept
     (the reference's resume switch, :118-119, :141-142).  diagnostics=True: every npz also holds the keys of
     workflow.diagnostic_maps (emission centroid and height, optical depths, ray turning point), which over the
-    sweep give the emission height against frequency."""
+    sweep give the emission height against frequency.  b0_angle, p_angle [deg]: the observer's view of the model
+    (include/rtgrff.h, "Observer view")."""
+    from .cubes import check_view
+    b0_angle, p_angle = check_view(b0_angle, p_angle)
     out_dir = Path(out_dir)
     out_dir.mkdir(parents=True, exist_ok=True)
     freqs_hz = np.logspace(np.log10(fmin_mhz), np.log10(fmax_mhz), n_freq) * 1e6
@@ -99,7 +102,8 @@ def tb_spectra(model, out_dir, N_pix=128, fmin_mhz=30.0, fmax_mhz=800.0, n_freq=
                 print(f"[{i+1:02d}/{len(freqs_hz)}] {freq_hz/1e6:8.3f} MHz | grid_n={grid_n} X_FOV={p['x_fov']:.3f} "
                       f"z_obs={p['z_observer']:.3f} dt={p['dt']:.3g} n_steps={p['n_steps']} stride={p['record_stride']}")
             g = np.linspace(-p["grid_extent"], p["grid_extent"], grid_n)       # script/...:263-265
-            ses.set_model_from_spherical(model, g, g, g, phi0_offset=phi0_offset, want_bvec=use_bvec)
+            ses.set_model_from_spherical(model, g, g, g, phi0_offset=phi0_offset, want_bvec=use_bvec, b0_angle=b0_angle,
+                                         p_angle=p_angle)
             xs, ys, zs, kv = synthetic.ray_launch_geometry(N_pix, float(p["x_fov"]), float(p["z_observer"]))
             area = pixel_area_cm2(float(p["x_fov"]), N_pix)
             render = ses.render_map_diag if diagnostics else ses.render_map
@@ -132,6 +136,10 @@ def main(argv=None):
     ap.add_argument("--n-freq", type=int, default=30)
     ap.add_argument("--start-from-idx", type=int, default=0)
     ap.add_argument("--phi0-offset", type=float, default=-140.0)
+    ap.add_argument("--b0-angle", type=float, default=0.0,
+                    help="solar B0 angle of the observer [deg], > 0 tilts the north pole towards the observer")
+    ap.add_argument("--p-angle", type=float, default=0.0,
+                    help="solar P angle of the observer [deg], > 0 turns north from image up towards east (left)")
     ap.add_argument("--device", default="cuda", choices=["cpu", "cuda"])
     ap.add_argument("--raytrace-device", default="cuda", choices=["cpu", "cuda"])
     ap.add_argument("--quiet", "-q", action="store_true")
@@ -142,7 +150,7 @@ def main(argv=None):
         raise RuntimeError("raytracinggrff_b200 is CUDA-only (no CPU path, no fallback)")
     model = synthetic.spherical_corona(150, 110, 128, r_max=8.0, active_region=True)
     rows = tb_spectra(model, a.out_dir, a.N_pix, a.fmin_mhz, a.fmax_mhz, a.n_freq, a.start_from_idx, a.phi0_offset,
-                      quiet=a.quiet, diagnostics=a.diagnostics)
+                      quiet=a.quiet, diagnostics=a.diagnostics, b0_angle=a.b0_angle, p_angle=a.p_angle)
     print(f"Saved {len(rows)} maps to {a.out_dir}")
 
 

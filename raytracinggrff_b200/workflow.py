@@ -80,7 +80,7 @@ def pack_parms_batch(sampled, area, s_input_on=False):
     return Parms_M
 
 
-def _upload_model(ses, model, grid_n, grid_extent, phi0_offset):
+def _upload_model(ses, model, grid_n, grid_extent, phi0_offset, b0_angle=0.0, p_angle=0.0):
     if "omega_pe" in model:
         xg, yg, zg = model["x_grid"], model["y_grid"], model["z_grid"]
         ses.set_omega_cube(model["omega_pe"], xg, yg, zg)
@@ -88,7 +88,7 @@ def _upload_model(ses, model, grid_n, grid_extent, phi0_offset):
     else:
         # a spherical (phi, latitude, r) model: the cube resampling of :251-293 on the GPU
         xg = yg = zg = np.linspace(-grid_extent, grid_extent, int(grid_n))
-        ses.set_model_from_spherical(model, xg, yg, zg, phi0_offset=phi0_offset)
+        ses.set_model_from_spherical(model, xg, yg, zg, phi0_offset=phi0_offset, b0_angle=b0_angle, p_angle=p_angle)
 
 
 def diagnostic_maps(diag, N_pix):
@@ -178,14 +178,21 @@ def run_ray_tracing_emission(model, N_pix=64, X_fov=1.44, freq_hz=75e6, z_observ
                              fallback_to_cpu=False, raytrace_device="cuda", grff_backend="get_mw",
                              perturb_ratio=2, session=None, return_samples=False, s_mode="per_step",
                              grid_n=128, grid_extent=3.0, phi0_offset=0.0, consider_beam=False, beam_fwhm=0.2,
-                             diagnostics=False):
+                             diagnostics=False, b0_angle=0.0, p_angle=0.0):
     """``n_workers`` (the reference's ``--workers``, script/resample_with_ray_tracing.py:333-352: contiguous ray
     chunks over a process pool, concatenated on the ray axis) maps to GPUs here: the rays are split into
     ``n_workers`` contiguous chunks exactly as there, chunk k runs on GPU k mod (number of visible GPUs) from its
     own host thread (the library calls release the GIL) with its own context and a replica of the cubes, and the
     chunks' maps are concatenated.  Rays never interact, so the result does not depend on the split.
     ``diagnostics`` (fused backend only): the result and the npz also hold where each pixel's emission comes from,
-    the keys of diagnostic_maps (RaySession.render_map_diag); every other key is the same as without."""
+    the keys of diagnostic_maps (RaySession.render_map_diag); every other key is the same as without.
+    ``b0_angle``, ``p_angle`` [deg]: the observer's view of a spherical model (include/rtgrff.h, "Observer view"); a
+    Cartesian cube model (one with ``omega_pe``) cannot be re-oriented and takes zero angles only."""
+    from .cubes import check_view
+    b0_angle, p_angle = check_view(b0_angle, p_angle)
+    if "omega_pe" in model and (b0_angle != 0.0 or p_angle != 0.0):
+        raise ValueError("b0_angle / p_angle need a spherical model: a Cartesian cube model (omega_pe) cannot be "
+                         "re-oriented")
     if freq0 is None:
         freq0 = freq_hz
     backend = grff_backend.lower()
@@ -217,7 +224,7 @@ def run_ray_tracing_emission(model, N_pix=64, X_fov=1.44, freq_hz=75e6, z_observ
     n_workers = max(1, int(n_workers))
     if n_workers == 1 or n_rays < 2:
         ses = session or RaySession(context=_lib.default_context())
-        _upload_model(ses, model, grid_n, grid_extent, phi0_offset)
+        _upload_model(ses, model, grid_n, grid_extent, phi0_offset, b0_angle, p_angle)
         tb, vi, sampled, diag = _emission_of_rays(ses, backend, x_flat, y_flat, z_start, kvec, p,
                                                   image_shape=(N_pix, N_pix))
     else:
@@ -232,7 +239,7 @@ def run_ray_tracing_emission(model, N_pix=64, X_fov=1.44, freq_hz=75e6, z_observ
             s, e = chunks[k]
             ses_k = RaySession(device=k % n_dev)                                  # its own context, stream and cube replica
             try:
-                _upload_model(ses_k, model, grid_n, grid_extent, phi0_offset)
+                _upload_model(ses_k, model, grid_n, grid_extent, phi0_offset, b0_angle, p_angle)
                 return _emission_of_rays(ses_k, backend, x_flat[s:e], y_flat[s:e], z_start[s:e], kvec[s:e], p)
             finally:
                 ses_k.close()
@@ -300,6 +307,10 @@ def main(argv=None):
     parser.add_argument("--consider-beam", action="store_true")
     parser.add_argument("--beam-fwhm", type=float, default=0.2)
     parser.add_argument("--phi0-offset", type=float, default=0)
+    parser.add_argument("--b0-angle", type=float, default=0.0,
+                        help="solar B0 angle of the observer [deg], > 0 tilts the north pole towards the observer")
+    parser.add_argument("--p-angle", type=float, default=0.0,
+                        help="solar P angle of the observer [deg], > 0 turns north from image up towards east (left)")
     parser.add_argument("--no-fallback", action="store_true", help="accepted for compatibility; there is no CPU path to fall back to")
     parser.add_argument("--no-plots", action="store_true", help="accepted for compatibility; no plots are made")
     parser.add_argument("--quiet", "-q", action="store_true")
@@ -319,7 +330,7 @@ def main(argv=None):
         freq0=args.freq, freq_log_step=0.0, save_plots=False, verbose=not args.quiet, device=args.device,
         fallback_to_cpu=not args.no_fallback, raytrace_device=args.raytrace_device, grff_backend=args.grff_backend,
         consider_beam=args.consider_beam, beam_fwhm=args.beam_fwhm, phi0_offset=args.phi0_offset, s_mode=args.s_mode,
-        diagnostics=args.diagnostics)
+        diagnostics=args.diagnostics, b0_angle=args.b0_angle, p_angle=args.p_angle)
     if not args.quiet:
         tb = res["emission_cube"]
         print(f"T_b map {tb.shape} at {args.freq / 1e6:.1f} MHz: max {tb.max():.3e} K -> {args.out_path}")
