@@ -78,6 +78,33 @@ inline unsigned int blocks_for(int64_t n, int block)
     return (unsigned int)b;
 }
 
+// Two adjacent float4 from one 32-byte-aligned address in a single read-only load (LDG.E.ENL2.256.CONSTANT
+// on sm_100a instead of two LDG.E.128): a field node with its B vector, half of a polynomial cell.
+struct Float4x2 {
+    float4 lo, hi;
+};
+
+__device__ __forceinline__ Float4x2 ldg256(const float4 *p)
+{
+    Float4x2 r;
+    asm("ld.global.nc.v8.f32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+        : "=f"(r.lo.x), "=f"(r.lo.y), "=f"(r.lo.z), "=f"(r.lo.w), "=f"(r.hi.x), "=f"(r.hi.y), "=f"(r.hi.z), "=f"(r.hi.w)
+        : "l"(p));
+    return r;
+}
+
+// The same load without allocating the line in L1 (LDG.E.NA.ENL2.256.CONSTANT): for the fused map's field sampler.
+// Its corner lines then stay out of the L1 that the stepper's polynomial cells, re-read dozens of times a step,
+// depend on; the sampler is served from L2 instead (config-4 map -1.5 %, DESIGN.md 4.1).
+__device__ __forceinline__ Float4x2 ldg256_no_l1(const float4 *p)
+{
+    Float4x2 r;
+    asm("ld.global.nc.L1::no_allocate.v8.f32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
+        : "=f"(r.lo.x), "=f"(r.lo.y), "=f"(r.lo.z), "=f"(r.lo.w), "=f"(r.hi.x), "=f"(r.hi.y), "=f"(r.hi.z), "=f"(r.hi.w)
+        : "l"(p));
+    return r;
+}
+
 }  // namespace rtgrff
 
 struct rtgrff_ctx {
@@ -107,11 +134,13 @@ struct rtgrff_ctx {
     rtgrff::GridGeom wgeom{};
     bool has_wcube = false;
 
-    // field cubes {ne, te, |B|, 0} and {bx, by, bz, 0}
-    rtgrff::DevBuf fcube, bcube;
+    // field nodes, z fastest: {ne, te, |B|, 0} (16 B), or {ne, te, |B|, 0, bx, by, bz, 0} (32 B, 32-byte aligned) when
+    // has_bvec: a trilinear corner with its B vector is then one 32-byte load.  field_stride() gives the node stride.
+    rtgrff::DevBuf fcube;
     rtgrff::GridGeom fgeom{};
     rtgrff::GridGeomF fgeomf{};
     bool has_fcube = false, has_bvec = false;
+    int field_stride() const { return has_bvec ? 2 : 1; }   // float4 per field node
 
     // records of the last trace: positions SoA [rec][3][ray] f64, S [rec][ray] f64
     rtgrff::DevBuf rec_pos, rec_s;

@@ -237,7 +237,8 @@ struct ComposeArgs {
     int nx, ny, nz;
     const double *xg, *yg, *zg;
     double *omega_pe;                        // out f64
-    float4 *fcube, *bcube;                   // out {ne, te, |B|, 0}, {bx, by, bz, 0} (bcube may be null)
+    float4 *fcube;                           // out field nodes {ne, te, |B|, 0} (field_stride 1)
+    int field_stride;                        // or {ne, te, |B|, 0, bx, by, bz, 0} (2: the B vector wanted)
     ViewRot view;                            // the view the slots were resampled with: B is turned back with it
 };
 
@@ -256,12 +257,13 @@ __global__ void __launch_bounds__(256) compose_cubes_kernel(const ComposeArgs a)
         if (!isfinite(te)) te = 1e4;                                                 // :284
         const double br = a.br[q], bt = a.bt[q], bp = a.bp[q];
         const double b = sqrt(br * br + bt * bt + bp * bp);                          // :293
-        a.fcube[q] = make_float4((float)ne, (float)te, (float)b, 0.0f);
-        if (a.bcube) {
+        float4 *node = a.fcube + q * a.field_stride;
+        node[0] = make_float4((float)ne, (float)te, (float)b, 0.0f);
+        if (a.field_stride == 2) {
             const int k = (int)(q % a.nz), j = (int)((q / a.nz) % a.ny), i = (int)(q / ((int64_t)a.ny * a.nz));
             double bx, by, bz;
             sph_to_view_b<VIEW>(a.view, a.xg[i], a.yg[j], a.zg[k], br, bt, bp, bx, by, bz);
-            a.bcube[q] = make_float4((float)bx, (float)by, (float)bz, 0.0f);
+            node[1] = make_float4((float)bx, (float)by, (float)bz, 0.0f);
         }
     }
 }

@@ -35,7 +35,8 @@ struct FreqDev {
 
 struct MapArgs {
     RayCube cube;
-    const float4 *fcube, *bcube;
+    const float4 *fcube;                 // field nodes; with BVEC the 32-byte ones that carry the B vector
+    int field_stride;                    // float4 per field node (rtgrff_ctx::field_stride)
     GridGeomF fg;
     int64_t n_rays;
     const double *x_start, *y_start, *z_start, *kvec;
@@ -318,8 +319,8 @@ __global__ void __launch_bounds__(RT_BLOCK, RT_MINB) render_map_kernel(const Map
                 if (sample_valid(x, y, z, sv)) {
                     ++n_samples;
                     float3 bv = make_float3(0.f, 0.f, 0.f);
-                    FieldSample f = BVEC ? sample_fields_bvec_fast(a.fcube, a.bcube, a.fg, x, y, z, a.fill_ne, a.fill_te, bv)
-                                         : sample_fields(a.fcube, a.fg, x, y, z, a.fill_ne, a.fill_te, a.fill_b);
+                    FieldSample f = BVEC ? sample_fields_bvec_fast(a.fcube, a.fg, x, y, z, a.fill_ne, a.fill_te, bv)
+                                         : sample_fields(a.fcube, a.field_stride, a.fg, x, y, z, a.fill_ne, a.fill_te, a.fill_b);
                     const float dist = first ? dist_first_np(x, y, z, px, py, pz) : dist_fast(x, y, z, px, py, pz);
                     const float ds = __fmul_rn(dist, a.r_sun_cm);
                     float cthf = 6.123233995736766e-17f, sthf = 1.0f;                       // theta = 90 deg

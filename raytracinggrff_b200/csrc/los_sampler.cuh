@@ -1,6 +1,6 @@
 // LOS resampler for sm_100a: n_e, T, |B| (and optionally the B vector) gathered along recorded
-// paths in ONE launch from one interleaved float4 cube, with the validity mask and the segment
-// lengths ds computed on the device.
+// paths in ONE launch from one channel-interleaved cube of field nodes, with the validity mask and
+// the segment lengths ds computed on the device.
 //
 // Replaces raytracingGRFF/gpu_raytrace.py:539-628 (trilinear_sample_uniform, launched once per
 // field with a fresh H2D of the field each time, :698-700) and the host-side per-ray Python loop
@@ -53,7 +53,8 @@ __device__ __forceinline__ float2 lerp_np2(float2 a, float2 b, float2 u, float2 
     lerp_np(lerp_np(lerp_np(c000.m, c100.m, tx), lerp_np(c010.m, c110.m, tx), ty),                \
             lerp_np(lerp_np(c001.m, c101.m, tx), lerp_np(c011.m, c111.m, tx), ty), tz)
 
-__device__ __forceinline__ FieldSample sample_fields(const float4 *__restrict__ cube, const GridGeomF &g,
+// n_e, T, |B| from the first float4 of each node; `stride` = float4 per node (1, or 2 with the B vector).
+__device__ __forceinline__ FieldSample sample_fields(const float4 *__restrict__ cube, int stride, const GridGeomF &g,
                                                      float px, float py, float pz, float fill_ne,
                                                      float fill_te, float fill_b)
 {
@@ -65,74 +66,25 @@ __device__ __forceinline__ FieldSample sample_fields(const float4 *__restrict__ 
         o.ne = fill_ne; o.te = fill_te; o.b = fill_b;
         return o;
     }
-    const size_t sy = (size_t)g.nz, sx = (size_t)g.ny * g.nz;
-    const float4 *p = cube + ((size_t)i * sx + (size_t)j * sy + (size_t)k);
-    const float4 c000 = __ldg(p), c001 = __ldg(p + 1), c010 = __ldg(p + sy), c011 = __ldg(p + sy + 1);
-    const float4 c100 = __ldg(p + sx), c101 = __ldg(p + sx + 1), c110 = __ldg(p + sx + sy),
-                 c111 = __ldg(p + sx + sy + 1);
+    const size_t sz = (size_t)stride, sy = (size_t)g.nz * sz, sx = (size_t)g.ny * sy;
+    const float4 *p = cube + ((size_t)i * sx + (size_t)j * sy + (size_t)k * sz);
+    const float4 c000 = __ldg(p), c001 = __ldg(p + sz), c010 = __ldg(p + sy), c011 = __ldg(p + sy + sz);
+    const float4 c100 = __ldg(p + sx), c101 = __ldg(p + sx + sz), c110 = __ldg(p + sx + sy),
+                 c111 = __ldg(p + sx + sy + sz);
     // nesting order of the reference: x first, then y, then z (gpu_raytrace.py:528-534)
     o.ne = RT_TRI_NP(x);
     o.te = RT_TRI_NP(y);
     o.b = RT_TRI_NP(z);
     return o;
 }
-
-// n_e, T, |B| and the B vector at one point with one cell search: the two cubes share the grid.
-// Same values as sample_fields + sample_bvec (the packed operations round like the scalar ones).
-__device__ __forceinline__ FieldSample sample_fields_bvec(const float4 *__restrict__ fcube,
-                                                          const float4 *__restrict__ bcube, const GridGeomF &g,
-                                                          float px, float py, float pz, float fill_ne, float fill_te,
-                                                          float fill_b, float3 &bv)
-{
-    FieldSample o;
-    int i, j, k;
-    float tx, ty, tz;
-    o.inb = cell_of(g, px, py, pz, i, j, k, tx, ty, tz);
-    bv = make_float3(0.f, 0.f, 0.f);
-    if (!o.inb) {
-        o.ne = fill_ne; o.te = fill_te; o.b = fill_b;
-        return o;
-    }
-    const size_t sy = (size_t)g.nz, sx = (size_t)g.ny * g.nz;
-    const size_t off = (size_t)i * sx + (size_t)j * sy + (size_t)k;
-    const float2 tx2 = make_float2(tx, tx), ux2 = make_float2(__fsub_rn(1.0f, tx), __fsub_rn(1.0f, tx));
-    const float2 ty2 = make_float2(ty, ty), uy2 = make_float2(__fsub_rn(1.0f, ty), __fsub_rn(1.0f, ty));
-    const float2 tz2 = make_float2(tz, tz), uz2 = make_float2(__fsub_rn(1.0f, tz), __fsub_rn(1.0f, tz));
-#define RT_LO(c) make_float2((c).x, (c).y)
-#define RT_HI(c) make_float2((c).z, (c).w)
-#define RT_TRI_NP2(H)                                                                                         \
-    lerp_np2(lerp_np2(lerp_np2(H(c000), H(c100), ux2, tx2), lerp_np2(H(c010), H(c110), ux2, tx2), uy2, ty2),  \
-             lerp_np2(lerp_np2(H(c001), H(c101), ux2, tx2), lerp_np2(H(c011), H(c111), ux2, tx2), uy2, ty2), uz2, tz2)
-    {
-        const float4 *p = fcube + off;
-        const float4 c000 = __ldg(p), c001 = __ldg(p + 1), c010 = __ldg(p + sy), c011 = __ldg(p + sy + 1);
-        const float4 c100 = __ldg(p + sx), c101 = __ldg(p + sx + 1), c110 = __ldg(p + sx + sy),
-                     c111 = __ldg(p + sx + sy + 1);
-        const float2 nt = RT_TRI_NP2(RT_LO);
-        o.ne = nt.x; o.te = nt.y;
-        o.b = RT_TRI_NP(z);
-    }
-    {
-        const float4 *p = bcube + off;
-        const float4 c000 = __ldg(p), c001 = __ldg(p + 1), c010 = __ldg(p + sy), c011 = __ldg(p + sy + 1);
-        const float4 c100 = __ldg(p + sx), c101 = __ldg(p + sx + 1), c110 = __ldg(p + sx + sy),
-                     c111 = __ldg(p + sx + sy + 1);
-        const float2 bxy = RT_TRI_NP2(RT_LO);
-        bv.x = bxy.x; bv.y = bxy.y;
-        bv.z = RT_TRI_NP(z);
-    }
-#undef RT_TRI_NP2
-#undef RT_LO
-#undef RT_HI
-    return o;
-}
+#undef RT_TRI_NP
 
 // n_e, T (numpy-exact, as sample_fields) and the B vector at one point for the fused map's theta-aware
 // path.  The B vector has no numpy twin in the reference (theta from B.t is an extension), so its
 // three channels use fused lerps a + t (b - a) — a third of the arithmetic — and |B| comes from the
 // vector: the |B| channel of the field cube is not interpolated at all.  o.b = |B vector| (float32).
-__device__ __forceinline__ FieldSample sample_fields_bvec_fast(const float4 *__restrict__ fcube,
-                                                               const float4 *__restrict__ bcube, const GridGeomF &g,
+// `nodes`: the 32-byte nodes {ne, te, |B|, 0, bx, by, bz, 0} (32-byte aligned), one load per corner, not kept in L1.
+__device__ __forceinline__ FieldSample sample_fields_bvec_fast(const float4 *__restrict__ nodes, const GridGeomF &g,
                                                                float px, float py, float pz, float fill_ne,
                                                                float fill_te, float3 &bv)
 {
@@ -146,58 +98,35 @@ __device__ __forceinline__ FieldSample sample_fields_bvec_fast(const float4 *__r
         o.ne = fill_ne; o.te = fill_te;
         return o;
     }
-    const size_t sy = (size_t)g.nz, sx = (size_t)g.ny * g.nz;
-    const size_t off = (size_t)i * sx + (size_t)j * sy + (size_t)k;
+    const size_t sy = (size_t)g.nz * 2, sx = (size_t)g.ny * sy;
+    const float4 *p = nodes + ((size_t)i * sx + (size_t)j * sy + (size_t)k * 2);
+    const Float4x2 c000 = ldg256_no_l1(p), c001 = ldg256_no_l1(p + 2);
+    const Float4x2 c010 = ldg256_no_l1(p + sy), c011 = ldg256_no_l1(p + sy + 2);
+    const Float4x2 c100 = ldg256_no_l1(p + sx), c101 = ldg256_no_l1(p + sx + 2);
+    const Float4x2 c110 = ldg256_no_l1(p + sx + sy), c111 = ldg256_no_l1(p + sx + sy + 2);
     const float2 tx2 = make_float2(tx, tx), ux2 = make_float2(__fsub_rn(1.0f, tx), __fsub_rn(1.0f, tx));
     const float2 ty2 = make_float2(ty, ty), uy2 = make_float2(__fsub_rn(1.0f, ty), __fsub_rn(1.0f, ty));
     const float2 tz2 = make_float2(tz, tz), uz2 = make_float2(__fsub_rn(1.0f, tz), __fsub_rn(1.0f, tz));
-#define RT_LO(c) make_float2((c).x, (c).y)
-#define RT_TRI_NP2(H)                                                                                         \
-    lerp_np2(lerp_np2(lerp_np2(H(c000), H(c100), ux2, tx2), lerp_np2(H(c010), H(c110), ux2, tx2), uy2, ty2),  \
-             lerp_np2(lerp_np2(H(c001), H(c101), ux2, tx2), lerp_np2(H(c011), H(c111), ux2, tx2), uy2, ty2), uz2, tz2)
-    {
-        const float4 *p = fcube + off;
-        const float4 c000 = __ldg(p), c001 = __ldg(p + 1), c010 = __ldg(p + sy), c011 = __ldg(p + sy + 1);
-        const float4 c100 = __ldg(p + sx), c101 = __ldg(p + sx + 1), c110 = __ldg(p + sx + sy),
-                     c111 = __ldg(p + sx + sy + 1);
-        const float2 nt = RT_TRI_NP2(RT_LO);
-        o.ne = nt.x; o.te = nt.y;
-    }
-#undef RT_TRI_NP2
-    {
-        const float4 *p = bcube + off;
-        const float4 c000 = __ldg(p), c001 = __ldg(p + 1), c010 = __ldg(p + sy), c011 = __ldg(p + sy + 1);
-        const float4 c100 = __ldg(p + sx), c101 = __ldg(p + sx + 1), c110 = __ldg(p + sx + sy),
-                     c111 = __ldg(p + sx + sy + 1);
+#define RT_NT(c) make_float2((c).lo.x, (c).lo.y)
+#define RT_BXY(c) make_float2((c).hi.x, (c).hi.y)
+    const float2 nt = lerp_np2(
+        lerp_np2(lerp_np2(RT_NT(c000), RT_NT(c100), ux2, tx2), lerp_np2(RT_NT(c010), RT_NT(c110), ux2, tx2), uy2, ty2),
+        lerp_np2(lerp_np2(RT_NT(c001), RT_NT(c101), ux2, tx2), lerp_np2(RT_NT(c011), RT_NT(c111), ux2, tx2), uy2, ty2),
+        uz2, tz2);
+    o.ne = nt.x; o.te = nt.y;
 #define RT_FL2(a, b, t) __ffma2_rn(t, __fadd2_rn(b, make_float2(-(a).x, -(a).y)), a)
 #define RT_FL(a, b, t) fmaf(t, (b) - (a), a)
-        const float2 bxy = RT_FL2(RT_FL2(RT_FL2(RT_LO(c000), RT_LO(c100), tx2), RT_FL2(RT_LO(c010), RT_LO(c110), tx2), ty2),
-                                  RT_FL2(RT_FL2(RT_LO(c001), RT_LO(c101), tx2), RT_FL2(RT_LO(c011), RT_LO(c111), tx2), ty2), tz2);
-        bv.x = bxy.x; bv.y = bxy.y;
-        bv.z = RT_FL(RT_FL(RT_FL(c000.z, c100.z, tx), RT_FL(c010.z, c110.z, tx), ty),
-                     RT_FL(RT_FL(c001.z, c101.z, tx), RT_FL(c011.z, c111.z, tx), ty), tz);
+    const float2 bxy = RT_FL2(RT_FL2(RT_FL2(RT_BXY(c000), RT_BXY(c100), tx2), RT_FL2(RT_BXY(c010), RT_BXY(c110), tx2), ty2),
+                              RT_FL2(RT_FL2(RT_BXY(c001), RT_BXY(c101), tx2), RT_FL2(RT_BXY(c011), RT_BXY(c111), tx2), ty2), tz2);
+    bv.x = bxy.x; bv.y = bxy.y;
+    bv.z = RT_FL(RT_FL(RT_FL(c000.hi.z, c100.hi.z, tx), RT_FL(c010.hi.z, c110.hi.z, tx), ty),
+                 RT_FL(RT_FL(c001.hi.z, c101.hi.z, tx), RT_FL(c011.hi.z, c111.hi.z, tx), ty), tz);
 #undef RT_FL2
 #undef RT_FL
-    }
-#undef RT_LO
+#undef RT_NT
+#undef RT_BXY
     return o;
 }
-
-// B vector at a point (extension used by the theta-aware GR+FF path); zeros outside the cube.
-__device__ __forceinline__ float3 sample_bvec(const float4 *__restrict__ cube, const GridGeomF &g,
-                                              float px, float py, float pz)
-{
-    int i, j, k;
-    float tx, ty, tz;
-    if (!cell_of(g, px, py, pz, i, j, k, tx, ty, tz)) return make_float3(0.f, 0.f, 0.f);
-    const size_t sy = (size_t)g.nz, sx = (size_t)g.ny * g.nz;
-    const float4 *p = cube + ((size_t)i * sx + (size_t)j * sy + (size_t)k);
-    const float4 c000 = __ldg(p), c001 = __ldg(p + 1), c010 = __ldg(p + sy), c011 = __ldg(p + sy + 1);
-    const float4 c100 = __ldg(p + sx), c101 = __ldg(p + sx + 1), c110 = __ldg(p + sx + sy),
-                 c111 = __ldg(p + sx + sy + 1);
-    return make_float3(RT_TRI_NP(x), RT_TRI_NP(y), RT_TRI_NP(z));
-}
-#undef RT_TRI_NP
 
 __device__ __forceinline__ bool sample_valid(float x, float y, float z, float s)
 {
@@ -241,6 +170,7 @@ __device__ __forceinline__ float dist_first_np(float ax, float ay, float az, flo
 
 struct SampleArgs {
     const float4 *fcube;
+    int field_stride;        // float4 per field node (rtgrff_ctx::field_stride)
     GridGeomF g;
     int64_t n_rec, n_rays;
     // exactly one of the two position sources is set
@@ -283,7 +213,9 @@ __global__ void __launch_bounds__(256) sample_paths_kernel(const SampleArgs a)
         float x, y, z, s;
         load_sample(a, rec, ray, x, y, z, s);
         const bool v = sample_valid(x, y, z, s);
-        const FieldSample f = sample_fields(a.fcube, a.g, x, y, z, a.fill_ne, a.fill_te, a.fill_b);
+        // the stride as a literal on each side: the 16-byte nodes keep the address arithmetic of a one-layout kernel
+        const FieldSample f = a.field_stride == 1 ? sample_fields(a.fcube, 1, a.g, x, y, z, a.fill_ne, a.fill_te, a.fill_b)
+                                                  : sample_fields(a.fcube, 2, a.g, x, y, z, a.fill_ne, a.fill_te, a.fill_b);
         float ds = 0.0f;
         if (v) {
             int64_t pr = rec - 1;
@@ -305,22 +237,22 @@ __global__ void __launch_bounds__(256) sample_paths_kernel(const SampleArgs a)
     }
 }
 
-// {ne, te, b} float32 cubes -> one float4 cube (w = 0); {bx,by,bz} likewise.
+// {ne, te, b} float32 cubes -> float4 {ne, te, b, 0} at out[q * stride]; {bx,by,bz} likewise (out = nodes + 1).
 __global__ void interleave3_kernel(const float *__restrict__ a, const float *__restrict__ b,
-                                   const float *__restrict__ c, float4 *__restrict__ out, int64_t n)
+                                   const float *__restrict__ c, float4 *__restrict__ out, int stride, int64_t n)
 {
     for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q < n;
          q += (int64_t)gridDim.x * blockDim.x)
-        out[q] = make_float4(a[q], b[q], c[q], 0.0f);
+        out[q * stride] = make_float4(a[q], b[q], c[q], 0.0f);
 }
 
-// the inverse: one channel-interleaved cube -> three planar arrays (rtgrff_export_cubes)
-__global__ void deinterleave3_kernel(const float4 *__restrict__ in, float *__restrict__ a, float *__restrict__ b,
-                                     float *__restrict__ c, int64_t n)
+// the inverse: the float4 at in[q * stride] -> three planar arrays (rtgrff_export_cubes)
+__global__ void deinterleave3_kernel(const float4 *__restrict__ in, int stride, float *__restrict__ a,
+                                     float *__restrict__ b, float *__restrict__ c, int64_t n)
 {
     for (int64_t q = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; q < n;
          q += (int64_t)gridDim.x * blockDim.x) {
-        const float4 v = in[q];
+        const float4 v = in[q * stride];
         a[q] = v.x; b[q] = v.y; c[q] = v.z;
     }
 }

@@ -23,7 +23,7 @@
 //  * Fast path of an RHS = one range test (VIMNMX3.U32 + ISETP on the bit patterns: 0 <= t < 1)
 //    + the evaluation, ~55 instructions.  Everything else — leaving the cell, the cube bounds,
 //    the re-fetch — is the slow path (move_cell), which 1-5 of a warp's 32 lanes take at a time:
-//    it is kept short by the polynomial cube (8 LDG.128 from one 128-byte line, no differencing)
+//    it is kept short by the polynomial cube (4 LDG.256 from one 128-byte line, no differencing)
 //    and by a per-step `edge` flag that drops the bounds logic in the interior.
 //  * One RHS body per RK4 stage (the stage loop is unrolled: constant weights), the three rays
 //    of a step (central + two pencil rays) are a rolled loop, the face handling is a run-time
@@ -88,20 +88,19 @@ __device__ __noinline__ void load_cell_nodes(const float4 *__restrict__ nodes, i
 }
 
 // Make the cell at element offset `off` the cached one.  With the cell-major polynomial cube
-// (build_poly_cube_kernel) that is 8 LDG.128 from one 128-byte line; without it: load_cell_nodes.
+// (build_poly_cube_kernel) that is 4 LDG.256 from one 128-byte line; without it: load_cell_nodes.
 __device__ __forceinline__ void load_cell(const RayCube &C, int off, Cell &c)
 {
     if (C.pc) {
         c.off = off;
         const float4 *p = C.pc + (size_t)off * 8;
-        const float4 q0 = __ldg(p), q1 = __ldg(p + 1), q2 = __ldg(p + 2), q3 = __ldg(p + 3);
-        const float4 q4 = __ldg(p + 4), q5 = __ldg(p + 5), q6 = __ldg(p + 6), q7 = __ldg(p + 7);
+        const Float4x2 q01 = ldg256(p), q23 = ldg256(p + 2), q45 = ldg256(p + 4), q67 = ldg256(p + 6);
 #define RT_A(q) make_float2((q).x, (q).y)
 #define RT_B(q) make_float2((q).z, (q).w)
-        c.l0 = RT_A(q0); c.lz = RT_B(q0); c.ly = RT_A(q1); c.lyz = RT_B(q1);
-        c.lx = RT_A(q2); c.lxz = RT_B(q2); c.lxy = RT_A(q3); c.lxyz = RT_B(q3);
-        c.h0 = RT_A(q4); c.hz = RT_B(q4); c.hy = RT_A(q5); c.hyz = RT_B(q5);
-        c.hx = RT_A(q6); c.hxz = RT_B(q6); c.hxy = RT_A(q7); c.hxyz = RT_B(q7);
+        c.l0 = RT_A(q01.lo); c.lz = RT_B(q01.lo); c.ly = RT_A(q01.hi); c.lyz = RT_B(q01.hi);
+        c.lx = RT_A(q23.lo); c.lxz = RT_B(q23.lo); c.lxy = RT_A(q23.hi); c.lxyz = RT_B(q23.hi);
+        c.h0 = RT_A(q45.lo); c.hz = RT_B(q45.lo); c.hy = RT_A(q45.hi); c.hyz = RT_B(q45.hi);
+        c.hx = RT_A(q67.lo); c.hxz = RT_B(q67.lo); c.hxy = RT_A(q67.hi); c.hxyz = RT_B(q67.hi);
 #undef RT_A
 #undef RT_B
         return;

@@ -505,7 +505,7 @@ int rtgrff_ctx_destroy(rtgrff_ctx *c)
         if (n) n->CommDestroy((NcclComm)c->comm);
         c->comm = nullptr;
     }
-    DevBuf *bufs[] = {&c->wcube, &c->pcube, &c->fcube, &c->bcube, &c->rec_pos, &c->rec_s, &c->smp_ne, &c->smp_te, &c->smp_b,
+    DevBuf *bufs[] = {&c->wcube, &c->pcube, &c->fcube, &c->rec_pos, &c->rec_s, &c->smp_ne, &c->smp_te, &c->smp_b,
                       &c->smp_ds, &c->smp_s, &c->smp_valid, &c->in0, &c->in1, &c->in2, &c->in3, &c->out0, &c->out1,
                       &c->out2, &c->out3, &c->out4, &c->out5, &c->stage, &c->counters, &c->gather_buf, &c->image_buf};
     for (DevBuf *b : bufs) b->release();
@@ -588,6 +588,17 @@ int rtgrff_set_omega_cube(rtgrff_ctx *c, const double *omega_pe, int nx, int ny,
     return RTGRFF_OK;
 }
 
+// The field nodes of nvox grid points at `stride` float4 each.  The 32-byte nodes are read with one 32-byte load
+// per corner (sample_fields_bvec_fast), which needs them 32-byte aligned: cudaMalloc gives 256 bytes.
+static int reserve_field_nodes(rtgrff_ctx *c, size_t nvox, int stride)
+{
+    c->has_fcube = c->has_bvec = false;     // overwritten from here on: nothing samples them until the caller is done
+    RT_TRY(c->fcube.reserve(nvox * stride * sizeof(float4)));
+    if ((uintptr_t)c->fcube.p % (stride * sizeof(float4)) != 0)
+        return fail(RTGRFF_ECUDA, "field nodes at %p are not %zu-byte aligned", c->fcube.p, stride * sizeof(float4));
+    return RTGRFF_OK;
+}
+
 int rtgrff_set_field_cubes(rtgrff_ctx *c, const float *ne, const float *te, const float *b, const float *bx,
                            const float *by, const float *bz, int nx, int ny, int nz, const double geom[12])
 {
@@ -598,21 +609,23 @@ int rtgrff_set_field_cubes(rtgrff_ctx *c, const float *ne, const float *te, cons
     GridGeom g;
     RT_TRY(geom_from(geom, nx, ny, nz, g));
     const size_t nvox = (size_t)nx * ny * nz, fb = nvox * sizeof(float);
+    const int stride = bvec ? 2 : 1;
     RT_TRY(c->stage.reserve(3 * fb));
     c->stage_has_omega = false;
     float *s0 = c->stage.as<float>(), *s1 = s0 + nvox, *s2 = s1 + nvox;
-    RT_TRY(c->fcube.reserve(nvox * sizeof(float4)));
+    RT_TRY(reserve_field_nodes(c, nvox, stride));
     RT_TRY(h2d_large(c, s0, ne, fb));
     RT_TRY(h2d_large(c, s1, te, fb));
     RT_TRY(h2d_large(c, s2, b, fb));
-    interleave3_kernel<<<blocks_for((int64_t)nvox, 256), 256, 0, c->stream>>>(s0, s1, s2, c->fcube.as<float4>(), (int64_t)nvox);
+    interleave3_kernel<<<blocks_for((int64_t)nvox, 256), 256, 0, c->stream>>>(s0, s1, s2, c->fcube.as<float4>(), stride,
+                                                                               (int64_t)nvox);
     RT_TRY(launched(c, "interleave3_kernel"));
     if (bvec) {
-        RT_TRY(c->bcube.reserve(nvox * sizeof(float4)));
         RT_TRY(h2d_large(c, s0, bx, fb));
         RT_TRY(h2d_large(c, s1, by, fb));
         RT_TRY(h2d_large(c, s2, bz, fb));
-        interleave3_kernel<<<blocks_for((int64_t)nvox, 256), 256, 0, c->stream>>>(s0, s1, s2, c->bcube.as<float4>(), (int64_t)nvox);
+        interleave3_kernel<<<blocks_for((int64_t)nvox, 256), 256, 0, c->stream>>>(s0, s1, s2, c->fcube.as<float4>() + 1,
+                                                                                   stride, (int64_t)nvox);
         RT_TRY(launched(c, "interleave3_kernel"));
     }
     c->fgeom = g;
@@ -770,8 +783,8 @@ int rtgrff_compose_cubes(rtgrff_ctx *c, int want_bvec)
     RT_TRY(geom_from(geom, nx, ny, nz, g));
     const size_t nvox = (size_t)nx * ny * nz;
     RT_TRY(c->stage.reserve(nvox * sizeof(double)));
-    RT_TRY(c->fcube.reserve(nvox * sizeof(float4)));
-    if (want_bvec) RT_TRY(c->bcube.reserve(nvox * sizeof(float4)));
+    const int stride = want_bvec ? 2 : 1;
+    RT_TRY(reserve_field_nodes(c, nvox, stride));
     RT_TRY(c->wcube.reserve(nvox * sizeof(float4)));
     ComposeArgs a;
     a.ne = c->slot[0].as<double>(); a.te = c->slot[1].as<double>();
@@ -780,7 +793,7 @@ int rtgrff_compose_cubes(rtgrff_ctx *c, int want_bvec)
     a.xg = c->slot_grids.as<double>(); a.yg = a.xg + nx; a.zg = a.yg + ny;
     a.omega_pe = c->stage.as<double>();
     a.fcube = c->fcube.as<float4>();
-    a.bcube = want_bvec ? c->bcube.as<float4>() : nullptr;
+    a.field_stride = stride;
     a.view = view;
     unsigned int blocks = blocks_for((int64_t)nvox, 256);
     if (view.on) compose_cubes_kernel<true><<<blocks, 256, 0, c->stream>>>(a);
@@ -871,6 +884,7 @@ static int prepare_sampler(rtgrff_ctx *c, SampleArgs &a, double r_sun_cm, double
     RT_TRY(c->smp_ne.reserve(n * 4)); RT_TRY(c->smp_te.reserve(n * 4)); RT_TRY(c->smp_b.reserve(n * 4));
     RT_TRY(c->smp_ds.reserve(n * 4)); RT_TRY(c->smp_s.reserve(n * 4)); RT_TRY(c->smp_valid.reserve(n));
     a.fcube = c->fcube.as<float4>();
+    a.field_stride = c->field_stride();
     a.g = c->fgeomf;
     a.r_sun_cm = (float)r_sun_cm;   // numpy 2: float32 array * python float stays float32 (gpu_raytrace.py:482-484)
     a.fill_ne = (float)fill_ne; a.fill_te = (float)fill_te; a.fill_b = (float)fill_b;
@@ -1161,8 +1175,9 @@ int rtgrff_export_cubes(rtgrff_ctx *c, double *omega_pe, float *ne, float *te, f
         const size_t n = (size_t)c->fgeom.nx * c->fgeom.ny * c->fgeom.nz;
         RT_TRY(c->out3.reserve(3 * n * sizeof(float)));
         float *d = c->out3.as<float>();
-        deinterleave3_kernel<<<blocks_for((int64_t)n, 256), 256, 0, c->stream>>>((pass ? c->bcube : c->fcube).as<float4>(), d,
-                                                                                  d + n, d + 2 * n, (int64_t)n);
+        deinterleave3_kernel<<<blocks_for((int64_t)n, 256), 256, 0, c->stream>>>(c->fcube.as<float4>() + pass,
+                                                                                  c->field_stride(), d, d + n, d + 2 * n,
+                                                                                  (int64_t)n);
         RT_TRY(launched(c, "deinterleave3_kernel"));
         for (int m = 0; m < 3; ++m)
             if (o[m]) RT_TRY(d2h(c, o[m], d + (size_t)m * n, n * sizeof(float)));
@@ -1311,7 +1326,7 @@ static int render_map_impl(rtgrff_ctx *c, int64_t n_rays, const double *x_start,
     MapArgs a;
     a.cube = rc;
     a.fcube = c->fcube.as<float4>();
-    a.bcube = c->has_bvec ? c->bcube.as<float4>() : nullptr;
+    a.field_stride = c->field_stride();
     a.fg = c->fgeomf;
     a.n_rays = n_rays;
     a.x_start = c->in0.as<double>(); a.y_start = c->in1.as<double>(); a.z_start = c->in2.as<double>();
